@@ -315,7 +315,8 @@ int mls_obs_unpack(const void* packed, const int64_t* src_frame, const int32_t* 
  *                   accumulated in fp64
  *   boot_round[m] = ring round of the bootstrap observation when the chain is alive after n_step steps, else -1
  *   boot_gamma[m] = gamma^n_step
- * The caller samples only transitions whose n-step window is already stored. */
+ * The caller samples only transitions whose n-step window and bootstrap observation (round + n_step) are already
+ * stored, so that round must not have been overwritten either: ring_rounds > n_step. */
 int mls_nstep_returns(const double* rew, const uint8_t* flags, int32_t ring_rounds, int64_t n_episodes,
                       int32_t n_nodes, const int32_t* round_index, const int32_t* episode, const int32_t* agent,
                       int32_t n_samples, int32_t n_step, double gamma, float* returns, int32_t* boot_round,

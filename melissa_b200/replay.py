@@ -77,18 +77,22 @@ class DeviceReplay:
 
     # ------------------------------------------------------------------ sampling
     def sample_indices(self, batch_size: int, n_step: int):
-        """Uniform over the stored transitions whose n-step window is complete (stored at least ``n_step`` rounds
-        ago or terminated earlier -- chains never outlive their TTL, so "stored n_step rounds ago" covers both).
-        -> (ring round, episode, agent) int32 tensors [M]."""
+        """Uniform over the stored transitions whose n-step window AND its bootstrap frame are stored: round rho is
+        usable when rounds rho .. rho+n_step are all in the ring (a chain still alive after n_step steps bootstraps
+        from the observation of round rho+n_step, which is only packed by the next ``begin_round``).  Needs
+        ``ring_rounds > n_step``.  -> (ring round, episode, agent) int32 tensors [M]."""
+        if n_step >= self.R:
+            raise ValueError(f"a ring of {self.R} rounds cannot hold an n-step window of {n_step} rounds plus its "
+                             "bootstrap frame (needs ring_rounds > n_step)")
         filled = min(self.head, self.R)
-        usable = filled - (n_step - 1)             # a window needs rounds rho .. rho+n_step-1 to be stored
+        usable = filled - n_step                   # rounds rho .. rho+n_step must be stored; the oldest is overwritten last
         if usable <= 0:
             raise RuntimeError("not enough rounds stored for an n-step window")
         if not self._nonempty:                     # one host check, then everything stays on the device
             if int(self.counts.sum().item()) == 0:
                 raise RuntimeError("replay holds no transitions yet")
             self._nonempty = True
-        # ring slots ordered oldest -> newest; the newest n_step-1 rounds cannot start a complete window
+        # ring slots ordered oldest -> newest; the newest n_step rounds cannot start a complete window
         order = ((torch.arange(usable, device=self.device) + (self.head - filled)) % self.R)
         cnt = self.counts[order]
         cum = torch.cumsum(cnt, 0)

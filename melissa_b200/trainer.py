@@ -68,7 +68,7 @@ class OffpolicyTrainer:
                 if self.max_update_per_collect is not None:
                     n_upd = min(n_upd, self.max_update_per_collect)
                 for _ in range(n_upd):
-                    if buffer.head < sub._n_step:
+                    if buffer.head <= sub._n_step:
                         break
                     out = self.policy.update(self.batch_size, buffer)
                     self.last_loss = out["loss"]

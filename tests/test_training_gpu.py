@@ -16,7 +16,7 @@ pytestmark = pytest.mark.gpu
 DUELING = lambda: ({"hidden_sizes": [128, 128]}, {"hidden_sizes": [128, 128]})
 
 
-def _setup(kind="l_dgn", N=20, B=64, P=512, seed=3, ring=12, n_step=4, target_freq=0, policy_cls=None, lr=1e-3, **kw):
+def _setup(kind="l_dgn", N=20, B=64, P=512, seed=3, ring=12, n_step=4, target_freq=0, policy_cls=None, lr=1e-3, heads=4, **kw):
     from melissa_b200.batched_env import BatchedGraphEnv, ResetTuplesDevice
     from melissa_b200.data_parallel import FlatParameters, FusedAdam
     from melissa_b200.networks import NETWORKS
@@ -25,7 +25,7 @@ def _setup(kind="l_dgn", N=20, B=64, P=512, seed=3, ring=12, n_step=4, target_fr
     pool = GraphPool.synthetic(N, 8, first_seed=seed)
     tup = reset_chain.episode_pool(seed, P, N, 8)
     torch.manual_seed(seed)
-    net = NETWORKS[kind](5, 128, 2, 4, N, dueling_param=DUELING(), device="cuda", **kw).cuda()
+    net = NETWORKS[kind](5, 128, 2, heads, N, dueling_param=DUELING(), device="cuda", **kw).cuda()
     flat = FlatParameters(net)
     optim = FusedAdam(flat, lr=lr)
     pol = (policy_cls or DQNPolicy)(net, optim, discount_factor=0.99, estimation_step=n_step, target_update_freq=target_freq, eps=0.1)
@@ -65,11 +65,12 @@ def test_obs_pack_unpack_is_lossless_and_counts_bad_rows():
     assert torch.equal(ar[:, :-1], env.obs.view(env.B, -1)[frames]) and ar[:, -1].tolist() == [5.0, 1.0, 19.0]
 
 
-def test_replay_stores_what_the_multi_agent_collector_would_and_nstep_returns_follow_tianshou():
+def test_replay_stores_what_the_multi_agent_collector_would_and_samples_only_windows_with_a_stored_bootstrap_frame():
     """The oracle environment is driven in lockstep with the device's actions.  Every agent transition of a round must be
     in the ring with: the observation the agent decided on, its action, the reward of the world step that followed,
     terminated exactly when its TTL ended -- the completion rule of multi_agent_collector.py:240-308 -- and the sampled
-    n-step returns must equal tianshou's compute_nstep_return on the agent's own chain."""
+    n-step returns must equal tianshou's compute_nstep_return on the agent's own chain.  Sampling never starts a window
+    in the newest n_step rounds: the bootstrap observation of round rho + n_step must already be stored."""
     N, B, P, R = 20, 64, 512, 12
     s = _setup(N=N, B=B, P=P, ring=R)
     env, replay, col, pool = s["env"], s["replay"], s["col"], s["pool"]
@@ -104,7 +105,7 @@ def test_replay_stores_what_the_multi_agent_collector_would_and_nstep_returns_fo
         rho, ep, ag = replay.sample_indices(4000, n_step)
         b = replay.gather(rho, ep, ag, n_step, 0.99)
         rho_n, ep_n, ag_n = rho.cpu().numpy(), ep.cpu().numpy(), ag.cpu().numpy()
-        assert rho_n.max() <= R - n_step and len(np.unique(rho_n)) > 1
+        assert rho_n.max() == R - 1 - n_step and len(np.unique(rho_n)) > 1     # window + bootstrap frame stored
         rows, ret, boot = b["obs"].cpu().numpy(), b["returns"].cpu().numpy(), b["boot_round"].cpu().numpy()
         for m in range(0, 4000, 37):
             r0, e, a = int(rho_n[m]), int(ep_n[m]), int(ag_n[m])
@@ -124,10 +125,12 @@ def test_replay_stores_what_the_multi_agent_collector_would_and_nstep_returns_fo
             assert ret[m] == pytest.approx(want, rel=1e-6, abs=1e-6)
             alive = not any(term_c[:n_step])
             assert (boot[m] >= 0) == alive and (not alive or boot[m] == (r0 + n_step) % R)
-    # uniformity: every stored complete-window transition is equally likely (coarse check per ring round)
+    # uniformity: every stored transition whose window and bootstrap frame are stored is equally likely (coarse check
+    # per ring round; with n_step 1 that is every round but the newest)
     rho, _, _ = replay.sample_indices(200000, 1)
     freq = np.bincount(rho.cpu().numpy(), minlength=R) / 200000
     cnt = replay.counts.cpu().numpy().astype(np.float64)
+    cnt[R - 1] = 0.0
     np.testing.assert_allclose(freq, cnt / cnt.sum(), atol=0.01)
 
 
@@ -185,15 +188,26 @@ def test_training_forward_agrees_with_the_rollout_kernels(kind, kw):
     assert float((q_b - q_t).abs().max()) <= 1e-2 * scale
 
 
-@pytest.mark.parametrize("agg", ["max", "mean", "add"])
-def test_fused_hl_dgn_training_forward_backward_matches_the_torch_path(agg):
-    from melissa_b200.networks import autograd as ag
-    s = _setup(kind="hl_dgn", N=20, aggregator=agg)
+def _rows(s, n, synthetic):
+    """Agent-observation rows: from a short rollout, or synthetic (one complete-graph sample, one isolated controlling
+    node)."""
+    if synthetic:
+        return train_oracle.agent_rows(s["N"], n, seed=s["N"] + n, complete=(0,), isolated=(1,)).cuda()
     for _ in range(6):
         s["col"].iterate(0.3)
-    env, net = s["env"], s["net"]
+    env = s["env"]
     b_idx, a_idx = torch.nonzero(env.active, as_tuple=True)
-    rows = torch.cat([env.obs.view(env.B, -1)[b_idx], a_idx.float()[:, None]], dim=1)[:200]
+    return torch.cat([env.obs.view(env.B, -1)[b_idx], a_idx.float()[:, None]], dim=1)[:n]
+
+
+@pytest.mark.parametrize("agg,synthetic,heads", [("max", False, 4), ("mean", False, 4), ("add", False, 4),
+                                                 ("max", True, 1), ("add", True, 2), ("mean", True, 4)],
+                         ids=["max", "mean", "add", "max-synthetic-h1", "add-synthetic-h2", "mean-synthetic-h4"])
+def test_fused_hl_dgn_training_forward_backward_matches_the_torch_path(agg, synthetic, heads):
+    from melissa_b200.networks import autograd as ag
+    s = _setup(kind="hl_dgn", N=20, aggregator=agg, heads=heads)
+    net = s["net"]
+    rows = _rows(s, 200, synthetic)
     assert ag.fused_training_available(net, rows)
     target = torch.linspace(-1, 1, rows.shape[0], device=rows.device)
     res = []
@@ -208,18 +222,19 @@ def test_fused_hl_dgn_training_forward_backward_matches_the_torch_path(agg):
         assert float((g_t[k] - g_f[k]).abs().max()) <= 1e-4 * max(float(g_t[k].abs().max()), 1e-6), k
 
 
-@pytest.mark.parametrize("kind,N", [("l_dgn", 20), ("l_dgn", 50), ("dgn_r", 20), ("dgn_r", 50)])
-def test_fused_gatv2_training_kernels_match_the_torch_autograd_path(kind, N):
+@pytest.mark.parametrize("kind,N,synthetic,heads", [("l_dgn", 20, False, 4), ("l_dgn", 50, False, 4), ("dgn_r", 20, False, 4),
+                                                    ("dgn_r", 50, False, 4), ("l_dgn", 50, True, 1), ("l_dgn", 20, True, 2),
+                                                    ("dgn_r", 50, True, 2), ("dgn_r", 20, True, 4)],
+                         ids=["l_dgn-20", "l_dgn-50", "dgn_r-20", "dgn_r-50", "l_dgn-50-synthetic-h1", "l_dgn-20-synthetic-h2",
+                              "dgn_r-50-synthetic-h2", "dgn_r-20-synthetic-h4"])
+def test_fused_gatv2_training_kernels_match_the_torch_autograd_path(kind, N, synthetic, heads):
     """mls_train_lists + mls_gatv2_edge_fwd / _bwd (the L-DGN training forward / backward) against the plain torch-op
     formulation of the same math (autograd.q_values_torch, itself pinned to the oracle on the CPU): Q-values to 1e-5 and
     every parameter gradient to 1e-4 of the gradient's scale (fp32, different summation orders and atomics)."""
     from melissa_b200.networks import autograd as ag
-    s = _setup(kind=kind, N=N)
-    for _ in range(6):
-        s["col"].iterate(0.3)
-    env, net = s["env"], s["net"]
-    b_idx, a_idx = torch.nonzero(env.active, as_tuple=True)
-    rows = torch.cat([env.obs.view(env.B, -1)[b_idx], a_idx.float()[:, None]], dim=1)[:400]
+    s = _setup(kind=kind, N=N, heads=heads)
+    net = s["net"]
+    rows = _rows(s, 400, synthetic)
     assert rows.shape[0] >= 50 and ag.fused_training_available(net, rows)
     target = torch.linspace(-1, 1, rows.shape[0], device=rows.device)
     grads = []
@@ -290,6 +305,8 @@ def test_bootstrap_path_with_short_windows_and_target_network():
     assert bool(alive.any()) and bool((~alive).any())
     base = raw["returns"].clone()
     b = pol.process_fn(Batch(raw), replay)
+    # double DQN on the bootstrap rows; that rows_at returns the observation of round rho + n_step is checked against
+    # the oracle environment in test_training_replay_gpu.py
     rows = replay.rows_at(raw["boot_round"][alive], raw["ep"][alive], raw["agent"][alive])
     q_on, _ = pol.model(rows)
     q_old, _ = pol.model_old(rows)

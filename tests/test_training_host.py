@@ -108,6 +108,60 @@ def test_nstep_restatement_on_hand_cases():
     assert train_oracle.nstep_return_chain(rew, term, 3, 1, g, lambda t: 10.0) == pytest.approx(4.0)
 
 
+def test_adam_restatement_continues_from_a_given_state():
+    rng = np.random.default_rng(4)
+    p0 = rng.standard_normal(33)
+    grads = [rng.standard_normal(33) for _ in range(5)]
+    want = train_oracle.adam_reference(p0, grads, lr=1e-2, weight_decay=0.01)
+    p, m, v = train_oracle.adam_reference(p0, grads[:2], lr=1e-2, weight_decay=0.01, state=(np.zeros(33), np.zeros(33), 0))
+    for t, g in enumerate(grads[2:], start=2):
+        p, m, v = train_oracle.adam_reference(p, [g], lr=1e-2, weight_decay=0.01, state=(m, v, t))
+    np.testing.assert_allclose(p, want, rtol=1e-14, atol=1e-15)
+
+
+def _dense_lists(edges):
+    """Fixed-capacity lists (self first, then the sources in index order) of every node of dense masks [B, i, j]."""
+    B, N, _ = edges.shape
+    cap = 36
+    tgt, src, cnt = [], [], []
+    for b in range(B):
+        for i in range(N):
+            s = [i] + torch.nonzero(edges[b, i]).flatten().tolist()
+            tgt.append(b * N + i)
+            src.append([b * N + j for j in s] + [0] * (cap - len(s)))
+            cnt.append(len(s))
+    as_i32 = lambda x: torch.tensor(x, dtype=torch.int32)
+    return as_i32(tgt), as_i32(src), as_i32(cnt)
+
+
+@pytest.mark.parametrize("heads", [1, 3, 4])
+@pytest.mark.parametrize("seed", [0, 1])
+def test_edge_references_equal_the_dense_oracle_convolutions(heads, seed):
+    """oracle/train_oracle.py's list-based float64 references of the training edge kernels against net_oracle's dense
+    GATv2Conv / TransformerConv (bias removed) on random radius graphs, isolated nodes included."""
+    torch.manual_seed(seed)
+    B, N, D, HC = 3, 12, 16, heads * 128
+    pos = torch.rand(B, N, 2, dtype=torch.float64) * 0.5
+    pos[0, 0] = 5.0                                                # an isolated node
+    edges = no.radius_graph_mask(pos)
+    x = torch.randn(B, N, D, dtype=torch.float64)
+    w = lambda *s: torch.randn(*s, dtype=torch.float64) * 0.3
+    sd = {"c.lin_l.weight": w(HC, D), "c.lin_l.bias": w(HC), "c.lin_r.weight": w(HC, D), "c.lin_r.bias": w(HC),
+          "c.att": w(1, heads, 128), "c.bias": torch.zeros(HC, dtype=torch.float64),
+          "c.lin_query.weight": w(HC, D), "c.lin_query.bias": w(HC), "c.lin_key.weight": w(HC, D), "c.lin_key.bias": w(HC),
+          "c.lin_value.weight": w(HC, D), "c.lin_value.bias": w(HC)}
+    lin = lambda k: torch.nn.functional.linear(x, sd[f"c.{k}.weight"], sd[f"c.{k}.bias"]).reshape(B * N, HC)
+    tgt, src, cnt = _dense_lists(edges)
+    want = no.gatv2_conv(sd, "c", x, edges, heads).reshape(B * N, HC)
+    got, alpha = train_oracle.gatv2_edge_reference(lin("lin_l"), lin("lin_r"), sd["c.att"].view(-1), tgt, src, cnt, heads)
+    torch.testing.assert_close(got, want, rtol=1e-12, atol=1e-12)
+    torch.testing.assert_close(alpha.sum(1), torch.ones(B * N, heads, dtype=torch.float64), rtol=1e-12, atol=1e-12)
+    want = no.transformer_conv(sd, "c", x, edges, heads).reshape(B * N, HC)
+    got, alpha = train_oracle.transformer_edge_reference(lin("lin_query"), lin("lin_key"), lin("lin_value"), tgt, src, cnt, heads)
+    torch.testing.assert_close(got, want, rtol=1e-12, atol=1e-12)
+    assert float(got[0].abs().max()) == 0.0 and float(alpha[:, 0].abs().max()) == 0.0   # isolated node; entry 0 skipped
+
+
 def _dp_worker(rank, world, port, out_dir):
     import torch.distributed as dist
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
