@@ -722,29 +722,6 @@ __global__ void gather_x0_kernel(const int* __restrict__ idx, const int* __restr
   }
 }
 
-struct ActArgsB {
-  float eps;
-  uint64_t seed, offset;
-  const double* rand3;
-  const unsigned long long* offset_dev;   // optional device-side addend (round counter under CUDA-graph replay)
-  uint64_t row0;                          // added to the row index that keys the Philox draw (sub-batch calls)
-};
-__device__ __forceinline__ int select_action_b(float q0, float q1, const ActArgsB& a, uint64_t row) {
-  int act = q1 > q0 ? 1 : 0;
-  if (fabsf(a.eps) > 1e-8f) {
-    double ue, u0, u1;
-    if (a.rand3) { ue = a.rand3[row * 3 + 0]; u0 = a.rand3[row * 3 + 1]; u1 = a.rand3[row * 3 + 2]; }
-    else {
-      Philox4 r = philox4x32_10(a.seed, row + a.row0, a.offset + (a.offset_dev ? *a.offset_dev : 0ull));
-      ue = u01_from_u32x2(r.v[0], r.v[1]);
-      u0 = (double)r.v[2] * (1.0 / 4294967296.0);
-      u1 = (double)r.v[3] * (1.0 / 4294967296.0);
-    }
-    if (ue < (double)a.eps) act = (u1 + 1.0) > (u0 + 1.0) ? 1 : 0;
-  }
-  return act;
-}
-
 // last head layer + dueling + action; hid row = [Q hidden (hh) | V hidden (hh)] in bf16
 __global__ void head_out_bf16_kernel(const bf16* __restrict__ hid, int hh, const int* __restrict__ idx, const int* __restrict__ count,
                                      int max_rows, const float* __restrict__ wq, const float* __restrict__ bq,
@@ -775,27 +752,6 @@ __global__ void head_out_bf16_kernel(const bf16* __restrict__ hid, int hh, const
     q_out[orow * 2 + 1] = o1;
     if (act_out && out_mode != 2) act_out[orow] = (int8_t)select_action_b(o0, o1, aa, (uint64_t)orow);
   }
-}
-
-// Output layer of the dueling heads from the three dot products the last hidden-layer GEMM left per row
-// (dots[t] = (<relu(hq), wq[0]>, <relu(hv), wv>), dots2[t] = (<relu(hq), wq[1]>, -)); same outputs as head_out_bf16_kernel.
-__global__ void head_final_kernel(const float* __restrict__ dots, const float* __restrict__ dots2, const int* __restrict__ idx,
-                                  const int* __restrict__ count, int max_rows, const float* __restrict__ bq, const float* __restrict__ bv,
-                                  int64_t row0, int per_graph_N, float* __restrict__ q_out, int8_t* __restrict__ act_out, int out_mode,
-                                  ActArgsB aa) {
-  const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  const int n = count ? min(*count, max_rows) : max_rows;
-  if (t >= n) return;
-  const float s0 = dots[t * 2] + bq[0], sv = dots[t * 2 + 1] + bv[0], s1 = dots2[t * 2] + bq[1];
-  const float mean = (s0 + s1) / 2.0f;
-  const float o0 = (s0 - mean) + sv, o1 = (s1 - mean) + sv;
-  int64_t orow;
-  if (out_mode == 0) orow = row0 + idx[t];
-  else if (out_mode == 1) orow = row0 / per_graph_N + idx[t] / per_graph_N;
-  else orow = t;
-  q_out[orow * 2 + 0] = o0;
-  q_out[orow * 2 + 1] = o1;
-  if (act_out && out_mode != 2) act_out[orow] = (int8_t)select_action_b(o0, o1, aa, (uint64_t)orow);
 }
 
 // Network without dueling heads: q = out_linear(latent) (l_dgn.py:88-90,149) on the bf16 latent rows.  One warp per row.
@@ -866,8 +822,8 @@ struct WsB {
   bf16 *t_h, *t_x0, *t_P;     // discrete-feature tables: [n_keys][hid], [n_keys][hid], [n_keys][nproj*HC]
   float* t_ab;                // [n_keys][2H]
   // ---- per pass
-  float* hd;                  // per-row output dots [T][4]
-  bf16 *h, *x0, *P, *x1, *z, *hid1, *hid2;
+  bf16 *h, *x0, *P, *x1, *z;
+  bf16 *hid1, *hid2;          // hidden layers of dueling heads that are not 128 wide (the fused head keeps them on chip)
   float* qg;
   int *idx, *slot, *count, *gfirst, *gcnt;
   int *nidx, *xrow, *ncount, *nfirst, *ncnt;   // needed rows (conv2 sources)
@@ -912,8 +868,8 @@ size_t carve_b(const MlsNetDesc* d, int Gc, unsigned char* base, WsB* ws) {
   const size_t o_th = take(KT * hid * 2), o_tx0 = take(KT * hid * 2), o_tP = take(KT * nproj * HC * 2), o_tab = take(KT * 2 * d->heads * 4);
   // per pass
   const size_t o_h = take(R * hid * 2), o_x0 = take(R * hid * 2), o_P = take(R * nproj * HC * 2);
-  const size_t o_x1 = take(hl ? 0 : R * HC * 2), o_z = take(T * latent * 2), o_h1 = take(T * hh2 * 2), o_h2 = take(T * hh2 * 2);
-  const size_t o_hd = take(T * 4 * 4);
+  const size_t hid_bytes = d->head_hidden == 128 ? 0 : T * hh2 * 2;
+  const size_t o_x1 = take(hl ? 0 : R * HC * 2), o_z = take(T * latent * 2), o_h1 = take(hid_bytes), o_h2 = take(hid_bytes);
   const size_t o_qg = take((size_t)Gc * 8), o_idx = take(R * 4), o_slot = take(R * 4), o_cnt = take(16);
   const bool c2 = !hl && conv2_attn_supported(d->n_nodes, d->heads);
   const size_t o_eabs = take(c2 ? R * 4 : 0), o_gmeta = take(c2 ? (size_t)Gc * 32 : 0);
@@ -934,7 +890,7 @@ size_t carve_b(const MlsNetDesc* d, int Gc, unsigned char* base, WsB* ws) {
     auto I = [&](size_t o) { return reinterpret_cast<int*>(base + o); };
     ws->w_enc1 = B(o_we); ws->w_c1 = B(o_wc1); ws->w_c2 = B(o_wc2); ws->w_h0 = B(o_wh0); ws->w_h1 = B(o_wh1);
     ws->b_c1 = F(o_bc1); ws->b_c2 = F(o_bc2); ws->b_h0 = F(o_bh0); ws->b_h1 = F(o_bh1);
-    ws->hv1 = F(o_hv1); ws->hv2 = F(o_hv2); ws->hd = F(o_hd);
+    ws->hv1 = F(o_hv1); ws->hv2 = F(o_hv2);
     ws->h = B(o_h); ws->x0 = B(o_x0); ws->P = B(o_P); ws->x1 = B(o_x1); ws->z = B(o_z); ws->hid1 = B(o_h1); ws->hid2 = B(o_h2);
     ws->qg = F(o_qg);
     ws->idx = I(o_idx); ws->slot = I(o_slot); ws->count = I(o_cnt); ws->ncount = I(o_cnt) + 1; ws->ecount = I(o_cnt) + 2; ws->ntotal = I(o_cnt) + 3;
@@ -1258,26 +1214,24 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
       prof_end(MLS_PROF_EDGE1);
     }
     if (!hl) {
-      // conv2 projections on x1 * dm (the row mask commutes with the GEMM, applied in its epilogue).  Source side
-      // (GATv2 x_l, Transformer k | v) on the needed rows; target side (GATv2 x_r, Transformer q) on the controlling
-      // nodes, whose x1 rows already sit compacted in z (snapshot).  fp16 outputs for the tensor-core attention.
+      // conv2 projections on x1 * dm (the row mask commutes with the GEMM, applied in its epilogue), both in one launch
+      // over the packed weight rows (Transformer [q; k; v], GATv2 [l; r]).  Source side (GATv2 x_l, Transformer k | v) on
+      // the needed rows; target side (GATv2 x_r, Transformer q) on the controlling nodes: x1[0 : count) itself
+      // (ctrl_first, the x1 tile is read once for both), else their snapshot columns of z.  fp16 outputs for the
+      // tensor-core attention.
       const int nsrc = nproj - 1;
       bf16* Psrc = ws.P;                                    // [needed rows][nsrc*HC]
       bf16* Ptgt = ws.P + (size_t)rows * nsrc * HC;         // [count][HC]
       float* dots_t = ws.ab + (size_t)rows * H;             // [count][H]
-      const bf16* w_src = tr ? ws.w_c2 + (size_t)HC * HC : ws.w_c2;            // weight rows: Transformer [q; k; v], GATv2 [l; r]
-      const bf16* w_tgt = tr ? ws.w_c2 : ws.w_c2 + (size_t)HC * HC;
-      const float* b_src = tr ? ws.b_c2 + HC : ws.b_c2;
-      const float* b_tgt = tr ? ws.b_c2 : ws.b_c2 + HC;
-      GemmEpilogue e{Psrc, nsrc * HC, b_src, obs, a->obs_stride, N, 0, tr ? nullptr : ws.att2, tr ? nullptr : ws.ab, ws.nidx};
+      GemmEpilogue e{Psrc, nsrc * HC, ws.b_c2, obs, a->obs_stride, N, 0, tr ? nullptr : ws.att2, tr ? nullptr : ws.ab, ws.nidx};
       e.c_fp16 = use_c2 ? 1 : 0;
+      e.Ct = Ptgt; e.ldct = HC; e.dots_t = tr ? nullptr : dots_t; e.row_index_t = ws.idx;
+      GemmShape sh{rows, nproj * HC, HC, ctrl_first ? ws.ntotal : ws.ncount};
+      sh.m_dev_t = ws.count; sh.t_lo = tr ? 0 : HC; sh.t_hi = sh.t_lo + HC;
+      if (!ctrl_first) { sh.A2 = ws.z + hid; sh.lda2 = latent; sh.k2_lo = 0; sh.k2_hi = HC; }
       prof_begin(MLS_PROF_PROJ2);
-      if ((rc = gemm_bf16_launch(ws.x1, HC, w_src, HC, GemmShape{rows, nsrc * HC, HC, ctrl_first ? ws.ntotal : ws.ncount}, e, sms, st))) return rc;
+      if ((rc = gemm_bf16_launch(ws.x1, HC, ws.w_c2, HC, sh, e, sms, st))) return rc;
       prof_end(MLS_PROF_PROJ2);
-      GemmEpilogue et{Ptgt, HC, b_tgt, obs, a->obs_stride, N, 0, tr ? nullptr : ws.att2, tr ? nullptr : dots_t, ws.idx};
-      et.c_fp16 = use_c2 ? 1 : 0;
-      // target side: the controlling nodes' relu(conv1) rows -- the snapshot columns of z, or x1[0 : count) itself (ctrl_first)
-      if ((rc = gemm_bf16_launch(ctrl_first ? ws.x1 : ws.z + hid, ctrl_first ? HC : latent, w_tgt, HC, GemmShape{rows, HC, HC, ws.count}, et, sms, st))) return rc;
       // conv2 attention only where a controlling agent reads it; the result goes straight into z
       prof_begin(MLS_PROF_EDGE2);
       if (use_c2) {
@@ -1317,37 +1271,33 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
         mls_count_launch(2);
       }
     } else {
-      GemmEpilogue e0{ws.hid1, hh2, ws.b_h0, nullptr, 0, N, 1, nullptr, nullptr};
-      prof_begin(MLS_PROF_HEAD0);
       GemmShape sh0{head_rows, hh2, latent, m_dev};
       if (ctrl_first) { sh0.A2 = ws.x1; sh0.lda2 = HC; sh0.k2_lo = hid; sh0.k2_hi = hid + HC; }   // snapshot columns come from x1
-      if ((rc = gemm_bf16_launch(ws.z, latent, ws.w_h0, latent, sh0, e0, sms, st))) return rc;
-      prof_end(MLS_PROF_HEAD0);
-      // last hidden layer: with 128-wide heads the output layer rides in the epilogue as three dot products per
-      // row and the hidden activations are never written
-      const bool fuse_out = hh == 128;
-      GemmEpilogue e1{fuse_out ? nullptr : ws.hid2, hh2, ws.b_h1, nullptr, 0, N, 1, nullptr, nullptr, nullptr, nullptr, nullptr, 0};
-      if (fuse_out) { e1.dotvec = ws.hv1; e1.dots = ws.hd; e1.dotvec2 = ws.hv2; e1.dots2 = ws.hd + (size_t)head_rows * 2; e1.dot_relu = 1; }
-      if ((rc = gemm_bf16_launch(ws.hid1, hh2, ws.w_h1, hh2, GemmShape{head_rows, hh2, hh2, m_dev}, e1, sms, st))) return rc;
-      const float* d1 = ws.hd;
-      const float* d2 = ws.hd + (size_t)head_rows * 2;
-      if (!hl) {
-        if (fuse_out)
-          head_final_kernel<<<(rows + 255) / 256, 256, 0, st>>>(d1, d2, ws.idx, ws.count, rows, w->q_b2, w->v_b2, (int64_t)g0 * N, N, a->q,
-                                                               a->act, a->ctrl_mode, aa);
-        else
+      prof_begin(MLS_PROF_HEAD0);
+      if (hh == 128) {
+        // both hidden layers, the output layer and the action in one kernel: the hidden activations stay on chip
+        HeadOut ho{w->q_b2, w->v_b2, hl ? nullptr : ws.idx, hl ? 0 : (int64_t)g0 * N, N, hl ? ws.qg : a->q, hl ? nullptr : a->act,
+                   hl ? 2 : a->ctrl_mode, aa};
+        if ((rc = head_dueling_launch(ws.z, latent, sh0, ws.w_h0, ws.w_h1, HeadVecs{ws.b_h0, ws.b_h1, ws.hv1, ws.hv2}, ho, sms, st))) return rc;
+        prof_end(MLS_PROF_HEAD0);
+      } else {
+        GemmEpilogue e0{ws.hid1, hh2, ws.b_h0, nullptr, 0, N, 1, nullptr, nullptr};
+        if ((rc = gemm_bf16_launch(ws.z, latent, ws.w_h0, latent, sh0, e0, sms, st))) return rc;
+        prof_end(MLS_PROF_HEAD0);
+        GemmEpilogue e1{ws.hid2, hh2, ws.b_h1, nullptr, 0, N, 1, nullptr, nullptr};
+        if ((rc = gemm_bf16_launch(ws.hid1, hh2, ws.w_h1, hh2, GemmShape{head_rows, hh2, hh2, m_dev}, e1, sms, st))) return rc;
+        if (!hl)
           head_out_bf16_kernel<<<(rows * 32 + 255) / 256, 256, 0, st>>>(ws.hid2, hh, ws.idx, ws.count, rows, w->q_w2, w->q_b2, w->v_w2,
                                                                          w->v_b2, (int64_t)g0 * N, N, a->q, a->act, a->ctrl_mode, aa);
-        mls_count_launch();
-      } else {
-        if (fuse_out)
-          head_final_kernel<<<(gc + 255) / 256, 256, 0, st>>>(d1, d2, nullptr, nullptr, gc, w->q_b2, w->v_b2, 0, N, ws.qg, nullptr, 2, aa);
         else
           head_out_bf16_kernel<<<(gc * 32 + 255) / 256, 256, 0, st>>>(ws.hid2, hh, nullptr, nullptr, gc, w->q_w2, w->q_b2, w->v_w2,
                                                                        w->v_b2, 0, N, ws.qg, nullptr, 2, aa);
+        mls_count_launch();
+      }
+      if (hl) {
         const long long nthr = a->ctrl_mode == 1 ? gc : (long long)gc * N;
         hl_scatter_b_kernel<<<(unsigned)((nthr + 255) / 256), 256, 0, st>>>(ws.qg, cm, N, gc, g0, a->ctrl_mode, a->q, a->act, aa);
-        mls_count_launch(2);
+        mls_count_launch();
       }
     }
     MLS_LAUNCH_CHECK();

@@ -71,4 +71,53 @@ __device__ __forceinline__ void radius_neighbours(const float* __restrict__ g_ob
   for (int w = 0; w < W; ++w) if (w == (i >> 5)) nb[w] &= ~(1u << (i & 31));
 }
 
+struct ActArgsB {
+  float eps;
+  uint64_t seed, offset;
+  const double* rand3;
+  const unsigned long long* offset_dev;   // optional device-side addend (round counter under CUDA-graph replay)
+  uint64_t row0;                          // added to the row index that keys the Philox draw (sub-batch calls)
+};
+__device__ __forceinline__ int select_action_b(float q0, float q1, const ActArgsB& a, uint64_t row) {
+  int act = q1 > q0 ? 1 : 0;
+  if (fabsf(a.eps) > 1e-8f) {
+    double ue, u0, u1;
+    if (a.rand3) { ue = a.rand3[row * 3 + 0]; u0 = a.rand3[row * 3 + 1]; u1 = a.rand3[row * 3 + 2]; }
+    else {
+      Philox4 r = philox4x32_10(a.seed, row + a.row0, a.offset + (a.offset_dev ? *a.offset_dev : 0ull));
+      ue = u01_from_u32x2(r.v[0], r.v[1]);
+      u0 = (double)r.v[2] * (1.0 / 4294967296.0);
+      u1 = (double)r.v[3] * (1.0 / 4294967296.0);
+    }
+    if (ue < (double)a.eps) act = (u1 + 1.0) > (u0 + 1.0) ? 1 : 0;
+  }
+  return act;
+}
+
+// Output layer of the 128-wide dueling heads for one row t, from the three dot products of its rectified last hidden layer
+// (d_q0 = <relu(hq), wq[0]>, d_v = <relu(hv), wv>, d_q1 = <relu(hq), wq[1]>): biases, dueling combination, output row
+// mapping and action.  Same outputs as head_out_bf16_kernel.
+struct HeadOut {
+  const float *bq, *bv;
+  const int* idx;             // out_mode 0 / 1: row t is node row idx[t] of the pass
+  int64_t row0;               // first node row of the pass (out_mode 0 / 1)
+  int per_graph_N;
+  float* q_out;
+  int8_t* act_out;
+  int out_mode;               // 0: per node row, 1: per graph (of the node row), 2: row t (HL-DGN graph rows, no action)
+  ActArgsB aa;
+};
+__device__ __forceinline__ void head_final_row(int t, float d_q0, float d_v, float d_q1, const HeadOut& h) {
+  const float s0 = d_q0 + h.bq[0], sv = d_v + h.bv[0], s1 = d_q1 + h.bq[1];
+  const float mean = (s0 + s1) / 2.0f;
+  const float o0 = (s0 - mean) + sv, o1 = (s1 - mean) + sv;
+  int64_t orow;
+  if (h.out_mode == 0) orow = h.row0 + h.idx[t];
+  else if (h.out_mode == 1) orow = h.row0 / h.per_graph_N + h.idx[t] / h.per_graph_N;
+  else orow = t;
+  h.q_out[orow * 2 + 0] = o0;
+  h.q_out[orow * 2 + 1] = o1;
+  if (h.act_out && h.out_mode != 2) h.act_out[orow] = (int8_t)select_action_b(o0, o1, h.aa, (uint64_t)orow);
+}
+
 }  // namespace mls

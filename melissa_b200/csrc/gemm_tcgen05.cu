@@ -33,6 +33,8 @@ struct GemmSmem {
 // MODE fixes the epilogue options at compile time for the hot launches (0 = read them from `epi` at run time):
 //   1 = one dot vector on the raw values, C written (GATv2 projections)   2 = ReLU, C written, no dots (hidden layers)
 //   3 = ReLU + two dot vectors on the rectified values, C not written (last hidden layer with the output layer fused)
+//   4 = split launch (GemmShape::t_lo): both conv2 projections, one dot vector per segment (GATv2)
+//   5 = split launch without dots (TransformerConv)
 // The epilogue bounds the tile rate, and the run-time selects were a fifth of its instructions.
 template <int BN, int MODE>
 __global__ void __launch_bounds__(kGemmThreads, 1)
@@ -54,11 +56,31 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
   auto tempty_bar = [&](int a) { return bar0 + 8u * (2 * kStages + 2 + a); };
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  constexpr bool kSplit = MODE >= 4;
   int M = shape.M;
   if (shape.m_dev) M = min(M, *shape.m_dev);
   const int n_m = (M + kBM - 1) / kBM, n_n = shape.N / BN;
-  const int n_tiles = n_m * n_n;
+  // split launch: the M tiles holding target rows take every column tile, the ones past them the source column tiles only
+  // (N tiles of one M tile stay adjacent, so the A tile is read from HBM once)
+  int Mt = 0, n_mt = 0, n_ns = 0;
+  const int t_w = shape.t_hi - shape.t_lo;
+  if (kSplit) {
+    Mt = shape.m_dev_t ? min(shape.M, *shape.m_dev_t) : shape.M;
+    n_mt = (Mt + kBM - 1) / kBM;
+    n_ns = (shape.N - t_w) / BN;
+  }
+  const int n_tiles = kSplit ? n_mt * n_n + max(n_m - n_mt, 0) * n_ns : n_m * n_n;
   const int n_kb = shape.K / kBK;
+  // tile -> first row, first (packed) column; true for a target column tile
+  auto tile_at = [&](int tile, int& m0, int& n0) -> bool {
+    if (!kSplit || tile < n_mt * n_n) { m0 = (tile / n_n) * kBM; n0 = (tile % n_n) * BN; return kSplit && n0 >= shape.t_lo && n0 < shape.t_hi; }
+    else {
+      const int t = tile - n_mt * n_n;
+      m0 = (n_mt + t / n_ns) * kBM; n0 = (t % n_ns) * BN;
+      if (n0 >= shape.t_lo) n0 += t_w;
+      return false;
+    }
+  };
 
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&tmA);
@@ -81,12 +103,14 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       int stage = 0;
       uint32_t phase = 0;
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const int m0 = (tile / n_n) * kBM, n0 = (tile % n_n) * BN;
+        int m0, n0;
+        const bool tgt = tile_at(tile, m0, n0);
         for (int kb = 0; kb < n_kb; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1);
           const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
           mbar_expect_tx(full_bar(stage), S::kStageBytes);
-          if (kb * kBK >= shape.k2_lo && kb * kBK < shape.k2_hi) tma_load_2d(sa, &tmA2, full_bar(stage), kb * kBK - shape.k2_lo, m0);
+          if ((!kSplit || tgt) && kb * kBK >= shape.k2_lo && kb * kBK < shape.k2_hi)
+            tma_load_2d(sa, &tmA2, full_bar(stage), kb * kBK - shape.k2_lo, m0);
           else tma_load_2d(sa, &tmA, full_bar(stage), kb * kBK, m0);
           tma_load_2d(sa + S::kABytes, &tmB, full_bar(stage), kb * kBK, n0);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
@@ -126,7 +150,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     // sixteen warps (the epilogue, not the MMA, bounds the tile rate with fewer): warp % 4 selects the TMEM lane quarter
     // (rows) a warp may read, (warp - 4) / 4 the column quarter
     const int ew = (warp - 4) & 3, half = (warp - 4) >> 2;
-    const bool has_dot = MODE == 0 ? epi.dotvec != nullptr : (MODE == 1 || MODE == 3);
+    const bool has_dot = MODE == 0 ? epi.dotvec != nullptr : (MODE == 1 || MODE == 3 || MODE == 4);
     const bool has_dot2 = MODE == 0 ? epi.dotvec2 != nullptr : MODE == 3;
     const bool dot_relu = MODE == 0 ? epi.dot_relu != 0 : MODE == 3;
     const bool relu = MODE == 0 ? epi.relu != 0 : (MODE == 2 || MODE == 3);
@@ -145,7 +169,8 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     // column slices (bias, dot vectors) of `tile` -> buffer `buf`, asynchronously
     auto fill = [&](int buf, int tile) {
       if (tile >= n_tiles) return;
-      const int fn0 = (tile % n_n) * BN;
+      int fm0, fn0;
+      tile_at(tile, fm0, fn0);
       for (int c = et; c < BN; c += kGemmEpiWarps * 32) {
         if (epi.bias) cp4(bias_s + buf * BN + c, epi.bias + fn0 + c);
         else bias_s[buf * BN + c] = 0.0f;
@@ -156,9 +181,12 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     // row scale of this thread's row in `tile`: node row index (one tile ahead), then the observation's dm flag
     auto ld_index = [&](int tile) -> int {
       if (!epi.obs || tile >= n_tiles) return -1;
-      const int rr = (tile / n_n) * kBM + ew * 32 + lane;
-      if (rr >= M) return -1;
-      return epi.row_index ? __ldg(epi.row_index + rr) : rr;
+      int tm0, tn0;
+      const bool tgt = tile_at(tile, tm0, tn0);
+      const int rr = tm0 + ew * 32 + lane;
+      if (rr >= (tgt ? Mt : M)) return -1;
+      const int* ri = tgt ? epi.row_index_t : epi.row_index;
+      return ri ? __ldg(ri + rr) : rr;
     };
     auto ld_scale = [&](int nr) -> float {
       if (nr < 0) return 1.0f;
@@ -173,7 +201,15 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
       const int acc = it & 1;
       const uint32_t acc_phase = (it >> 1) & 1;
-      const int m0 = (tile / n_n) * kBM, n0 = (tile % n_n) * BN;
+      int m0, n0;
+      const bool tgt = tile_at(tile, m0, n0);
+      // output segment of this column tile: C / dots with the source columns packed left, or the target segment
+      const int Mr = !kSplit ? M : tgt ? Mt : M;
+      const int oc0 = !kSplit ? n0 : tgt ? n0 - shape.t_lo : (n0 >= shape.t_hi ? n0 - t_w : n0);
+      const int n_grp = !kSplit ? shape.N >> 7 : (tgt ? t_w : shape.N - t_w) >> 7;
+      __nv_bfloat16* const Cseg = !kSplit ? epi.C : tgt ? epi.Ct : epi.C;
+      const int ldc = !kSplit ? epi.ldc : tgt ? epi.ldct : epi.ldc;
+      float* const dots_seg = !kSplit ? epi.dots : tgt ? epi.dots_t : epi.dots;
       const int r = m0 + ew * 32 + lane;
       const float scale = scale_cur;
       // software pipeline: the next tile's scale (its index arrived during the previous tile) and the index after that
@@ -209,7 +245,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
             }
           }
           if (relu) { x0 = fmaxf(x0, 0.f); x1 = fmaxf(x1, 0.f); x2 = fmaxf(x2, 0.f); x3 = fmaxf(x3, 0.f); }
-          if (has_cf && r < M)                                // lane = row: 16-byte stores, 128 contiguous bytes per lane and chunk
+          if (has_cf && r < Mr)                                // lane = row: 16-byte stores, 128 contiguous bytes per lane and chunk
             *reinterpret_cast<float4*>(epi.Cf + (size_t)r * epi.ldcf + n0 + c0 + j) = make_float4(x0, x1, x2, x3);
           if (!has_c) {
           } else if (epi.c_fp16) {
@@ -229,9 +265,9 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         if (has_dot && (c0 & 32) == 32) {                 // end of this warp's half (64 columns) of a 128-column group
           // the group's two halves come from two warps: two atomic adds onto a zeroed cell (launcher) -- with exactly two
           // terms the sum does not depend on their order (0 + x + y == 0 + y + x), so the result is deterministic
-          if (r < M) {
-            atomicAdd(epi.dots + (size_t)r * (shape.N >> 7) + ((n0 + c0) >> 7), dot);
-            if (has_dot2) atomicAdd(epi.dots2 + (size_t)r * (shape.N >> 7) + ((n0 + c0) >> 7), dot2);
+          if (r < Mr) {
+            atomicAdd(dots_seg + (size_t)r * n_grp + ((oc0 + c0) >> 7), dot);
+            if (has_dot2) atomicAdd(epi.dots2 + (size_t)r * n_grp + ((oc0 + c0) >> 7), dot2);
           }
           dot = 0.f; dot2 = 0.f;
         }
@@ -246,13 +282,13 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       const int sub = lane / kLanesPerRow, cl = lane % kLanesPerRow;
       if (has_c) {
         const int gr0 = m0 + ew * 32 + sub;
-        __nv_bfloat16* crow = epi.C + (size_t)gr0 * epi.ldc + n0 + cb + cl * 8;
-        const size_t cstep = (size_t)kRowsPerIter * epi.ldc;
+        __nv_bfloat16* crow = Cseg + (size_t)gr0 * ldc + oc0 + cb + cl * 8;
+        const size_t cstep = (size_t)kRowsPerIter * ldc;
         const unsigned char* srow = stage_out + sub * S::kOutRowBytes + cl * 16;
 #pragma unroll 4
         for (int rr = 0; rr < 32; rr += kRowsPerIter) {
           const uint4 val = *reinterpret_cast<const uint4*>(srow + rr * S::kOutRowBytes);
-          if (gr0 + rr < M) *reinterpret_cast<uint4*>(crow) = val;
+          if (gr0 + rr < Mr) *reinterpret_cast<uint4*>(crow) = val;
           crow += cstep;
         }
       }
@@ -265,6 +301,233 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc(tmem_base, 2 * BN);
+}
+
+// ------------------------------------------------------------------------------ fused dueling heads (128-wide hidden layers)
+// Per 128-row tile: head0 = A @ W_h0^T (K = latent) into TMEM; epilogue phase 1 drains it to relu(. + b_h0) in bf16 (MODE 2's
+// rounding) and writes it into shared memory as the K-major, 128B-swizzled A operand of head1; head1 = hid @ W_h1^T (the
+// block-diagonal [Q1 0; 0 V1], K = 256, four B-only K-blocks through the stage ring) reuses the tile's accumulator; phase 2
+// forms MODE 3's two dot products per 64-column quarter, the quarters meet in shared memory, and head_final_row writes Q
+// and the action.  Neither the hidden activations nor the dots touch global memory.
+// The MMA thread issues head0 of the next tile before head1 of this one, so the stage ring keeps streaming A rows from
+// HBM while the epilogue builds the hidden tile.
+struct HeadSmem {
+  static constexpr int kStages = 3;
+  static constexpr int kN = 256;                                   // [Q hidden | V hidden]
+  static constexpr int kABytes = kBM * kBK * 2;                    // 16 KiB
+  static constexpr int kBBytes = kN * kBK * 2;                     // 32 KiB
+  static constexpr int kStageBytes = kABytes + kBBytes;
+  static constexpr int kHidOffset = kStages * kStageBytes;        // hidden tile: kN / kBK K-blocks of 128 x 64 bf16
+  static constexpr int kVecOffset = kHidOffset + (kN / kBK) * kABytes;   // b_h0, b_h1, hv1, hv2 (kN floats each)
+  static constexpr int kPartOffset = kVecOffset + 4 * kN * 4;      // dot partials, double buffered: [2][4 quarters][128 rows] float2
+  static constexpr int kBarOffset = kPartOffset + 2 * 4 * kBM * 8;
+  static constexpr int kTotal = kBarOffset + 256 + 1024;           // barriers + alignment slack
+};
+static_assert(HeadSmem::kTotal <= 232448, "fused head shared memory");
+
+__global__ void __launch_bounds__(kGemmThreads, 1)
+head_dueling_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                            const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmB1,
+                            const GemmShape shape, const HeadVecs vec, const HeadOut out) {
+  using S = HeadSmem;
+  constexpr int kStages = S::kStages, kN = S::kN, kKb1 = kN / kBK;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + S::kBarOffset);
+  // bars[0..S) full, [S..2S) empty, [2S..2S+2) tmem_full, [2S+2..2S+4) tmem_empty, 2S+4 hid_full, 2S+5 hid_empty, 2S+6 out_full
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 7);
+  const uint32_t bar0 = smem_u32(bars);
+  auto full_bar = [&](int s) { return bar0 + 8u * s; };
+  auto empty_bar = [&](int s) { return bar0 + 8u * (kStages + s); };
+  auto tfull_bar = [&](int a) { return bar0 + 8u * (2 * kStages + a); };
+  auto tempty_bar = [&](int a) { return bar0 + 8u * (2 * kStages + 2 + a); };
+  const uint32_t hfull_bar = bar0 + 8u * (2 * kStages + 4), hempty_bar = bar0 + 8u * (2 * kStages + 5);
+  const uint32_t ofull_bar = bar0 + 8u * (2 * kStages + 6);
+  unsigned char* hid = smem + S::kHidOffset;
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  int M = shape.M;
+  if (shape.m_dev) M = min(M, *shape.m_dev);
+  const int n_tiles = (M + kBM - 1) / kBM;
+  const int n_it = (int)blockIdx.x < n_tiles ? (n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+  const int n_kb = shape.K / kBK;
+
+  if (warp == 0 && lane == 0) {
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmB);
+    prefetch_tmap(&tmB1);
+  }
+  if (warp == 1 && lane == 0) {
+    for (int s = 0; s < kStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
+    for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), kGemmEpiWarps * 32); }
+    mbar_init(hfull_bar, kGemmEpiWarps * 32);
+    mbar_init(hempty_bar, 1);
+    mbar_init(ofull_bar, 1);
+    fence_barrier_init();
+  }
+  if (warp == 2) tmem_alloc(smem_u32(tmem_slot), 2 * kN);        // 2 accumulator stages; head1 reuses its tile's stage
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+
+  if (warp == 0) {
+    // ===================================================================== TMA producer (same order as the MMA thread)
+    if (lane == 0) {
+      int stage = 0;
+      uint32_t phase = 0;
+      auto load_head0 = [&](int it) {
+        const int m0 = (blockIdx.x + it * gridDim.x) * kBM;
+        for (int kb = 0; kb < n_kb; ++kb) {
+          mbar_wait(empty_bar(stage), phase ^ 1);
+          const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
+          mbar_expect_tx(full_bar(stage), S::kStageBytes);
+          if (kb * kBK >= shape.k2_lo && kb * kBK < shape.k2_hi) tma_load_2d(sa, &tmA2, full_bar(stage), kb * kBK - shape.k2_lo, m0);
+          else tma_load_2d(sa, &tmA, full_bar(stage), kb * kBK, m0);
+          tma_load_2d(sa + S::kABytes, &tmB, full_bar(stage), kb * kBK, 0);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+      };
+      auto load_head1 = [&]() {
+        for (int kb = 0; kb < kKb1; ++kb) {
+          mbar_wait(empty_bar(stage), phase ^ 1);
+          const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
+          mbar_expect_tx(full_bar(stage), S::kBBytes);
+          tma_load_2d(sa + S::kABytes, &tmB1, full_bar(stage), kb * kBK, 0);
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+      };
+      if (n_it > 0) load_head0(0);
+      for (int it = 0; it < n_it; ++it) {
+        if (it + 1 < n_it) load_head0(it + 1);
+        load_head1();
+      }
+    }
+  } else if (warp == 1) {
+    // ===================================================================== MMA issuer (one thread)
+    if (lane == 0) {
+      constexpr uint32_t idesc = make_idesc(kBM, kN);
+      int stage = 0;
+      uint32_t phase = 0;
+      auto mma_head0 = [&](int it) {
+        const int acc = it & 1;
+        mbar_wait(tempty_bar(acc), ((it >> 1) & 1) ^ 1);    // phase 2 of the tile two back has drained this accumulator
+        tc_fence_after();
+        const uint32_t d_tmem = tmem_base + (uint32_t)(acc * kN);
+        for (int kb = 0; kb < n_kb; ++kb) {
+          mbar_wait(full_bar(stage), phase);
+          tc_fence_after();
+          const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
+          const uint64_t da = make_smem_desc(sa), db = make_smem_desc(sa + S::kABytes);
+#pragma unroll
+          for (int k = 0; k < kBK / kUmmaK; ++k)
+            umma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, (kb | k) ? 1u : 0u);
+          umma_commit(empty_bar(stage));
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit(tfull_bar(acc));
+      };
+      auto mma_head1 = [&](int it) {
+        const uint32_t d_tmem = tmem_base + (uint32_t)((it & 1) * kN);
+        mbar_wait(hfull_bar, it & 1);                        // phase 1 has drained the accumulator and written the hidden tile
+        tc_fence_after();
+        for (int kb = 0; kb < kKb1; ++kb) {
+          mbar_wait(full_bar(stage), phase);
+          tc_fence_after();
+          const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
+          const uint64_t da = make_smem_desc(smem_u32(hid + kb * S::kABytes)), db = make_smem_desc(sa + S::kABytes);
+#pragma unroll
+          for (int k = 0; k < kBK / kUmmaK; ++k)
+            umma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, (kb | k) ? 1u : 0u);
+          umma_commit(empty_bar(stage));
+          if (++stage == kStages) { stage = 0; phase ^= 1; }
+        }
+        umma_commit(hempty_bar);                             // the hidden tile may be overwritten
+        umma_commit(ofull_bar);                              // head1 accumulator complete -> phase 2
+      };
+      if (n_it > 0) mma_head0(0);
+      for (int it = 0; it < n_it; ++it) {
+        if (it + 1 < n_it) mma_head0(it + 1);
+        mma_head1(it);
+      }
+    }
+  } else if (warp >= 4) {
+    // ===================================================================== epilogue
+    // warp % 4 selects the TMEM lane quarter (rows), (warp - 4) / 4 the 64-column quarter = one K-block of the hidden tile
+    const int ew = (warp - 4) & 3, quarter = (warp - 4) >> 2;
+    const int cb = quarter * 64;
+    const int et = threadIdx.x - 128;
+    float* b0_s = reinterpret_cast<float*>(smem + S::kVecOffset);
+    float* b1_s = b0_s + kN;
+    float* v1_s = b1_s + kN;
+    float* v2_s = v1_s + kN;
+    float2* part_s = reinterpret_cast<float2*>(smem + S::kPartOffset);
+    for (int c = et; c < kN; c += kGemmEpiWarps * 32) {
+      b0_s[c] = vec.b_h0[c]; b1_s[c] = vec.b_h1[c]; v1_s[c] = vec.hv1[c]; v2_s[c] = vec.hv2[c];
+    }
+    asm volatile("bar.sync 1, 512;" ::: "memory");
+    const int row = ew * 32 + lane;
+    unsigned char* hrow = hid + quarter * S::kABytes + row * 128;
+    for (int it = 0; it < n_it; ++it) {
+      const int acc = it & 1;
+      const int m0 = (blockIdx.x + it * gridDim.x) * kBM;
+      const uint32_t t_acc = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)(acc * kN);
+      // ---- phase 1: relu(head0 + b_h0) -> bf16 -> hidden tile (128B swizzle: 16-byte chunk index ^ row % 8)
+      mbar_wait(tfull_bar(acc), (it >> 1) & 1);
+      mbar_wait(hempty_bar, (it & 1) ^ 1);                   // head1 of the previous tile has read the hidden tile
+      tc_fence_after();
+#pragma unroll 1
+      for (int c0 = cb; c0 < cb + 64; c0 += 32) {
+        uint32_t v[32];
+        tmem_ld32(t_acc + (uint32_t)c0, v);
+        uint32_t packed[16];
+#pragma unroll
+        for (int j = 0; j < 32; j += 2) {
+          const float x0 = fmaxf(fmaf(__uint_as_float(v[j]), 1.0f, b0_s[c0 + j]), 0.f);
+          const float x1 = fmaxf(fmaf(__uint_as_float(v[j + 1]), 1.0f, b0_s[c0 + j + 1]), 0.f);
+          __nv_bfloat162 p = __floats2bfloat162_rn(x0, x1);
+          packed[j >> 1] = *reinterpret_cast<uint32_t*>(&p);
+        }
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const int ch = ((c0 - cb) >> 3) + q;
+          *reinterpret_cast<uint4*>(hrow + ((ch ^ (row & 7)) << 4)) =
+              make_uint4(packed[4 * q], packed[4 * q + 1], packed[4 * q + 2], packed[4 * q + 3]);
+        }
+      }
+      fence_proxy_async();                                   // generic-proxy stores -> visible to the tensor core
+      tc_fence_before();
+      mbar_arrive(hfull_bar);
+      // ---- phase 2: relu(head1 + b_h1), MODE 3's two dot products over this warp's 64 columns
+      mbar_wait(ofull_bar, it & 1);
+      tc_fence_after();
+      float dot = 0.f, dot2 = 0.f;
+#pragma unroll 1
+      for (int c0 = cb; c0 < cb + 64; c0 += 32) {
+        uint32_t v[32];
+        tmem_ld32(t_acc + (uint32_t)c0, v);
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          const float y = fmaxf(fmaf(__uint_as_float(v[j]), 1.0f, b1_s[c0 + j]), 0.f);
+          dot = fmaf(y, v1_s[c0 + j], dot);
+          dot2 = fmaf(y, v2_s[c0 + j], dot2);
+        }
+      }
+      tc_fence_before();
+      mbar_arrive(tempty_bar(acc));
+      float2* part = part_s + (it & 1) * 4 * kBM;
+      part[quarter * kBM + row] = make_float2(dot, dot2);
+      asm volatile("bar.sync 1, 512;" ::: "memory");
+      if (quarter == 0 && m0 + row < M) {
+        // a 128-column group is two quarters: (0 + x) + y is the value the GEMM's two atomic adds onto a zeroed cell give
+        const float2 p0 = part[row], p1 = part[kBM + row], p2 = part[2 * kBM + row], p3 = part[3 * kBM + row];
+        head_final_row(m0 + row, (0.f + p0.x) + p1.x, (0.f + p2.x) + p3.x, (0.f + p0.y) + p1.y, out);
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) tmem_dealloc(tmem_base, 2 * S::kN);
 }
 
 // ------------------------------------------------------------------------------ host side
@@ -298,6 +561,17 @@ int make_tmap_bf16(CUtensorMap* tm, const void* base, int rows, int cols, int ld
   return MLS_OK;
 }
 
+// A (and the optional second A matrix of a K range) -> TMA descriptors; clears the K range when there is no A2
+static int make_a_tmaps(const __nv_bfloat16* A, int lda, GemmShape& shape, CUtensorMap* ta, CUtensorMap* ta2) {
+  int rc = make_tmap_bf16(ta, A, shape.M, shape.K, lda, kBM);
+  if (rc) return rc;
+  *ta2 = *ta;
+  if (!shape.A2) { shape.k2_lo = shape.k2_hi = 0; return MLS_OK; }
+  MLS_CHECK_ARG(shape.k2_lo % kBK == 0 && shape.k2_hi % kBK == 0 && shape.k2_lo >= 0 && shape.k2_lo < shape.k2_hi && shape.k2_hi <= shape.K && shape.lda2 % 8 == 0,
+                "GEMM second A matrix: K range must be multiples of %d inside [0, K)", kBK);
+  return make_tmap_bf16(ta2, shape.A2, shape.M, shape.k2_hi - shape.k2_lo, shape.lda2, kBM);
+}
+
 size_t gemm_smem_bytes(int BN) { return BN == 256 ? GemmSmem<256>::kTotal : GemmSmem<128>::kTotal; }
 
 template <int BN, int MODE>
@@ -322,29 +596,32 @@ int gemm_bf16_launch(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, in
   MLS_CHECK_ARG(shape.N % 128 == 0, "GEMM N must be a multiple of 128 (got %d)", shape.N);
   MLS_CHECK_ARG(lda % 8 == 0 && ldb % 8 == 0 && (!epi.C || epi.ldc % 8 == 0), "GEMM leading dimensions must be multiples of 8 elements");
   MLS_CHECK_ARG(!epi.Cf || (epi.ldcf % 4 == 0 && (reinterpret_cast<uintptr_t>(epi.Cf) & 15) == 0), "fp32 GEMM output must be 16-byte aligned");
-  MLS_CHECK_ARG(!epi.dotvec || shape.N % 256 == 0, "the fused per-group dot products need N to be a multiple of 256");
+  const bool split = shape.t_lo < shape.t_hi;
+  const int BN = (shape.N % 256 == 0 && shape.t_lo % 256 == 0 && shape.t_hi % 256 == 0) ? 256 : 128;
+  MLS_CHECK_ARG(!epi.dotvec || BN == 256, "the fused per-group dot products need N (and a split's bounds) to be multiples of 256");
+  if (split) {
+    MLS_CHECK_ARG(shape.t_lo % 128 == 0 && shape.t_hi % 128 == 0 && shape.t_hi - shape.t_lo < shape.N &&
+                      (shape.t_lo == 0 || shape.t_hi == shape.N) && shape.t_lo >= 0 && shape.t_hi <= shape.N && epi.C && epi.Ct &&
+                      epi.ldct % 8 == 0 && !epi.Cf && !epi.relu && !epi.dotvec2 && (!epi.dotvec || epi.dots_t),
+                  "split GEMM: the target columns must be a 128-aligned prefix or suffix of N with both outputs given");
+  } else {
+    shape.t_lo = shape.t_hi = 0;
+  }
   if (shape.M <= 0) return MLS_OK;
   if (epi.dotvec) {                                         // the epilogue accumulates two partial sums per cell
-    MLS_CUDA(cudaMemsetAsync(epi.dots, 0, (size_t)shape.M * (shape.N >> 7) * sizeof(float), st));
+    const int t_w = shape.t_hi - shape.t_lo;
+    MLS_CUDA(cudaMemsetAsync(epi.dots, 0, (size_t)shape.M * ((shape.N - t_w) >> 7) * sizeof(float), st));
+    if (split) MLS_CUDA(cudaMemsetAsync(epi.dots_t, 0, (size_t)shape.M * (t_w >> 7) * sizeof(float), st));
     if (epi.dotvec2) MLS_CUDA(cudaMemsetAsync(epi.dots2, 0, (size_t)shape.M * (shape.N >> 7) * sizeof(float), st));
   }
-  const int BN = (shape.N % 256 == 0) ? 256 : 128;
-  CUtensorMap ta, tb;
-  int rc = make_tmap_bf16(&ta, A, shape.M, shape.K, lda, kBM);
+  CUtensorMap ta, tb, ta2;
+  int rc = make_a_tmaps(A, lda, shape, &ta, &ta2);
   if (rc) return rc;
   rc = make_tmap_bf16(&tb, B, shape.N, shape.K, ldb, BN);
   if (rc) return rc;
-  CUtensorMap ta2 = ta;
-  if (shape.A2) {
-    MLS_CHECK_ARG(shape.k2_lo % kBK == 0 && shape.k2_hi % kBK == 0 && shape.k2_lo >= 0 && shape.k2_lo < shape.k2_hi && shape.k2_hi <= shape.K && shape.lda2 % 8 == 0,
-                  "GEMM second A matrix: K range must be multiples of %d inside [0, K)", kBK);
-    rc = make_tmap_bf16(&ta2, shape.A2, shape.M, shape.k2_hi - shape.k2_lo, shape.lda2, kBM);
-    if (rc) return rc;
-  } else {
-    shape.k2_lo = shape.k2_hi = 0;
-  }
   int mode = 0;
-  if (!epi.Cf) {
+  if (split) mode = epi.dotvec ? 4 : 5;
+  else if (!epi.Cf) {
     if (epi.C && epi.dotvec && !epi.dotvec2 && !epi.dot_relu && !epi.relu) mode = 1;
     else if (epi.C && !epi.dotvec && epi.relu) mode = 2;
     else if (!epi.C && epi.dotvec && epi.dotvec2 && epi.dot_relu && epi.relu) mode = 3;
@@ -354,10 +631,35 @@ int gemm_bf16_launch(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, in
       case 1: return launch_bn<256, 1>(ta, tb, ta2, shape, epi, sm_count, st);
       case 2: return launch_bn<256, 2>(ta, tb, ta2, shape, epi, sm_count, st);
       case 3: return launch_bn<256, 3>(ta, tb, ta2, shape, epi, sm_count, st);
+      case 4: return launch_bn<256, 4>(ta, tb, ta2, shape, epi, sm_count, st);
+      case 5: return launch_bn<256, 5>(ta, tb, ta2, shape, epi, sm_count, st);
       default: return launch_bn<256, 0>(ta, tb, ta2, shape, epi, sm_count, st);
     }
   }
+  if (mode == 5) return launch_bn<128, 5>(ta, tb, ta2, shape, epi, sm_count, st);
   return launch_bn<128, 0>(ta, tb, ta2, shape, epi, sm_count, st);
+}
+
+int head_dueling_launch(const __nv_bfloat16* A, int lda, GemmShape shape, const __nv_bfloat16* w_h0, const __nv_bfloat16* w_h1,
+                        const HeadVecs& vec, const HeadOut& out, int sm_count, cudaStream_t st) {
+  MLS_CHECK_ARG(shape.N == HeadSmem::kN && shape.K % kBK == 0 && shape.K >= kBK && lda % 8 == 0,
+                "fused dueling heads: N must be %d and K a multiple of %d", HeadSmem::kN, kBK);
+  if (shape.M <= 0) return MLS_OK;
+  CUtensorMap ta, ta2, tb, tb1;
+  int rc = make_a_tmaps(A, lda, shape, &ta, &ta2);
+  if (rc) return rc;
+  if ((rc = make_tmap_bf16(&tb, w_h0, HeadSmem::kN, shape.K, shape.K, HeadSmem::kN))) return rc;
+  if ((rc = make_tmap_bf16(&tb1, w_h1, HeadSmem::kN, HeadSmem::kN, HeadSmem::kN, HeadSmem::kN))) return rc;
+  static bool configured = false;
+  if (!configured) {
+    MLS_CUDA(cudaFuncSetAttribute(head_dueling_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, HeadSmem::kTotal));
+    configured = true;
+  }
+  const int n_tiles = (shape.M + kBM - 1) / kBM;
+  head_dueling_tcgen05_kernel<<<n_tiles < sm_count ? n_tiles : sm_count, kGemmThreads, HeadSmem::kTotal, st>>>(ta, tb, ta2, tb1, shape, vec, out);
+  mls_count_launch();
+  MLS_LAUNCH_CHECK();
+  return MLS_OK;
 }
 
 }  // namespace mls
@@ -387,4 +689,41 @@ extern "C" int mls_test_gemm_bf16_ex(const void* A, const void* B, const float* 
                         dot_relu};
   return mls::gemm_bf16_launch(reinterpret_cast<const __nv_bfloat16*>(A), K, reinterpret_cast<const __nv_bfloat16*>(B), K, shape,
                                epi, sms, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// Both conv2 projections in one split launch (tests/test_dense_fusion_gpu.py): packed weight rows W [nproj*HC][HC]
+// (GATv2 [l; r], nproj 2; Transformer [q; k; v], nproj 3), target rows from A2 when given, else from A.
+extern "C" int mls_test_conv2_proj(const void* A, int lda, const void* A2, int lda2, const void* W, const float* bias, const float* obs,
+                                   long long obs_stride, int nodes, const int* row_index, const int* row_index_t, const float* att,
+                                   float* dots, float* dots_t, void* C, void* Ct, int M, int HC, int nproj, const int* m_dev,
+                                   const int* m_dev_t, void* stream) {
+  int dev = 0, sms = 0;
+  MLS_CUDA(cudaGetDevice(&dev));
+  MLS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  mls::GemmShape shape{M, nproj * HC, HC, m_dev};
+  shape.m_dev_t = m_dev_t; shape.t_lo = nproj == 3 ? 0 : HC; shape.t_hi = shape.t_lo + HC;
+  if (A2) { shape.A2 = reinterpret_cast<const __nv_bfloat16*>(A2); shape.lda2 = lda2; shape.k2_lo = 0; shape.k2_hi = HC; }
+  mls::GemmEpilogue epi{reinterpret_cast<__nv_bfloat16*>(C), (nproj - 1) * HC, bias, obs, obs_stride, nodes, 0, att, dots, row_index};
+  epi.Ct = reinterpret_cast<__nv_bfloat16*>(Ct); epi.ldct = HC; epi.dots_t = dots_t; epi.row_index_t = row_index_t;
+  return mls::gemm_bf16_launch(reinterpret_cast<const __nv_bfloat16*>(A), lda, reinterpret_cast<const __nv_bfloat16*>(W), HC, shape,
+                               epi, sms, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// The fused 128-wide dueling heads (tests/test_dense_fusion_gpu.py): A [M][K] (columns [k2_lo, k2_hi) from A2 when given),
+// W_h0 [256][K], W_h1 [256][256]; Q and actions as the forward writes them.
+extern "C" int mls_test_head_dueling(const void* A, int lda, const void* A2, int lda2, int k2_lo, int k2_hi, int M, int K, const int* m_dev,
+                                     const void* w_h0, const float* b_h0, const void* w_h1, const float* b_h1, const float* hv1,
+                                     const float* hv2, const float* bq, const float* bv, const int* idx, long long row0, int per_graph_N,
+                                     float* q_out, signed char* act_out, int out_mode, float eps, unsigned long long seed,
+                                     unsigned long long offset, const double* rand3, void* stream) {
+  int dev = 0, sms = 0;
+  MLS_CUDA(cudaGetDevice(&dev));
+  MLS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  mls::GemmShape shape{M, 256, K, m_dev};
+  if (A2) { shape.A2 = reinterpret_cast<const __nv_bfloat16*>(A2); shape.lda2 = lda2; shape.k2_lo = k2_lo; shape.k2_hi = k2_hi; }
+  mls::HeadOut out{bq, bv, idx, row0, per_graph_N, q_out, reinterpret_cast<int8_t*>(act_out), out_mode,
+                   mls::ActArgsB{eps, seed, offset, rand3, nullptr, 0}};
+  return mls::head_dueling_launch(reinterpret_cast<const __nv_bfloat16*>(A), lda, shape, reinterpret_cast<const __nv_bfloat16*>(w_h0),
+                                  reinterpret_cast<const __nv_bfloat16*>(w_h1), mls::HeadVecs{b_h0, b_h1, hv1, hv2}, out, sms,
+                                  reinterpret_cast<cudaStream_t>(stream));
 }

@@ -10,6 +10,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "dgn_kernels.cuh"
 
 namespace mls {
 
@@ -44,6 +45,13 @@ struct GemmEpilogue {
   // fp32-grade route, whose operands are 3-way bf16 splits concatenated along K (dgn_forward.cu).
   float* Cf;
   int ldcf;
+  // target segment of a split launch (GemmShape::t_lo): C, dots and row_index above serve the source columns; the target
+  // columns [t_lo, t_hi) go to Ct[m][n - t_lo] (row stride ldct), dots_t[m][(n - t_lo) / 128] and the row scale goes
+  // through row_index_t.  bias and dotvec are indexed by the packed column n in both segments.
+  __nv_bfloat16* Ct;
+  int ldct;
+  float* dots_t;
+  const int* row_index_t;
 };
 
 struct GemmShape {
@@ -54,6 +62,12 @@ struct GemmShape {
   // (snapshot columns of relu(conv1) live in x1, the rest in z)
   const __nv_bfloat16* A2;
   int lda2, k2_lo, k2_hi;
+  // optional split of the N columns (t_lo < t_hi, multiples of 256 or, without dots, of 128): the conv2 projections of
+  // the source rows (columns outside [t_lo, t_hi)) and of the target rows (inside) in one launch over the packed weight
+  // rows.  Target columns are computed for rows [0, min(M, *m_dev_t)) only, source columns for rows [0, min(M, *m_dev)),
+  // and the second A matrix, if given, applies to the target columns only.
+  const int* m_dev_t;
+  int t_lo, t_hi;
 };
 
 size_t gemm_smem_bytes(int BN);
@@ -62,5 +76,16 @@ int make_tmap_bf16(CUtensorMap* tm, const void* base, int rows, int cols, int ld
 // host: build the two TMA descriptors + launch.  A: [M, K] row stride lda; B: [N, K] row stride ldb.
 int gemm_bf16_launch(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, int ldb, GemmShape shape,
                      GemmEpilogue epi, int sm_count, cudaStream_t st);
+
+// Dueling heads with 128-wide hidden layers in one persistent kernel: per row m < min(M, *m_dev),
+//     hid = relu(A[m] @ W_h0^T + b_h0) (bf16),  h2 = relu(hid @ W_h1^T + b_h1),
+//     head_final_row(m, <h2[0:128], hv1[0:128]>, <h2[128:256], hv1[128:256]>, <h2[0:128], hv2[0:128]>)
+// with the rounding points and accumulation orders of the two-GEMM chain (MODE 2, then MODE 3).  shape: N = 256, K = latent,
+// optional A2 K range.  W_h0 [256][K], W_h1 [256][256] (block diagonal [Q1 0; 0 V1]).
+struct HeadVecs {
+  const float *b_h0, *b_h1, *hv1, *hv2;     // [256] each
+};
+int head_dueling_launch(const __nv_bfloat16* A, int lda, GemmShape shape, const __nv_bfloat16* w_h0, const __nv_bfloat16* w_h1,
+                        const HeadVecs& vec, const HeadOut& out, int sm_count, cudaStream_t st);
 
 }  // namespace mls
