@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define MLS_VERSION 210
+#define MLS_VERSION 211
 #define MLS_MAX_NODES 256
 
 /* ---- errors ------------------------------------------------------------------------- */
@@ -368,6 +368,34 @@ int mls_transformer_edge_fwd(const float* k, const float* v, int64_t lds, const 
 int mls_transformer_edge_bwd(const float* k, const float* v, int64_t lds, const float* q, int64_t ldq, const int32_t* tgt_row,
                              const int32_t* src_row, const int32_t* src_cnt, int32_t n_targets, int32_t heads,
                              const float* alpha, const float* dout, float* d_k, float* d_v, float* d_q, void* stream);
+
+/* ---- prioritized replay (melissa_b200/csrc/replay_per.cu).  Replaces tianshou PrioritizedReplayBuffer's numpy
+ * SegmentTree (init_weight / sample_indices / get_weight / update_weight) for the device replay ring.
+ * One fp64 sum tree per ring slot over its L = n_episodes * n_nodes cells (leaf = cell episode * N + agent, holding
+ * p^alpha; 0 where the agent did not act), fanout 32, levels stored leaves first and root last; the trees of a ring
+ * are [ring_rounds][mls_per_tree_size(L)] doubles.  max_prio / min_prio are device doubles (tianshou starts both at 1). */
+
+/* fp64 nodes of one slot's tree over n_cells leaves (leaves + internal levels + root); -1 if n_cells < 1. */
+int64_t mls_per_tree_size(int64_t n_cells);
+/* Round build: every leaf of `tree` (one slot) = (*max_prio)^alpha where flags bit 0 (acted) is set, else 0; then every
+ * internal level.  The slot's root is the round's total priority. */
+int mls_per_build(const uint8_t* flags /*[L]*/, int64_t n_episodes, int32_t n_nodes, const double* max_prio, double alpha,
+                  double* tree, void* stream);
+/* Proportional sampling, one sample per u[m] in [0, 1).  The usable slots are (first_slot + k) % ring_rounds for
+ * k < n_slots, oldest first, their leaves concatenated in that order; with S_i the inclusive prefix sums, T their total and
+ * v = u * T the sample is the leaf min{i : leaf_i > 0 and S_i >= v}, or the last positive leaf if v passes it.  A leaf of
+ * priority 0 is never returned (if the usable slots hold none that is positive: slot first_slot, cell 0, leaf 0).
+ * -> round_index (ring slot), episode, agent; leaf (NULL ok) = the leaf's value. */
+int mls_per_sample(const double* trees, int32_t ring_rounds, int64_t n_episodes, int32_t n_nodes, int32_t first_slot,
+                   int32_t n_slots, const double* u, int32_t n_samples, int32_t* round_index, int32_t* episode,
+                   int32_t* agent, double* leaf, void* stream);
+/* Priority update after a learning step: leaf (round_index[m], episode[m], agent[m]) = (|td[m]| + eps)^alpha, the last
+ * occurrence of a leaf in the batch wins; its ancestors are recomputed from their children level by level (no atomics:
+ * the tree stays a deterministic function of its leaves); *max_prio / *min_prio take the max / min of |td| + eps.
+ * Samples outside the ring are ignored. */
+int mls_per_update(double* trees, int32_t ring_rounds, int64_t n_episodes, int32_t n_nodes, const int32_t* round_index,
+                   const int32_t* episode, const int32_t* agent, const float* td, int32_t n_samples, double alpha,
+                   double eps, double* max_prio, double* min_prio, void* stream);
 
 #ifdef __cplusplus
 }

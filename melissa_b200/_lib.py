@@ -93,7 +93,8 @@ EXPORTS = ["mls_version", "mls_last_error", "mls_device_info", "mls_words_per_ro
            "mls_env_info", "mls_dgn_workspace_bytes", "mls_dgn_chunk_graphs", "mls_dgn_forward", "mls_dgn_prepare",
            "mls_dgn_csr_cache_bytes", "mls_dgn_csr_cache_build", "mls_obs_pack", "mls_obs_unpack", "mls_nstep_returns",
            "mls_adam_step", "mls_train_list_capacity", "mls_train_lists", "mls_gatv2_edge_fwd", "mls_gatv2_edge_bwd_blocks",
-           "mls_gatv2_edge_bwd", "mls_transformer_edge_fwd", "mls_transformer_edge_bwd"]
+           "mls_gatv2_edge_bwd", "mls_transformer_edge_fwd", "mls_transformer_edge_bwd", "mls_per_tree_size",
+           "mls_per_build", "mls_per_sample", "mls_per_update"]
 PACKED_NODE_BYTES = 12
 
 _lib = None
@@ -146,6 +147,12 @@ def lib():
     L.mls_gatv2_edge_bwd.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, vp, vp, vp, C.c_int32, C.c_int32, vp, vp, vp, vp, vp, vp]
     L.mls_transformer_edge_fwd.argtypes = [vp, vp, C.c_int64, vp, C.c_int64, vp, vp, vp, C.c_int32, C.c_int32, vp, vp, vp]
     L.mls_transformer_edge_bwd.argtypes = [vp, vp, C.c_int64, vp, C.c_int64, vp, vp, vp, C.c_int32, C.c_int32, vp, vp, vp, vp, vp, vp]
+    L.mls_per_tree_size.argtypes = [C.c_int64]
+    L.mls_per_tree_size.restype = C.c_int64
+    L.mls_per_build.argtypes = [vp, C.c_int64, C.c_int32, vp, C.c_double, vp, vp]
+    L.mls_per_sample.argtypes = [vp, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, vp, C.c_int32, vp, vp, vp, vp, vp]
+    L.mls_per_update.argtypes = [vp, C.c_int32, C.c_int64, C.c_int32, vp, vp, vp, vp, C.c_int32, C.c_double, C.c_double,
+                                 vp, vp, vp]
     for name in EXPORTS:
         getattr(L, name)
     _lib = L

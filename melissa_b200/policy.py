@@ -325,12 +325,16 @@ class DQNPolicy:
         return {"loss": loss.detach()}
 
     def update(self, sample_size: int, buffer, **kwargs):
-        """tianshou BasePolicy.update: sample -> process_fn -> learn."""
+        """tianshou BasePolicy.update: sample -> process_fn -> learn -> post_process_fn (a prioritized replay receives
+        the TD errors as new priorities before this returns, so before the next ``begin_round`` can reuse a slot)."""
         rho, ep, agent = buffer.sample_indices(int(sample_size), self._n_step)
         batch = Batch(buffer.gather(rho, ep, agent, self._n_step, self._gamma))
         batch.rho = rho
         batch = self.process_fn(batch, buffer)
-        return self.learn(batch, buffer=buffer, **kwargs)
+        out = self.learn(batch, buffer=buffer, **kwargs)
+        if hasattr(buffer, "update_weight"):          # prioritized replay: tianshou's post_process_fn
+            buffer.update_weight((rho, ep, agent), batch.weight)
+        return out
 
 
 class DGNPolicy(DQNPolicy):

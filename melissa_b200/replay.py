@@ -18,6 +18,7 @@ Everything stays on the device; sampling returns the reference's agent-observati
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -76,11 +77,10 @@ class DeviceReplay:
         self.head += 1
 
     # ------------------------------------------------------------------ sampling
-    def sample_indices(self, batch_size: int, n_step: int):
-        """Uniform over the stored transitions whose n-step window AND its bootstrap frame are stored: round rho is
-        usable when rounds rho .. rho+n_step are all in the ring (a chain still alive after n_step steps bootstraps
-        from the observation of round rho+n_step, which is only packed by the next ``begin_round``).  Needs
-        ``ring_rounds > n_step``.  -> (ring round, episode, agent) int32 tensors [M]."""
+    def _usable_rounds(self, n_step: int):
+        """Round rho is usable when rounds rho .. rho+n_step are all in the ring (a chain still alive after n_step steps
+        bootstraps from the observation of round rho+n_step, which is only packed by the next ``begin_round``).
+        -> (ring slot of the oldest usable round, number of usable rounds); the newest n_step rounds are not usable."""
         if n_step >= self.R:
             raise ValueError(f"a ring of {self.R} rounds cannot hold an n-step window of {n_step} rounds plus its "
                              "bootstrap frame (needs ring_rounds > n_step)")
@@ -92,8 +92,14 @@ class DeviceReplay:
             if int(self.counts.sum().item()) == 0:
                 raise RuntimeError("replay holds no transitions yet")
             self._nonempty = True
-        # ring slots ordered oldest -> newest; the newest n_step rounds cannot start a complete window
-        order = ((torch.arange(usable, device=self.device) + (self.head - filled)) % self.R)
+        return (self.head - filled) % self.R, usable
+
+    def sample_indices(self, batch_size: int, n_step: int):
+        """Uniform over the stored transitions of the usable rounds (``_usable_rounds``): their n-step window AND its
+        bootstrap frame are stored.  Needs ``ring_rounds > n_step``.  -> (ring round, episode, agent) int32 tensors [M]."""
+        first, usable = self._usable_rounds(n_step)
+        # ring slots ordered oldest -> newest
+        order = (torch.arange(usable, device=self.device) + first) % self.R
         cnt = self.counts[order]
         cum = torch.cumsum(cnt, 0)
         total = cum[-1]
@@ -131,3 +137,82 @@ class DeviceReplay:
         _lib.check(self.lib.mls_obs_unpack(self.frames.data_ptr(), frame.data_ptr(), agent.to(torch.int32).contiguous().data_ptr(),
                                            self.N, M, self.N * 8 + 1, rows.data_ptr(), _lib.current_stream_ptr()))
         return rows
+
+
+class DevicePrioritizedReplay(DeviceReplay):
+    """Prioritized replay over the same ring: tianshou 1.0 ``PrioritizedReplayBuffer(alpha, beta, weight_norm)``,
+    restated (PARITY UNPINNED: tianshou is not a dependency; tests/per_reference.py ``PrioritizedRingReference`` is the
+    float64 restatement the tests hold the kernels to).
+
+    * one fp64 sum tree per ring slot, leaves = cells ``episode * N + agent`` holding ``p^alpha``
+      (``csrc/replay_per.cu``); ``max_prio = min_prio = 1`` at construction, eps = float32 machine epsilon;
+    * ``begin_round`` gives every transition of the new round ``max_prio^alpha`` and every other cell 0;
+    * ``sample_indices`` draws proportionally to priority over the usable rounds of ``DeviceReplay``;
+    * ``gather`` adds ``weight = (leaf / min_prio)^(-beta)`` (divided by its batch maximum with ``weight_norm``), fp32;
+    * ``update_weight`` sets the sampled leaves to ``(|td| + eps)^alpha`` (last occurrence wins) and raises
+      ``max_prio`` / lowers ``min_prio`` with ``|td| + eps``.
+
+    Everything runs on the caller's stream; after the first ``sample_indices`` no method synchronises with the host.
+    Differences from tianshou's numpy code: the leaf and ``|td| + eps`` are evaluated in fp64 (tianshou rounds them to
+    float32 before storing them in its float64 tree), and a leaf of priority 0 is never sampled."""
+
+    def __init__(self, n_episodes: int, n_nodes: int, ring_rounds: int, alpha: float, beta: float,
+                 weight_norm: bool = True, device="cuda", seed: int = 0):
+        if not alpha > 0.0:
+            raise ValueError(f"alpha must be > 0 (got {alpha})")
+        if not beta >= 0.0:
+            raise ValueError(f"beta must be >= 0 (got {beta})")
+        super().__init__(n_episodes, n_nodes, ring_rounds, device=device, seed=seed)
+        self.alpha, self.beta, self.weight_norm = float(alpha), float(beta), bool(weight_norm)
+        self.eps = float(np.finfo(np.float32).eps)
+        size = int(self.lib.mls_per_tree_size(self.B * self.N))
+        self.tree = torch.zeros(self.R, size, dtype=torch.float64, device=self.device)   # [slot][leaves .. root]
+        self.prio = torch.ones(2, dtype=torch.float64, device=self.device)               # max_prio, min_prio
+
+    def set_beta(self, beta: float) -> None:
+        if not beta >= 0.0:
+            raise ValueError(f"beta must be >= 0 (got {beta})")
+        self.beta = float(beta)
+
+    def begin_round(self, obs: torch.Tensor, active: torch.Tensor):
+        super().begin_round(obs, active)
+        slot = self._pending
+        _lib.check(self.lib.mls_per_build(self.flags[slot].data_ptr(), self.B, self.N, self.prio.data_ptr(), self.alpha,
+                                          self.tree[slot].data_ptr(), _lib.current_stream_ptr()))
+
+    def sample_indices(self, batch_size: int, n_step: int):
+        """Proportional to priority over the stored transitions of the usable rounds (same rule and errors as
+        ``DeviceReplay.sample_indices``).  -> (ring round, episode, agent) int32 tensors [M]."""
+        first, usable = self._usable_rounds(n_step)
+        M = int(batch_size)
+        u = torch.rand(M, device=self.device, generator=self.gen, dtype=torch.float64)
+        rho, ep, agent = (torch.empty(M, dtype=torch.int32, device=self.device) for _ in range(3))
+        _lib.check(self.lib.mls_per_sample(self.tree.data_ptr(), self.R, self.B, self.N, first, usable, u.data_ptr(), M,
+                                           rho.data_ptr(), ep.data_ptr(), agent.data_ptr(), None, _lib.current_stream_ptr()))
+        return rho, ep, agent
+
+    def _weights(self, rho, ep, agent):
+        """Importance weights of (ring round, episode, agent) triples: (leaf / min_prio)^(-beta), normalised by the
+        batch maximum with ``weight_norm``.  fp32 [M]."""
+        leaf = self.tree[rho.long(), ep.long() * self.N + agent.long()]
+        w = (leaf / self.prio[1]).pow(-self.beta)
+        if self.weight_norm:
+            w = w / w.max()
+        return w.to(torch.float32)
+
+    def gather(self, rho, ep, agent, n_step: int, gamma: float):
+        """``DeviceReplay.gather`` plus ``weight`` (fp32 [M], see ``_weights``)."""
+        out = super().gather(rho, ep, agent, n_step, gamma)
+        out["weight"] = self._weights(rho, ep, agent)
+        return out
+
+    def update_weight(self, index, new_weight: torch.Tensor):
+        """tianshou ``update_weight(index, new_weight)`` with index = the (ring round, episode, agent) triple of
+        ``sample_indices`` and new_weight the TD errors ``DQNPolicy.learn`` leaves in ``batch.weight``."""
+        rho, ep, agent = (t.to(torch.int32).contiguous() for t in index)
+        td = new_weight.detach().to(torch.float32).contiguous()
+        if td.dim() != 1 or any(t.shape != td.shape for t in (rho, ep, agent)):
+            raise ValueError("update_weight needs one TD error per sampled (round, episode, agent)")
+        _lib.check(self.lib.mls_per_update(self.tree.data_ptr(), self.R, self.B, self.N, rho.data_ptr(), ep.data_ptr(),
+                                           agent.data_ptr(), td.data_ptr(), int(td.shape[0]), self.alpha, self.eps,
+                                           self.prio.data_ptr(), self.prio[1:].data_ptr(), _lib.current_stream_ptr()))
