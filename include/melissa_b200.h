@@ -41,6 +41,7 @@ int mls_words_per_row(int n_nodes);
 /* process-wide tuning options (A/B switches for benchmarking; defaults are the fast paths):
  *   "attn_mma"  1 = conv1 attention through the pair-logit table + tcgen05 aggregation (discrete-feature mode)
  *   "conv2_mma" 1 = conv2 attention with half2 logits + tcgen05 aggregation (graphs of <= 64 nodes)
+ *   "max_ctas"  test only: n > 0 caps the grid of the persistent kernels at n CTAs (many tiles per CTA); 0 = off
  * get returns -1 for an unknown key. */
 int mls_set_option(const char* key, int value);
 int mls_get_option(const char* key);

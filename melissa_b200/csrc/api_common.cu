@@ -42,9 +42,11 @@ extern "C" int mls_device_info(int32_t* sm_count, int32_t* cc_major, int32_t* cc
 //                x1); 0 = needed rows in node order per graph + a separate snapshot copy in z
 //   "fp32_tc":   1 = precision fp32 runs its dense layers on the tensor cores through 3-way bf16 operand splits
 //                (fp32-grade, dgn_forward.cu); 0 = SIMT sgemm
+//   "max_ctas":  test only: n > 0 caps the grid of the persistent kernels (the tcgen05 GEMM and fused dueling heads, conv2
+//                attention, the conv1 table kernels) at n CTAs, so that small inputs give every CTA many tiles; 0 = off
 #include <stdlib.h>
 #include <string.h>
-static int g_attn_mma = -1, g_conv2_mma = -1, g_fp32_tc = -1, g_attn_hp = -1, g_ctrl_first = -1;
+static int g_attn_mma = -1, g_conv2_mma = -1, g_fp32_tc = -1, g_attn_hp = -1, g_ctrl_first = -1, g_max_ctas = -1;
 extern "C" int mls_get_option(const char* key) {
   if (key && !strcmp(key, "attn_mma")) {
     if (g_attn_mma < 0) { const char* e = getenv("MLS_ATTN_MMA"); g_attn_mma = e ? atoi(e) : 1; }
@@ -66,7 +68,15 @@ extern "C" int mls_get_option(const char* key) {
     if (g_conv2_mma < 0) { const char* e = getenv("MLS_CONV2_MMA"); g_conv2_mma = e ? atoi(e) : 1; }
     return g_conv2_mma;
   }
+  if (key && !strcmp(key, "max_ctas")) {
+    if (g_max_ctas < 0) { const char* e = getenv("MLS_MAX_CTAS"); g_max_ctas = e && atoi(e) > 0 ? atoi(e) : 0; }
+    return g_max_ctas;
+  }
   return -1;
+}
+int mls_cap_grid(int grid) {
+  const int cap = mls_get_option("max_ctas");
+  return cap > 0 && grid > cap ? cap : grid;
 }
 extern "C" int mls_set_option(const char* key, int value) {
   if (key && !strcmp(key, "conv2_mma")) { g_conv2_mma = value ? 1 : 0; return MLS_OK; }
@@ -74,6 +84,7 @@ extern "C" int mls_set_option(const char* key, int value) {
   if (key && !strcmp(key, "attn_hp")) { g_attn_hp = value < 0 ? 0 : (value > 2 ? 2 : value); return MLS_OK; }
   if (key && !strcmp(key, "attn_mma")) { g_attn_mma = value ? 1 : 0; return MLS_OK; }
   if (key && !strcmp(key, "ctrl_first")) { g_ctrl_first = value ? 1 : 0; return MLS_OK; }
+  if (key && !strcmp(key, "max_ctas")) { g_max_ctas = value > 0 ? value : 0; return MLS_OK; }
   mls_set_error("unknown option %s", key ? key : "(null)");
   return MLS_ERR_INVALID;
 }

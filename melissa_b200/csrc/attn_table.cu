@@ -246,7 +246,8 @@ constexpr int kBPanel = 64 * 128;              // value panel: 64 sources x 64 c
 constexpr int kStageA = 4 * kAHead;            // 32 KiB
 constexpr int kStageB = 8 * kBPanel;           // 64 KiB
 constexpr int kStage = kStageA + kStageB;      // 96 KiB
-constexpr int kMetaSrc = 64 * kMaxNbr;         // CSR source lists of a tile
+constexpr int kMetaSrc = 64 * kMaxNbr;         // CSR source lists of a tile: G * csr_stride(N) <= 2048 for G * N <= 64, N <= 62
+static_assert(64 / 33 * csr_stride(33) <= kMetaSrc && csr_stride(62) <= kMetaSrc, "tile CSR lists");
 constexpr int kMetaTab = kMetaSrc + 64 * 4 /*need list, counts*/ + 64 * 2 /*ids*/ + 128 * 2 /*CSR row pointers*/ + 64 * 4 /*dm*/;
 constexpr int kMeta = kMetaTab + 2 * 64 * 4 /*x_out row and snapshot slot of every TMEM column*/;
 constexpr int kTSmem = 2 * kStage + 2 * kMeta + 256 /*barriers*/ + 1024;
@@ -427,6 +428,7 @@ __global__ void __launch_bounds__(kTThreads, 1) attn_table_mma_kernel(const Attn
     const int p = warp < 4 ? warp - 2 : warp - 10;                            // warps 2, 3, 12..23 -> 0..13
     const int team = p & 1, pt = (p >> 1) * 32 + lane;                        // 0..223
     const int self = a.transformer ? 0 : 1;
+    const int cpg = csr_stride(N) / 16;                                         // 16-byte chunks of a graph's CSR lists
     unsigned char* sA = smem + team * kStage;
     const uint32_t sB32 = smem_u32(sA + kStageA);
     uint8_t* src_s = meta + team * kMeta;                                       // [gt][N*32]
@@ -475,10 +477,10 @@ __global__ void __launch_bounds__(kTThreads, 1) attn_table_mma_kernel(const Attn
         const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
         pv = __ldg(a.csr_ptr + cg * (N + 1) + il);
       }
-      if (pt < rt * 2) {                                                       // N*32 bytes (2N chunks of 16 B) per graph
-        const int gl = pt / (2 * N), cl = pt - gl * 2 * N;
+      if (pt < gt * cpg) {                                                     // csr_stride(N) bytes (cpg chunks of 16 B) per graph
+        const int gl = pt / cpg, cl = pt - gl * cpg;
         const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
-        sv = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * N * kMaxNbr) + cl);
+        sv = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * csr_stride(N)) + cl);
       }
       // the tile's needed targets, compacted (team warps 0 and 1 hold node rows 0..63)
       const uint32_t nbal = __ballot_sync(0xffffffffu, pt < rt && xrv >= 0);
@@ -506,7 +508,7 @@ __global__ void __launch_bounds__(kTThreads, 1) attn_table_mma_kernel(const Attn
       }
       if (pt < rt) { cid[pt] = cv; dm_s[pt] = dmv; }
       if (pt < gt * (N + 1)) ptr_s[pt] = (uint16_t)pv;
-      if (pt < rt * 2) reinterpret_cast<uint4*>(src_s)[pt] = sv;
+      if (pt < gt * cpg) reinterpret_cast<uint4*>(src_s)[pt] = sv;
       if (pt < 64 && lane == 0) cnt_s[pt >> 5] = __popc(nbal);
       bar_team(team);
       if (pt < rt && xrv >= 0) {
@@ -532,7 +534,7 @@ __global__ void __launch_bounds__(kTThreads, 1) attn_table_mma_kernel(const Attn
         const int gl = i / N, il = i - gl * N, rbase = gl * N;
         const uint16_t* ptr = ptr_s + gl * (N + 1);
         const int r0 = ptr[il], d = (int)ptr[il + 1] - r0;
-        const uint8_t* src = src_s + gl * N * kMaxNbr + r0;
+        const uint8_t* src = src_s + gl * csr_stride(N) + r0;
         const float* Erow = a.E + (size_t)cid[i] * kAttnUcap * 4 + h;
         // entry 0 = the self loop (GATv2), then the CSR neighbours; batches of 8 independent table reads
         const int cnt = d + self;
@@ -736,6 +738,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
     const int team = (warp - 10) / 3, pt = ((warp - 10) % 3) * 32 + lane;      // 0..95
     const int hp = team & 1;
     const int self = a.transformer ? 0 : 1;
+    const int cpg = csr_stride(N) / 16;                                         // 16-byte chunks of a graph's CSR lists
     unsigned char* sA = smem + team * kStage2;
     unsigned char* sBv = sA + kStageA2;
     const uint32_t sB32 = smem_u32(sBv);
@@ -780,17 +783,17 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
         const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
         pv = __ldg(a.csr_ptr + cg * (N + 1) + il);
       }
-      {                                                                        // N*32 bytes (2N chunks of 16 B) per graph: <= 124 chunks
+      {                                                                        // csr_stride(N) bytes (cpg chunks of 16 B) per graph: <= 128 chunks
         const int c0 = pt, c1 = pt + kTeam4;
-        if (c0 < rt * 2) {
-          const int gl = c0 / (2 * N), cl = c0 - gl * 2 * N;
+        if (c0 < gt * cpg) {
+          const int gl = c0 / cpg, cl = c0 - gl * cpg;
           const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
-          sv0 = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * N * kMaxNbr) + cl);
+          sv0 = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * csr_stride(N)) + cl);
         }
-        if (c1 < rt * 2) {
-          const int gl = c1 / (2 * N), cl = c1 - gl * 2 * N;
+        if (c1 < gt * cpg) {
+          const int gl = c1 / cpg, cl = c1 - gl * cpg;
           const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
-          sv1 = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * N * kMaxNbr) + cl);
+          sv1 = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * csr_stride(N)) + cl);
         }
       }
       const uint32_t nbal = __ballot_sync(0xffffffffu, pt < rt && xrv >= 0);
@@ -818,8 +821,8 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
       }
       if (pt < rt) { cid[pt] = cv; dm_s[pt] = dmv; }
       if (pt < gt * (N + 1)) ptr_s[pt] = (uint16_t)pv;
-      if (pt < rt * 2) reinterpret_cast<uint4*>(src_s)[pt] = sv0;
-      if (pt + kTeam4 < rt * 2) reinterpret_cast<uint4*>(src_s)[pt + kTeam4] = sv1;
+      if (pt < gt * cpg) reinterpret_cast<uint4*>(src_s)[pt] = sv0;
+      if (pt + kTeam4 < gt * cpg) reinterpret_cast<uint4*>(src_s)[pt + kTeam4] = sv1;
       if (pt < 64 && lane == 0) cnt_s[pt >> 5] = __popc(nbal);
       bar_team4(team);
       if (pt < rt && xrv >= 0) {
@@ -845,7 +848,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
         const int gl = i / N, il = i - gl * N, rbase = gl * N;
         const uint16_t* ptr = ptr_s + gl * (N + 1);
         const int r0 = ptr[il], d = (int)ptr[il + 1] - r0;
-        const uint8_t* src = src_s + gl * N * kMaxNbr + r0;
+        const uint8_t* src = src_s + gl * csr_stride(N) + r0;
         const float* Erow = a.E + (size_t)cid[i] * kAttnUcap * 4 + h;
         const int cnt = d + self;
         unsigned char* arow = sA + hl * kAHead;
@@ -913,7 +916,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
 // followed by its STORE warp (tile -> global); a stage returns to its team on tcgen05.commit.
 constexpr int kRecFixed = 16 + 64 * 4 + 64 * 4 + 64 * 2;   // 656 bytes: header, x_out rows, snapshot slots, key ids
 constexpr int kRecChunk = 512;                             // entries per in-kernel chunk
-__host__ __device__ inline int rec_entry_cap(int rows) { return (rows * (kMaxNbr + 1) + 7) & ~7; }
+__host__ __device__ inline int rec_entry_cap(int rows) { return (rows * (kMaxList + 1) + 7) & ~7; }   // sources + self loop
 __host__ __device__ inline int rec_stride(int rows) { return kRecFixed + 10 * rec_entry_cap(rows); }
 
 // One warp per tile.  Lane l owns tile rows l and l + 32.
@@ -954,7 +957,7 @@ __global__ void __launch_bounds__(256, 4) attn_table_prep_kernel(const AttnTable
       const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl[q]) * a.gid_stride) : (size_t)(g0 + gl[q]);
       p0[q] = __ldg(a.csr_ptr + cg * (N + 1) + il);
       const int d = (int)__ldg(a.csr_ptr + cg * (N + 1) + il + 1) - p0[q];
-      srcp[q] = a.csr_src + cg * N * kMaxNbr + p0[q];
+      srcp[q] = a.csr_src + cg * csr_stride(N) + p0[q];
       if (xr[q] >= 0) cnt[q] = d + self;
       if (il == 0) cg_s[gl[q]] = (int)cg;
     }
@@ -1006,7 +1009,7 @@ __global__ void __launch_bounds__(256, 4) attn_table_prep_kernel(const AttnTable
     if (c == 0) continue;
     const int glr = r / N, rbase = glr * N;
     const float4* Erow = reinterpret_cast<const float4*>(a.E) + (size_t)cid_s[r] * kAttnUcap;
-    const uint8_t* src = a.csr_src + (size_t)cg_s[glr] * N * kMaxNbr + p0_s[r];
+    const uint8_t* src = a.csr_src + (size_t)cg_s[glr] * csr_stride(N) + p0_s[r];
     uint16_t* jo = jr + off_s[rki];
     __half* wo = wts + off_s[rki];
     const int rk = rki << 8;
@@ -1388,7 +1391,7 @@ int attn_table_conv_launch(const AttnTableArgs& a, int sm_count, cudaStream_t st
   pair_logit_kernel<<<sm_count * 2, 256, 0, st>>>(a);
   const int G = a.pool_mode >= 0 ? 1 : kAttnMaxRows / a.N;     // pooling: one graph per tile
   const int n_tiles = (a.n_graphs + G - 1) / G;
-  const int grid = n_tiles < sm_count ? n_tiles : sm_count;
+  const int grid = mls_cap_grid(n_tiles < sm_count ? n_tiles : sm_count);   // all three kernels below take any grid
   if (grid > 0) {
     const int mode = mls_get_option("attn_hp");
     if (mode >= 2 && a.pool_mode < 0 && a.rec && a.tile_idx) {                 // per-tile records + row-major MMA (default)

@@ -23,7 +23,7 @@ struct AttnTableArgs {
   const uint32_t* key;       // [rows] feature key of every node row
   int N, H, n_graphs;
   const uint16_t* csr_ptr;   // [graphs][N+1]
-  const uint8_t* csr_src;    // [graphs][N*32]
+  const uint8_t* csr_src;    // [graphs][csr_stride(N)]
   const int* slot;           // [rows] controlling-list slot or -1
   // optional "needed" row map (ctrl_need_list_kernel): x_out row of every node row, -1 = nobody reads this node's
   // conv output (its softmax weights are not even built); needed rows of a graph are consecutive, in node order

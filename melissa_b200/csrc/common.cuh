@@ -9,6 +9,8 @@
 void mls_set_error(const char* fmt, ...);
 void mls_count_launch(int n = 1);
 extern "C" int mls_get_option(const char* key);
+// grid of a persistent kernel (a CTA loops over tiles blockIdx.x, blockIdx.x + gridDim.x, ...) under option "max_ctas"
+int mls_cap_grid(int grid);
 
 #define MLS_CHECK_ARG(cond, ...)          \
   do {                                    \

@@ -58,7 +58,7 @@ __device__ __forceinline__ uint64_t desc_mn(uint32_t smem_addr, uint32_t lbo16, 
 }
 
 // Targets are processed in blocks of at most kTB targets and kEdgeCap edge entries (one block for the typical graph:
-// ~17 controlling nodes, ~106 entries; the worst case -- 64 targets x 33 entries -- takes several): the per-item shared
+// ~17 controlling nodes, ~106 entries; the worst case -- 64 targets x 34 entries -- takes several): the per-item shared
 // memory is sized for a block, not for the worst case, so that seven CTAs fit an SM.
 constexpr int kTB = 32;
 constexpr int kEdgeCap = 256;
@@ -198,7 +198,7 @@ __global__ void __launch_bounds__(kThreads, TR ? 4 : kCtasPerSm) conv2_attn_kern
     __syncthreads();
     if (cnt == 0 && gn < a.n_graphs) { issue_A(n0.x, n0.y, n0.z, n0.w); issue_B(n0.x, n0.y, n0.z, n0.w, n1.x, n1.y); }
     for (int t0 = 0; t0 < cnt;) {
-      // ---- block [t0, t1): at most kTB targets and kEdgeCap entries (a single target has at most 33)
+      // ---- block [t0, t1): at most kTB targets and kEdgeCap entries (a single target has at most kMaxList + 1 = 34)
       const int eb = s_eptr[t0];
       int t1;
       if (t0 == 0 && cnt <= kTB && s_eptr[cnt] - eb <= kEdgeCap) {
@@ -339,7 +339,7 @@ int launch(const Conv2Args& a, int sm_count, cudaStream_t st) {
   }
   const int per_sm = TR ? 4 : kCtasPerSm;
   long long items = (long long)a.n_graphs * a.H;
-  long long grid = (long long)sm_count * per_sm;
+  long long grid = mls_cap_grid(sm_count * per_sm);         // graphs stride by gridDim.x / H: any multiple of H works
   grid -= grid % a.H;
   if (grid < a.H) grid = a.H;
   if (grid > items) grid = items;                           // items is a multiple of H

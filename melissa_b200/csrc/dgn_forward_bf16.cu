@@ -152,8 +152,8 @@ __global__ void __launch_bounds__(256) enc0_keys_kernel(int n_keys, int in_dim, 
 
 // ------------------------------------------------------------------------------ graph CSR
 // radius_graph(pos, r=0.2, loop=False, max_num_neighbors=32) once per chunk and graph, as source
-// lists per target: csr_ptr[g][N+1] (uint16 offsets into the graph's list), csr_src[g][N*32] (uint8
-// source node ids, index order).  Self loops are NOT stored (GATv2 adds its own).  The lists are
+// lists per target: csr_ptr[g][N+1] (uint16 offsets into the graph's list), csr_src[g][csr_stride(N)] (uint8
+// source node ids, index order; up to 33 per target, see kMaxList).  Self loops are NOT stored (GATv2 adds its own).  The lists are
 // shared by all heads and by both conv layers.  One CTA per graph.
 template <int W>
 __global__ void __launch_bounds__(256) graph_csr_kernel(const float* __restrict__ obs, int64_t obs_stride, int N, int n_graphs,
@@ -196,7 +196,7 @@ __global__ void __launch_bounds__(256) graph_csr_kernel(const float* __restrict_
   }
   __syncthreads();
   uint16_t* gp = csr_ptr + (size_t)g * (N + 1);
-  uint8_t* gs = csr_src + (size_t)g * N * kMaxNbr;
+  uint8_t* gs = csr_src + (size_t)g * csr_stride(N);
   for (int t = threadIdx.x; t <= N; t += blockDim.x) gp[t] = (uint16_t)s_ptr[t];
   if (adj_out) for (int t = threadIdx.x; t < N * W; t += blockDim.x) adj_out[(size_t)g * N * W + t] = s_mask[t];   // source masks per target
   for (int i = warp; i < N; i += nwarps) {
@@ -218,7 +218,7 @@ struct EdgeArgs {
   int64_t obs_stride;
   int N, H, n_graphs;
   const uint16_t* csr_ptr; // [graphs][N+1]
-  const uint8_t* csr_src;  // [graphs][N*32]
+  const uint8_t* csr_src;  // [graphs][csr_stride(N)]
   const float* ab;        // GATv2: [rows][2H] = (<att_h, x_l[row,h]>, <att_h, x_r[row,h]>) from the projection GEMM
   const uint32_t* row_key; // optional [rows]: P / ab are tables indexed by row_key[row] (discrete-feature mode), else by row
   const float* att;       // GATv2 [H*C]
@@ -308,8 +308,8 @@ __global__ void __launch_bounds__(EdgeCfg<TRANSFORMER>::kThreads, EdgeCfg<TRANSF
   float* s_dm = s_b + N;                                                         // [N]
   int* s_slot = reinterpret_cast<int*>(s_dm + N);                                // [N]
   float* poolbuf = reinterpret_cast<float*>(s_slot + N);                         // [warps][kC]  (16 B aligned: 4N floats before it)
-  uint8_t* s_src = reinterpret_cast<uint8_t*>(poolbuf + (a.pool_mode >= 0 ? kEdgeWarps * kC : 0));     // [N*32] (16 B aligned)
-  uint16_t* s_ptr = reinterpret_cast<uint16_t*>(s_src + N * kMaxNbr);            // [N+1]
+  uint8_t* s_src = reinterpret_cast<uint8_t*>(poolbuf + (a.pool_mode >= 0 ? kEdgeWarps * kC : 0));     // [csr_stride(N)] (16 B aligned)
+  uint16_t* s_ptr = reinterpret_cast<uint16_t*>(s_src + csr_stride(N));          // [N+1]
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   if (a.run_if_gt && *a.run_if_gt <= a.run_thresh) return;
   // one (graph, head) per CTA; the fallback launch behind the table kernel uses a small grid and strides
@@ -343,9 +343,9 @@ __global__ void __launch_bounds__(EdgeCfg<TRANSFORMER>::kThreads, EdgeCfg<TRANSF
       if (!compact) edge_cp_async16(sT32 + j * (kC * 2) + c * 16, row + tgt_col + c * 8);
     }
     {
-      const uint32_t sS32 = (uint32_t)__cvta_generic_to_shared(s_src);      // the graph's whole list block (N*32 bytes, 32 B aligned)
-      const uint8_t* gs = a.csr_src + cg * N * kMaxNbr;
-      for (int t = tid; t < N * 2; t += kEdgeThreads) edge_cp_async16(sS32 + t * 16, gs + t * 16);
+      const uint32_t sS32 = (uint32_t)__cvta_generic_to_shared(s_src);      // the graph's whole list block (16 B aligned)
+      const uint8_t* gs = a.csr_src + cg * csr_stride(N);
+      for (int t = tid; t < csr_stride(N) / 16; t += kEdgeThreads) edge_cp_async16(sS32 + t * 16, gs + t * 16);
     }
     const uint16_t* gp = a.csr_ptr + cg * (N + 1);
     for (int t = tid; t <= N; t += kEdgeThreads) s_ptr[t] = gp[t];
@@ -399,7 +399,7 @@ __global__ void __launch_bounds__(EdgeCfg<TRANSFORMER>::kThreads, EdgeCfg<TRANSF
     long long orow = (long long)(base + i);
     if (a.xrow_out) { orow = a.xrow_out[base + i]; if (orow < 0) continue; }
     const int r0 = s_ptr[i];
-    const int d = (int)s_ptr[i + 1] - r0 + self;            // warp uniform, <= 33
+    const int d = (int)s_ptr[i + 1] - r0 + self;            // warp uniform, <= kMaxList + 1
     const int ti = a.Pt ? tk : i;                           // row of the target side in stT / s_b
     float tg[8];                                            // the target's 8 channels stay in registers
     {
@@ -634,7 +634,7 @@ __global__ void ctrl_need_list_kernel(const uint8_t* __restrict__ ctrl_mask, con
   // graph's block starts 16-byte aligned, eabs[slot] = absolute position of the slot's first entry
   const size_t cg = graph_id ? (size_t)graph_id[(size_t)g * gid_stride] : (size_t)g;
   const uint16_t* gp = csr_ptr + cg * (N + 1);
-  const uint8_t* gs = csr_src + cg * N * kMaxNbr;
+  const uint8_t* gs = csr_src + cg * csr_stride(N);
   int etot = 0;
   int r0v[W], dv[W], offv[W];
 #pragma unroll
@@ -873,10 +873,10 @@ size_t carve_b(const MlsNetDesc* d, int Gc, unsigned char* base, WsB* ws) {
   const size_t o_qg = take((size_t)Gc * 8), o_idx = take(R * 4), o_slot = take(R * 4), o_cnt = take(16);
   const bool c2 = !hl && conv2_attn_supported(d->n_nodes, d->heads);
   const size_t o_eabs = take(c2 ? R * 4 : 0), o_gmeta = take(c2 ? (size_t)Gc * 32 : 0);
-  const size_t o_eent = take(c2 ? (R * (kMaxNbr + 1) + (size_t)Gc * 8 + 64) * 2 : 0);
+  const size_t o_eent = take(c2 ? (R * (kMaxList + 1) + (size_t)Gc * 8 + 64) * 2 : 0);   // sources + GATv2 self loop
   const size_t o_gf = take((size_t)Gc * 4), o_gc = take((size_t)Gc * 4);
   const size_t o_nidx = take(hl ? 0 : R * 4), o_xrow = take(hl ? 0 : R * 4), o_nf = take(hl ? 0 : (size_t)Gc * 4), o_nc = take(hl ? 0 : (size_t)Gc * 4);
-  const size_t o_cptr = take(((size_t)Gc * (d->n_nodes + 1) + 64) * 2), o_csrc = take((size_t)Gc * d->n_nodes * kMaxNbr + 64);
+  const size_t o_cptr = take(((size_t)Gc * (d->n_nodes + 1) + 64) * 2), o_csrc = take((size_t)Gc * csr_stride(d->n_nodes) + 64);
   const size_t o_adjm = take(hl ? 0 : (size_t)Gc * d->n_nodes * Wn * 4);
   const size_t o_ab = take(R * 2 * d->heads * 4);
   const size_t o_key = take(R * 4);
@@ -913,7 +913,7 @@ template <bool TR>
 int launch_edge(cudaStream_t st, const EdgeArgs& ea) {
   constexpr int kEdgeThreads = EdgeCfg<TR>::kThreads, kEdgeWarps = kEdgeThreads / 32;
   const size_t smem = (size_t)ea.N * kC * 2 * (TR ? 3 : 2) + (size_t)ea.N * 4 * 4 + (ea.pool_mode >= 0 ? kEdgeWarps * kC * 4 : 0) +
-                      ((size_t)ea.N + 1) * 2 + (size_t)ea.N * kMaxNbr + 16;
+                      ((size_t)ea.N + 1) * 2 + (size_t)csr_stride(ea.N) + 16;
   static size_t configured = 0;
   if (smem > 227 * 1024) {
     mls_set_error("bf16 attention kernel needs %zu bytes of shared memory for %d nodes (max 232448): use precision fp32", smem, ea.N);
@@ -964,7 +964,7 @@ size_t carve_cache(int N, int G, unsigned char* base, CsrCache* c) {
   const int Wn = mls_words_per_row(N);
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = al(off + bytes); return o; };
-  const size_t o_p = take(((size_t)G * (N + 1) + 64) * 2), o_s = take((size_t)G * N * kMaxNbr + 64), o_a = take((size_t)G * N * Wn * 4);
+  const size_t o_p = take(((size_t)G * (N + 1) + 64) * 2), o_s = take((size_t)G * csr_stride(N) + 64), o_a = take((size_t)G * N * Wn * 4);
   if (c) { c->ptr = reinterpret_cast<uint16_t*>(base + o_p); c->src = base + o_s; c->adjm = reinterpret_cast<uint32_t*>(base + o_a); }
   return off;
 }

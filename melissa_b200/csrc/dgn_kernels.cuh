@@ -22,6 +22,13 @@ namespace mls {
 
 constexpr int kC = 128;                 // channels per head the edge kernels are written for
 constexpr int kMaxNbr = 32;             // torch_cluster radius_graph max_num_neighbors
+// radius_graph(loop=False) keeps the first max_num_neighbors + 1 hits and then drops the self hit: a node that is not among
+// the first 33 hits of its own scan (index > 32 with more than 33 nodes in reach) keeps 33 sources, one more than
+// max_num_neighbors.  A source list therefore holds up to kMaxList entries (plus the GATv2 self loop where that is added).
+constexpr int kMaxList = kMaxNbr + 1;
+// bytes of one graph's CSR source lists (uint8 ids), a multiple of 16: N * 32 while no node can have 33 sources (N <= 33),
+// else N * 33 rounded up
+__host__ __device__ constexpr int csr_stride(int N) { return N <= kMaxList ? N * kMaxNbr : (N * kMaxList + 15) & ~15; }
 __device__ __forceinline__ float r2_threshold() { return (float)(0.2 * 0.2); }
 
 __device__ __forceinline__ float warp_sum(float v) {

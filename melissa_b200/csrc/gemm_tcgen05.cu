@@ -582,7 +582,7 @@ static int launch_bn(const CUtensorMap& ta, const CUtensorMap& tb, const CUtenso
     configured = true;
   }
   const int n_tiles = ((shape.M + kBM - 1) / kBM) * (shape.N / BN);
-  const int grid = n_tiles < sm_count ? n_tiles : sm_count;
+  const int grid = mls_cap_grid(n_tiles < sm_count ? n_tiles : sm_count);   // the tile loops take any grid
   if (grid <= 0) return MLS_OK;
   gemm_bf16_tcgen05_kernel<BN, MODE><<<grid, kGemmThreads, GemmSmem<BN>::kTotal, st>>>(ta, tb, ta2, shape, epi);
   mls_count_launch();
@@ -619,6 +619,8 @@ int gemm_bf16_launch(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, in
   if (rc) return rc;
   rc = make_tmap_bf16(&tb, B, shape.N, shape.K, ldb, BN);
   if (rc) return rc;
+  // tests/test_persistent_tiles_gpu.py reaches every instantiation below through these flag combinations and names the
+  // mode in its test ids: keep the two in step
   int mode = 0;
   if (split) mode = epi.dotvec ? 4 : 5;
   else if (!epi.Cf) {
@@ -656,7 +658,7 @@ int head_dueling_launch(const __nv_bfloat16* A, int lda, GemmShape shape, const 
     configured = true;
   }
   const int n_tiles = (shape.M + kBM - 1) / kBM;
-  head_dueling_tcgen05_kernel<<<n_tiles < sm_count ? n_tiles : sm_count, kGemmThreads, HeadSmem::kTotal, st>>>(ta, tb, ta2, tb1, shape, vec, out);
+  head_dueling_tcgen05_kernel<<<mls_cap_grid(n_tiles < sm_count ? n_tiles : sm_count), kGemmThreads, HeadSmem::kTotal, st>>>(ta, tb, ta2, tb1, shape, vec, out);
   mls_count_launch();
   MLS_LAUNCH_CHECK();
   return MLS_OK;
@@ -688,6 +690,24 @@ extern "C" int mls_test_gemm_bf16_ex(const void* A, const void* B, const float* 
   mls::GemmEpilogue epi{reinterpret_cast<__nv_bfloat16*>(C), N, bias, obs, obs_stride, nodes, relu, dotvec, dots, row_index, dotvec2, dots2,
                         dot_relu};
   return mls::gemm_bf16_launch(reinterpret_cast<const __nv_bfloat16*>(A), K, reinterpret_cast<const __nv_bfloat16*>(B), K, shape,
+                               epi, sms, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// Every option of the plain launch (tests/test_persistent_tiles_gpu.py): the above plus the fp32 output Cf and a second A
+// matrix for the K range [k2_lo, k2_hi) (A2 = NULL: none).
+extern "C" int mls_test_gemm_bf16_full(const void* A, int lda, const void* A2, int lda2, int k2_lo, int k2_hi, const void* B,
+                                       const float* bias, const float* obs, long long obs_stride, int nodes, const int* row_index,
+                                       const float* dotvec, const float* dotvec2, float* dots, float* dots2, int dot_relu, void* C,
+                                       float* Cf, int M, int N, int K, int relu, const int* m_dev, void* stream) {
+  int dev = 0, sms = 0;
+  MLS_CUDA(cudaGetDevice(&dev));
+  MLS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  mls::GemmShape shape{M, N, K, m_dev};
+  if (A2) { shape.A2 = reinterpret_cast<const __nv_bfloat16*>(A2); shape.lda2 = lda2; shape.k2_lo = k2_lo; shape.k2_hi = k2_hi; }
+  mls::GemmEpilogue epi{reinterpret_cast<__nv_bfloat16*>(C), N, bias, obs, obs_stride, nodes, relu, dotvec, dots, row_index, dotvec2, dots2,
+                        dot_relu};
+  epi.Cf = Cf; epi.ldcf = N;
+  return mls::gemm_bf16_launch(reinterpret_cast<const __nv_bfloat16*>(A), lda, reinterpret_cast<const __nv_bfloat16*>(B), K, shape,
                                epi, sms, reinterpret_cast<cudaStream_t>(stream));
 }
 

@@ -134,14 +134,19 @@ def test_forward_graphs_matches_oracle(kind, kw, N, B):
 
 
 def test_chunked_batches_and_many_graphs():
-    """More graphs than one workspace chunk: results must not depend on chunking."""
-    N, B = 20, 1500
+    """More graphs than one workspace chunk (32768 rows: 1638 graphs of 20 nodes): three passes, the last one partial;
+    results must not depend on chunking.  The oracle checks graphs on both sides of each pass boundary."""
+    import ctypes
+    from melissa_b200 import _lib
+    N, B = 20, 3400
     sd = _random_sd("l_dgn", 3)
     om = _obs_matrix(N, B, 13)
     cm = np.random.default_rng(3).random((B, N)) < 0.2
     m = _module("l_dgn", N, sd)
+    gc = _lib.lib().mls_dgn_chunk_graphs(ctypes.byref(m._desc()), B)
+    assert 2 * gc < B < 3 * gc, gc
     q, act = m.forward_graphs(torch.as_tensor(om, device="cuda"), torch.as_tensor(cm, device="cuda").to(torch.uint8))
-    sel = np.r_[0:40, 700:740, 1460:1500]
+    sel = np.r_[0:16, gc - 16:gc + 16, 2 * gc - 16:2 * gc + 16, B - 16:B]
     want = no.forward_graphs("l_dgn", sd, torch.as_tensor(om[sel]), torch.as_tensor(cm[sel]), N).numpy()
     _assert_q(q.cpu().numpy()[sel], want, "chunked")
 
@@ -233,22 +238,60 @@ def test_bf16_forward_graphs_within_stated_tolerance(kind, kw, N, B):
     np.testing.assert_array_equal(act[cm], (q[..., 1] > q[..., 0]).astype(np.int8)[cm])
 
 
+# runs in a child process: MLS_BF16_CHUNK_TILES is read once per process.  Prints the pass size, writes Q.
+_BF16_CHUNK_CHILD = """
+import sys, ctypes, numpy as np, torch
+sys.path.insert(0, sys.argv[1])
+from melissa_b200 import _lib
+from melissa_b200.networks import NETWORKS
+kind, N, d = sys.argv[2], int(sys.argv[3]), sys.argv[4]
+kw = dict(aggregator="max") if kind == "hl_dgn" else {}
+dueling = ({"hidden_sizes": [128, 128]}, {"hidden_sizes": [128, 128]})
+m = NETWORKS[kind](5, 128, 2, 4, N, dueling_param=dueling, device="cuda", **kw)
+m.load_state_dict(torch.load(d + "/sd.pt"))
+m = m.cuda().set_precision("bf16")
+rows = np.load(d + "/rows.npy")
+q, _ = m(rows)
+np.save(d + "/q.npy", q.cpu().numpy())
+print(_lib.lib().mls_dgn_chunk_graphs(ctypes.byref(m._desc()), rows.shape[0]))
+"""
+
+
 @pytest.mark.parametrize("kind", ["l_dgn", "dgn_r", "hl_dgn"])
-def test_bf16_agent_rows_and_chunking(kind):
-    N, bs = 50, 900           # more graphs than one bf16 workspace chunk (378 graphs at N=50)
+def test_bf16_agent_rows_and_chunking(kind, tmp_path):
+    """Agent rows through the bf16 path, in one pass and, in a child process with 40-tile passes (102 graphs of 50 nodes),
+    in nine: every pass computes its graphs with the same kernels, tiles and reductions, so Q must not change in any bit."""
+    import ctypes
+    import os
+    import subprocess
+    import sys
+    from melissa_b200 import _lib
+    N, bs = 50, 900
     kw = dict(aggregator="max") if kind == "hl_dgn" else {}
     sd = _random_sd(kind, 61)
     om = _obs_matrix(N, bs, 29)
     ctrl = np.random.default_rng(7).integers(0, N, size=bs).astype(np.float32)
     rows = np.concatenate([om.reshape(bs, -1), ctrl[:, None]], axis=1)
-    sel = np.r_[0:16, 370:390, 884:900]
+    sel = np.r_[0:16, 94:110, 196:212, 884:900]
     want = no.FORWARDS[kind](sd, torch.as_tensor(rows[sel]), N, **kw).numpy()
     m = _module(kind, N, sd, **kw).set_precision("bf16")
+    assert _lib.lib().mls_dgn_chunk_graphs(ctypes.byref(m._desc()), bs) == bs      # one pass in this process
     q, _ = m(rows)
     q = q.cpu().numpy()
     scale = max(1.0, float(np.abs(want).max()))
     assert float(np.abs(q[sel] - want).max()) <= BF16_TOL * scale
     assert np.isfinite(q).all()
+    torch.save(sd, tmp_path / "sd.pt")
+    np.save(tmp_path / "rows.npy", rows)
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = dict(os.environ, MLS_BF16_CHUNK_TILES="40")
+    res = subprocess.run([sys.executable, *(["-s"] if sys.flags.no_user_site else []), "-c", _BF16_CHUNK_CHILD, root, kind, str(N),
+                          str(tmp_path)], env=env, capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0, res.stderr[-3000:]
+    gc = int(res.stdout.split()[-1])
+    assert gc < bs and gc == 40 * 128 // N, gc
+    q_chunked = np.load(tmp_path / "q.npy")
+    assert np.array_equal(q_chunked.view(np.uint32), q.view(np.uint32)), float(np.abs(q_chunked - q).max())
 
 
 def test_large_graphs_200_nodes():
