@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define MLS_VERSION 211
+#define MLS_VERSION 212
 #define MLS_MAX_NODES 256
 
 /* ---- errors ------------------------------------------------------------------------- */
@@ -369,6 +369,23 @@ int mls_transformer_edge_fwd(const float* k, const float* v, int64_t lds, const 
 int mls_transformer_edge_bwd(const float* k, const float* v, int64_t lds, const float* q, int64_t ldq, const int32_t* tgt_row,
                              const int32_t* src_row, const int32_t* src_cnt, int32_t n_targets, int32_t heads,
                              const float* alpha, const float* dout, float* d_k, float* d_v, float* d_q, void* stream);
+
+/* ---- bf16 training precision of the dense layers (melissa_b200/csrc/train_linear.cu; DGNBase.set_train_precision("bf16")).
+ * torch.nn.Linear forward and backward with bf16 operands, fp32 accumulation on the tcgen05 GEMM and fp32 everywhere else
+ * (fp32 master weights, fp32 activations between layers).  x [rows][in] (row stride ldx), W [out][in] contiguous:
+ *   y  = fp32acc(bf16(x) . bf16(W)^T) + b       (b added in fp32 in the GEMM epilogue; b NULL: none)
+ *   dx = fp32acc(bf16(dy) . bf16(W))            (dx NULL: not computed)
+ *   dW = fp32acc(bf16(dy)^T . bf16(x))
+ *   db = sum over rows of dy in fp32, from the unrounded dy      (db NULL: not computed)
+ * No atomics: the results are bitwise reproducible.  rows = 0 launches nothing; the backward then writes dW = 0, db = 0.
+ * The caller provides scratch of mls_linear_bf16_workspace_bytes(rows, in, out) bytes on a 256-byte boundary (NULL ok
+ * when rows = 0); the library allocates nothing. */
+size_t mls_linear_bf16_workspace_bytes(int64_t rows, int32_t in, int32_t out);
+int mls_linear_bf16_fwd(const float* x, int64_t ldx, const float* w, const float* b, int64_t rows, int32_t in, int32_t out,
+                        float* y, int64_t ldy, void* workspace, size_t workspace_bytes, void* stream);
+int mls_linear_bf16_bwd(const float* x, int64_t ldx, const float* w, const float* dy, int64_t lddy, int64_t rows, int32_t in,
+                        int32_t out, float* dx, int64_t lddx, float* dw, float* db, void* workspace, size_t workspace_bytes,
+                        void* stream);
 
 /* ---- prioritized replay (melissa_b200/csrc/replay_per.cu).  Replaces tianshou PrioritizedReplayBuffer's numpy
  * SegmentTree (init_weight / sample_indices / get_weight / update_weight) for the device replay ring.

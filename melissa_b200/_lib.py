@@ -94,7 +94,8 @@ EXPORTS = ["mls_version", "mls_last_error", "mls_device_info", "mls_words_per_ro
            "mls_dgn_csr_cache_bytes", "mls_dgn_csr_cache_build", "mls_obs_pack", "mls_obs_unpack", "mls_nstep_returns",
            "mls_adam_step", "mls_train_list_capacity", "mls_train_lists", "mls_gatv2_edge_fwd", "mls_gatv2_edge_bwd_blocks",
            "mls_gatv2_edge_bwd", "mls_transformer_edge_fwd", "mls_transformer_edge_bwd", "mls_per_tree_size",
-           "mls_per_build", "mls_per_sample", "mls_per_update"]
+           "mls_per_build", "mls_per_sample", "mls_per_update", "mls_linear_bf16_workspace_bytes", "mls_linear_bf16_fwd",
+           "mls_linear_bf16_bwd"]
 PACKED_NODE_BYTES = 12
 
 _lib = None
@@ -153,6 +154,11 @@ def lib():
     L.mls_per_sample.argtypes = [vp, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, vp, C.c_int32, vp, vp, vp, vp, vp]
     L.mls_per_update.argtypes = [vp, C.c_int32, C.c_int64, C.c_int32, vp, vp, vp, vp, C.c_int32, C.c_double, C.c_double,
                                  vp, vp, vp]
+    L.mls_linear_bf16_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.c_int32]
+    L.mls_linear_bf16_workspace_bytes.restype = C.c_size_t
+    L.mls_linear_bf16_fwd.argtypes = [vp, C.c_int64, vp, vp, C.c_int64, C.c_int32, C.c_int32, vp, C.c_int64, vp, C.c_size_t, vp]
+    L.mls_linear_bf16_bwd.argtypes = [vp, C.c_int64, vp, vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, vp, C.c_int64, vp, vp, vp,
+                                      C.c_size_t, vp]
     for name in EXPORTS:
         getattr(L, name)
     _lib = L

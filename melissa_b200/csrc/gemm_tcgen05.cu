@@ -69,10 +69,19 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     n_mt = (Mt + kBM - 1) / kBM;
     n_ns = (shape.N - t_w) / BN;
   }
-  const int n_tiles = kSplit ? n_mt * n_n + max(n_m - n_mt, 0) * n_ns : n_m * n_n;
+  const int n_base = kSplit ? n_mt * n_n + max(n_m - n_mt, 0) * n_ns : n_m * n_n;
+  const int n_ks = MODE == 0 && shape.k_split > 1 ? shape.k_split : 1;    // split-K: work item = tile + n_base * range
+  const int n_tiles = n_base * n_ks;
   const int n_kb = shape.K / kBK;
+  // K blocks [kb0, kb1) of a work item
+  auto k_range = [&](int tile, int& kb0, int& kb1) {
+    const int ks = n_ks > 1 ? tile / n_base : 0;
+    kb0 = (int)((long long)ks * n_kb / n_ks);
+    kb1 = (int)((long long)(ks + 1) * n_kb / n_ks);
+  };
   // tile -> first row, first (packed) column; true for a target column tile
   auto tile_at = [&](int tile, int& m0, int& n0) -> bool {
+    if (n_ks > 1) tile %= n_base;
     if (!kSplit || tile < n_mt * n_n) { m0 = (tile / n_n) * kBM; n0 = (tile % n_n) * BN; return kSplit && n0 >= shape.t_lo && n0 < shape.t_hi; }
     else {
       const int t = tile - n_mt * n_n;
@@ -105,7 +114,9 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         int m0, n0;
         const bool tgt = tile_at(tile, m0, n0);
-        for (int kb = 0; kb < n_kb; ++kb) {
+        int kb0, kb1;
+        k_range(tile, kb0, kb1);
+        for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1);
           const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
           mbar_expect_tx(full_bar(stage), S::kStageBytes);
@@ -130,14 +141,16 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         mbar_wait(tempty_bar(acc), acc_phase ^ 1);          // epilogue has drained this accumulator
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)(acc * BN);
-        for (int kb = 0; kb < n_kb; ++kb) {
+        int kb0, kb1;
+        k_range(tile, kb0, kb1);
+        for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(full_bar(stage), phase);                // TMA bytes have landed
           tc_fence_after();
           const uint32_t sa = smem_u32(smem + stage * S::kStageBytes);
           const uint64_t da = make_smem_desc(sa), db = make_smem_desc(sa + S::kABytes);
 #pragma unroll
           for (int k = 0; k < kBK / kUmmaK; ++k)            // +32 B per K=16 step inside the swizzle atom
-            umma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, (kb | k) ? 1u : 0u);
+            umma_bf16(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, ((kb - kb0) | k) ? 1u : 0u);
           umma_commit(empty_bar(stage));                    // frees the smem slot when these MMAs retire
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
@@ -246,7 +259,8 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
           }
           if (relu) { x0 = fmaxf(x0, 0.f); x1 = fmaxf(x1, 0.f); x2 = fmaxf(x2, 0.f); x3 = fmaxf(x3, 0.f); }
           if (has_cf && r < Mr)                                // lane = row: 16-byte stores, 128 contiguous bytes per lane and chunk
-            *reinterpret_cast<float4*>(epi.Cf + (size_t)r * epi.ldcf + n0 + c0 + j) = make_float4(x0, x1, x2, x3);
+            *reinterpret_cast<float4*>(epi.Cf + (n_ks > 1 ? (tile / n_base) * epi.cf_split_stride : 0) + (size_t)r * epi.ldcf + n0 + c0 + j) =
+                make_float4(x0, x1, x2, x3);
           if (!has_c) {
           } else if (epi.c_fp16) {
             asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(packed[j >> 1]) : "f"(x1), "f"(x0));
@@ -581,7 +595,7 @@ static int launch_bn(const CUtensorMap& ta, const CUtensorMap& tb, const CUtenso
     MLS_CUDA(cudaFuncSetAttribute(gemm_bf16_tcgen05_kernel<BN, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmSmem<BN>::kTotal));
     configured = true;
   }
-  const int n_tiles = ((shape.M + kBM - 1) / kBM) * (shape.N / BN);
+  const int n_tiles = ((shape.M + kBM - 1) / kBM) * (shape.N / BN) * (MODE == 0 && shape.k_split > 1 ? shape.k_split : 1);
   const int grid = mls_cap_grid(n_tiles < sm_count ? n_tiles : sm_count);   // the tile loops take any grid
   if (grid <= 0) return MLS_OK;
   gemm_bf16_tcgen05_kernel<BN, MODE><<<grid, kGemmThreads, GemmSmem<BN>::kTotal, st>>>(ta, tb, ta2, shape, epi);
@@ -607,6 +621,10 @@ int gemm_bf16_launch(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, in
   } else {
     shape.t_lo = shape.t_hi = 0;
   }
+  if (shape.k_split > 1)
+    MLS_CHECK_ARG(!split && epi.Cf && !epi.C && !epi.bias && !epi.obs && !epi.dotvec && !epi.relu && shape.k_split <= shape.K / kBK &&
+                      epi.cf_split_stride % 4 == 0,
+                  "split-K GEMM: fp32 output only, without epilogue options, and at most one range per 64-wide K block");
   if (shape.M <= 0) return MLS_OK;
   if (epi.dotvec) {                                         // the epilogue accumulates two partial sums per cell
     const int t_w = shape.t_hi - shape.t_lo;

@@ -52,6 +52,8 @@ struct GemmEpilogue {
   int ldct;
   float* dots_t;
   const int* row_index_t;
+  // split-K (GemmShape::k_split > 1): partial product s goes to Cf + s * cf_split_stride
+  long long cf_split_stride;
 };
 
 struct GemmShape {
@@ -68,6 +70,10 @@ struct GemmShape {
   // and the second A matrix, if given, applies to the target columns only.
   const int* m_dev_t;
   int t_lo, t_hi;
+  // optional split of K into k_split ranges of whole 64-wide blocks (0 / 1: none; fp32 output Cf only, no bias): every
+  // (tile, range) pair is a work item and writes its partial product to its own Cf slice; the caller adds the slices up.
+  // Gives weight-gradient products (M, N of a few tiles, K = the batch's rows) enough work items to fill the GPU.
+  int k_split;
 };
 
 size_t gemm_smem_bytes(int BN);

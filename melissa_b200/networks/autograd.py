@@ -10,14 +10,16 @@ rather than PyG's: one agent observation controls ONE node, so only the rows tha
     conv2 at the controlling node c          <- sources  S1 = {c} + radius-neighbours(c)
     conv1 at the nodes of S1 (x1 rows)       <- sources  S2 = S1 + their radius-neighbours
 
-as edge lists over (sample, target, source) triples with scatter softmax; the dense layers are plain ``F.linear``.
-Runs wherever the parameters live (the training loop keeps them on the GPU).
+as edge lists over (sample, target, source) triples with scatter softmax; the dense layers are plain ``F.linear``, or with
+``net.set_train_precision("bf16")`` the bf16 tensor-core Function ``_LinearBF16``.
+Runs wherever the parameters live (the training loop keeps them on the GPU; bf16 training precision needs CUDA tensors).
 """
 from __future__ import annotations
 
 import math
 
 import torch
+import torch.nn as nn
 import torch.nn.functional as F
 
 R2 = float(torch.tensor(0.2, dtype=torch.float64).pow(2).to(torch.float32))     # torch_cluster: r*r narrowed to fp32
@@ -80,7 +82,7 @@ def _used_rows(n_rows, *index_lists):
     return rows, remap
 
 
-def _gatv2(conv, x, edges, heads, N):
+def _gatv2(conv, x, edges, heads, N, lin):
     """PyG GATv2Conv(concat=True, negative_slope=0.2, add_self_loops=True, share_weights=False) on an edge list.
     x [bs, N, D]; returns [bs*N, H*C] with rows of non-target nodes = bias only (never read)."""
     sm, ti, sj = edges
@@ -90,8 +92,8 @@ def _gatv2(conv, x, edges, heads, N):
     xf = x.reshape(bs * N, -1)
     rows_s, map_s = _used_rows(bs * N, src)
     rows_t, map_t = _used_rows(bs * N, tgt)
-    xl = conv.lin_l(xf[rows_s]).view(-1, heads, C)[map_s[src]]               # [E, H, C] source side
-    xr = conv.lin_r(xf[rows_t]).view(-1, heads, C)[map_t[tgt]]               # [E, H, C] target side
+    xl = lin(conv.lin_l, xf[rows_s]).view(-1, heads, C)[map_s[src]]          # [E, H, C] source side
+    xr = lin(conv.lin_r, xf[rows_t]).view(-1, heads, C)[map_t[tgt]]          # [E, H, C] target side
     s = F.leaky_relu(xl + xr, 0.2)
     e = (s * conv.att.view(1, heads, C)).sum(-1)
     a = _segment_softmax(e, tgt, bs * N)
@@ -99,7 +101,7 @@ def _gatv2(conv, x, edges, heads, N):
     return out.view(bs * N, heads * C) + conv.bias
 
 
-def _transformer(conv, x, edges, heads, N):
+def _transformer(conv, x, edges, heads, N, lin):
     """PyG TransformerConv(root_weight=False, beta=False): no self loops, no output bias, ``lin_skip`` unused."""
     sm, ti, sj = edges
     bs = x.shape[0]
@@ -109,25 +111,93 @@ def _transformer(conv, x, edges, heads, N):
     xf = x.reshape(bs * N, -1)
     rows_s, map_s = _used_rows(bs * N, src)
     rows_t, map_t = _used_rows(bs * N, tgt)
-    q = conv.lin_query(xf[rows_t]).view(-1, heads, C)[map_t[tgt]]
-    k = conv.lin_key(xf[rows_s]).view(-1, heads, C)[map_s[src]]
-    v = conv.lin_value(xf[rows_s]).view(-1, heads, C)[map_s[src]]
+    q = lin(conv.lin_query, xf[rows_t]).view(-1, heads, C)[map_t[tgt]]
+    k = lin(conv.lin_key, xf[rows_s]).view(-1, heads, C)[map_s[src]]
+    v = lin(conv.lin_value, xf[rows_s]).view(-1, heads, C)[map_s[src]]
     e = (q * k).sum(-1) / math.sqrt(C)
     a = _segment_softmax(e, tgt, bs * N)
     out = torch.zeros(bs * N, heads, C, dtype=x.dtype, device=x.device).index_add_(0, tgt, a[:, :, None] * v)
     return out.view(bs * N, HC)
 
 
-def _mlp(params, x):
-    return params.model(x)
+def _mlp(params, x, lin):
+    for m in params.model:
+        x = lin(m, x) if isinstance(m, nn.Linear) else m(x)
+    return x
 
 
-def _dueling(net, z):
+def _dueling(net, z, lin):
     if not net.use_dueling:
-        return net.out_linear(z)
-    q = _mlp(net.Q, z)
-    v = _mlp(net.V, z)
+        return lin(net.out_linear, z)
+    q = _mlp(net.Q, z, lin)
+    v = _mlp(net.V, z, lin)
     return q - q.mean(dim=1, keepdim=True) + v
+
+
+def _require_f32_cuda(what, *tensors):
+    """The CUDA training Functions read their operands as fp32 device memory: refuse anything else before any launch
+    (under torch.autocast the dense layers would hand them bf16 tensors of half the expected size)."""
+    for t in tensors:
+        if t.dtype != torch.float32 or not t.is_cuda:
+            from .. import _lib
+            raise _lib.MelissaLibraryError(
+                f"{what} takes float32 CUDA tensors, got {t.dtype} on {t.device}; there is no CPU path, and mixed-precision "
+                'training is net.set_train_precision("bf16") (bf16 tensor-core GEMMs, fp32 weights), not torch.autocast')
+
+
+class _LinearBF16(torch.autograd.Function):
+    """nn.Linear in bf16 training precision (``mls_linear_bf16_fwd`` / ``_bwd``, ``csrc/train_linear.cu``): bf16 operands,
+    fp32 accumulation on the tcgen05 GEMM, fp32 in and out.  y = bf16(x) bf16(W)^T + b, dx = bf16(dy) bf16(W),
+    dW = bf16(dy)^T bf16(x), db = sum of the unrounded dy over rows; dx only when autograd asks for it."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias):
+        _require_f32_cuda("the bf16 linear layer", x, weight, *(() if bias is None else (bias,)))
+        from .. import _lib
+        L = _lib.lib()
+        out_f, in_f = weight.shape
+        x2 = x.reshape(-1, in_f)
+        if x2.stride(1) != 1 or x2.stride(0) < in_f:
+            x2 = x2.contiguous()
+        w = weight.contiguous()
+        rows = x2.shape[0]
+        y = torch.empty(rows, out_f, dtype=torch.float32, device=x.device)
+        if rows:
+            ws = torch.empty(L.mls_linear_bf16_workspace_bytes(rows, in_f, out_f), dtype=torch.uint8, device=x.device)
+            _lib.check(L.mls_linear_bf16_fwd(x2.data_ptr(), x2.stride(0), w.data_ptr(), None if bias is None else bias.data_ptr(),
+                                             rows, in_f, out_f, y.data_ptr(), out_f, ws.data_ptr(), ws.numel(),
+                                             _lib.current_stream_ptr()))
+        ctx.save_for_backward(x2, w)
+        ctx.has_bias, ctx.x_shape = bias is not None, x.shape
+        return y.view(*x.shape[:-1], out_f)
+
+    @staticmethod
+    def backward(ctx, dy):
+        from .. import _lib
+        L = _lib.lib()
+        x2, w = ctx.saved_tensors
+        out_f, in_f = w.shape
+        rows = x2.shape[0]
+        dy2 = dy.reshape(-1, out_f)
+        if dy2.stride(1) != 1 or dy2.stride(0) < out_f:
+            dy2 = dy2.contiguous()
+        need_dx, _, need_db = ctx.needs_input_grad
+        dev = x2.device
+        dx = torch.empty(rows, in_f, dtype=torch.float32, device=dev) if need_dx else None
+        dw = torch.empty(out_f, in_f, dtype=torch.float32, device=dev)
+        db = torch.empty(out_f, dtype=torch.float32, device=dev) if (ctx.has_bias and need_db) else None
+        ws = torch.empty(max(1, L.mls_linear_bf16_workspace_bytes(rows, in_f, out_f)), dtype=torch.uint8, device=dev)
+        _lib.check(L.mls_linear_bf16_bwd(x2.data_ptr(), x2.stride(0), w.data_ptr(), dy2.data_ptr(), dy2.stride(0), rows, in_f, out_f,
+                                         None if dx is None else dx.data_ptr(), in_f, dw.data_ptr(),
+                                         None if db is None else db.data_ptr(), ws.data_ptr(), ws.numel(), _lib.current_stream_ptr()))
+        return None if dx is None else dx.view(ctx.x_shape), dw, db
+
+
+def _linear_op(net):
+    """How ``net``'s dense layers are evaluated in training: ``layer(x)`` (fp32) or through ``_LinearBF16``."""
+    if net.train_precision == "bf16":
+        return lambda layer, x: _LinearBF16.apply(x, layer.weight, layer.bias)
+    return lambda layer, x: layer(x)
 
 
 class _GATv2Edge(torch.autograd.Function):
@@ -136,6 +206,7 @@ class _GATv2Edge(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, xl, xr, att, tgt_row, src_row, src_cnt):
+        _require_f32_cuda("the GATv2 edge phase", xl, xr, att)
         from .. import _lib
         L = _lib.lib()
         xl, xr, att = xl.contiguous(), xr.contiguous(), att.contiguous()
@@ -169,6 +240,7 @@ class _TransformerEdge(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, q, k, v, tgt_row, src_row, src_cnt):
+        _require_f32_cuda("the TransformerConv edge phase", q, k, v)
         from .. import _lib
         L = _lib.lib()
         q, k, v = q.contiguous(), k.contiguous(), v.contiguous()
@@ -222,14 +294,15 @@ def train_lists(obs_rows: torch.Tensor, n_agents: int):
 def q_values_l_dgn_fused(net, obs_rows: torch.Tensor) -> torch.Tensor:
     """L-DGN / DGN-R Q-values with the two attention edge phases (and their backward) on the CUDA kernels of
     ``csrc/train_gatv2.cu``; same math as ``q_values_torch`` (``l_dgn.py:92-151``, ``dgn_r.py:82-129``), dense layers through
-    ``F.linear``.  CUDA tensors only."""
+    ``F.linear`` or ``_LinearBF16`` (training precision).  CUDA tensors only."""
     N, heads = net.agents_num, net.num_heads
     tr = net.KIND == "dgn_r"
+    lin = _linear_op(net)
 
     def conv(c, x_src, x_tgt, tgt, src, cnt):
         if tr:
-            return _TransformerEdge.apply(c.lin_query(x_tgt), c.lin_key(x_src), c.lin_value(x_src), tgt, src, cnt)
-        return _GATv2Edge.apply(c.lin_l(x_src), c.lin_r(x_tgt), c.att.view(-1), tgt, src, cnt) + c.bias
+            return _TransformerEdge.apply(lin(c.lin_query, x_tgt), lin(c.lin_key, x_src), lin(c.lin_value, x_src), tgt, src, cnt)
+        return _GATv2Edge.apply(lin(c.lin_l, x_src), lin(c.lin_r, x_tgt), c.att.view(-1), tgt, src, cnt) + c.bias
 
     pos, feats, dm, ctrl = split_rows(obs_rows, N, net.input_dim)
     bs, dev = obs_rows.shape[0], obs_rows.device
@@ -239,7 +312,7 @@ def q_values_l_dgn_fused(net, obs_rows: torch.Tensor) -> torch.Tensor:
     rows_u = torch.nonzero(used, as_tuple=True)[0]
     remap = torch.zeros(bs * N, dtype=torch.int32, device=dev)
     remap[rows_u] = torch.arange(rows_u.numel(), dtype=torch.int32, device=dev)
-    x0 = F.relu(_mlp(net.encoder, feats.reshape(bs * N, -1)[rows_u]))          # [used rows, hid]
+    x0 = F.relu(_mlp(net.encoder, feats.reshape(bs * N, -1)[rows_u], lin))     # [used rows, hid]
     tgt_l = tgt_row.long()
     tgt_u = remap[tgt_l].long()                                                 # a slot's node is its own first source
     # conv1 at the S1 slots: sources are (used) node rows, targets the slots' own nodes
@@ -254,7 +327,7 @@ def q_values_l_dgn_fused(net, obs_rows: torch.Tensor) -> torch.Tensor:
     src2 = torch.where(torch.arange(cap, device=dev)[None, :] < s1_cnt[:, None], src2, torch.zeros_like(src2)).contiguous()
     ar_b = torch.arange(bs, dtype=torch.int32, device=dev)
     x2 = F.relu(conv(net.conv2, x1m, x1m[ctrl_slot], ar_b, src2, s1_cnt))                                      # [bs, HC]
-    return _dueling(net, torch.cat([snap1, snap2, x2], dim=1))
+    return _dueling(net, torch.cat([snap1, snap2, x2], dim=1), lin)
 
 
 def q_values_hl_dgn_fused(net, obs_rows: torch.Tensor) -> torch.Tensor:
@@ -263,6 +336,7 @@ def q_values_hl_dgn_fused(net, obs_rows: torch.Tensor) -> torch.Tensor:
     from .. import _lib
     L = _lib.lib()
     N = net.agents_num
+    lin = _linear_op(net)
     pos, feats, dm, ctrl = split_rows(obs_rows, N, net.input_dim)
     obs_c = obs_rows.contiguous().float()
     bs, dev = obs_rows.shape[0], obs_rows.device
@@ -272,12 +346,12 @@ def q_values_hl_dgn_fused(net, obs_rows: torch.Tensor) -> torch.Tensor:
     src_cnt = torch.empty(bs * N, dtype=torch.int32, device=dev)
     _lib.check(L.mls_train_lists(obs_c.data_ptr(), obs_c.shape[1], bs, N, R2, 2, None, None, tgt_row.data_ptr(), src_row.data_ptr(),
                                  src_cnt.data_ptr(), None, _lib.current_stream_ptr()))
-    x0 = F.relu(_mlp(net.encoder, feats.reshape(bs * N, -1)))
-    out = _GATv2Edge.apply(net.conv1.lin_l(x0), net.conv1.lin_r(x0), net.conv1.att.view(-1), tgt_row, src_row, src_cnt)
+    x0 = F.relu(_mlp(net.encoder, feats.reshape(bs * N, -1), lin))
+    out = _GATv2Edge.apply(lin(net.conv1.lin_l, x0), lin(net.conv1.lin_r, x0), net.conv1.att.view(-1), tgt_row, src_row, src_cnt)
     x1 = F.relu(out + net.conv1.bias).view(bs, N, -1) * dm
     agg = net.aggregator_name
     z = x1.amax(dim=1) if agg == "max" else (x1.mean(dim=1) if agg == "mean" else x1.sum(dim=1))
-    return _dueling(net, z)
+    return _dueling(net, z, lin)
 
 
 def fused_training_available(net, obs_rows) -> bool:
@@ -299,24 +373,25 @@ def q_values_torch(net, obs_rows: torch.Tensor) -> torch.Tensor:
     N, heads = net.agents_num, net.num_heads
     pos, feats, dm, ctrl = split_rows(obs_rows, N, net.input_dim)
     bs = obs_rows.shape[0]
+    lin = _linear_op(net)
     mask = radius_mask(pos)
     ar = torch.arange(bs, device=obs_rows.device)
-    x0 = F.relu(_mlp(net.encoder, feats))                                       # [bs, N, hid]
+    x0 = F.relu(_mlp(net.encoder, feats, lin))                                  # [bs, N, hid]
     kind = net.KIND
     if kind == "hl_dgn":
         every = torch.ones(bs, N, dtype=torch.bool, device=obs_rows.device)
-        x1 = F.relu(_gatv2(net.conv1, x0, _edges(mask, every, True), heads, N)).view(bs, N, -1) * dm
+        x1 = F.relu(_gatv2(net.conv1, x0, _edges(mask, every, True), heads, N, lin)).view(bs, N, -1) * dm
         agg = net.aggregator_name
         z = x1.amax(dim=1) if agg == "max" else (x1.mean(dim=1) if agg == "mean" else x1.sum(dim=1))
-        return _dueling(net, z)
+        return _dueling(net, z, lin)
     tr = kind == "dgn_r"
     conv = _transformer if tr else _gatv2
     is_ctrl = torch.zeros(bs, N, dtype=torch.bool, device=obs_rows.device)
     is_ctrl[ar, ctrl] = True
     s1 = is_ctrl | mask[ar, ctrl]                                               # conv2 sources = conv1 targets
-    x1 = F.relu(conv(net.conv1, x0, _edges(mask, s1, not tr), heads, N)).view(bs, N, -1)
+    x1 = F.relu(conv(net.conv1, x0, _edges(mask, s1, not tr), heads, N, lin)).view(bs, N, -1)
     snap1, snap2 = x0[ar, ctrl], x1[ar, ctrl]                                   # x1 snapshot is taken BEFORE the dm mask
     x1 = x1 * dm
-    x2 = F.relu(conv(net.conv2, x1, _edges(mask, is_ctrl, not tr), heads, N)).view(bs, N, -1)
+    x2 = F.relu(conv(net.conv2, x1, _edges(mask, is_ctrl, not tr), heads, N, lin)).view(bs, N, -1)
     z = torch.cat([snap1, snap2, x2[ar, ctrl]], dim=1)
-    return _dueling(net, z)
+    return _dueling(net, z, lin)

@@ -110,6 +110,7 @@ class DGNBase(nn.Module):
         self.edge_attributes = edge_attributes      # accepted; no effect on results (convs get no edge_attr)
         self.use_dueling = dueling_param is not None
         self.precision = "fp32"
+        self.train_precision = "fp32"
         self._ws = _Workspace()
         self._prepared = None
 
@@ -139,6 +140,16 @@ class DGNBase(nn.Module):
         if precision not in _lib.PRECISIONS:
             raise ValueError(precision)
         self.precision = precision
+        return self
+
+    def set_train_precision(self, precision: str):
+        """Precision of the dense layers in the differentiable training forward and its backward
+        (``networks/autograd.py``): "fp32" (default) or "bf16" -- bf16 operands, fp32 accumulation on the tensor cores,
+        fp32 master weights and fp32 activations between layers (``mls_linear_bf16_*``; CUDA tensors only).
+        Independent of :meth:`set_precision`, which selects the rollout forward."""
+        if precision not in ("fp32", "bf16"):
+            raise ValueError(precision)
+        self.train_precision = precision
         return self
 
     def _desc(self):
