@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define MLS_VERSION 212
+#define MLS_VERSION 213
 #define MLS_MAX_NODES 256
 
 /* ---- errors ------------------------------------------------------------------------- */
@@ -42,7 +42,8 @@ int mls_words_per_row(int n_nodes);
  *   "attn_mma"  1 = conv1 attention through the pair-logit table + tcgen05 aggregation (discrete-feature mode)
  *   "conv2_mma" 1 = conv2 attention with half2 logits + tcgen05 aggregation (graphs of <= 64 nodes)
  *   "max_ctas"  test only: n > 0 caps the grid of the persistent kernels at n CTAs (many tiles per CTA); 0 = off
- * get returns -1 for an unknown key. */
+ * set returns MLS_ERR_INVALID and get returns -1 for an unknown key (since version 213 also for the two removed
+ * switches of the conv1 kernel choice and the needed-row layout). */
 int mls_set_option(const char* key, int value);
 int mls_get_option(const char* key);
 /* kernels launched by this library since it was loaded (process wide; for bench accounting). */

@@ -35,34 +35,21 @@ extern "C" int mls_device_info(int32_t* sm_count, int32_t* cc_major, int32_t* cc
 //   "attn_mma":  1 = in discrete-feature mode run conv1's attention through the pair-logit table and the tensor-core
 //                aggregation kernel (attn_table.cu); 0 = gather kernel only
 //   "conv2_mma": 1 = conv2 attention with half2 logits + tensor-core aggregation (conv2_attn.cu); 0 = gather kernel
-//   "attn_hp":   2 = conv1 table kernel fed by per-tile records of a pre-pass, row-major output (default); 1 = (tile, head pair)
-//                items built in the kernel, channel-major output staged through shared memory; 0 = (tile) items, two stages
-//   "ctrl_first": 1 = bf16 forward of L-DGN / DGN-R: the needed rows are ordered [controlling nodes by slot][others], relu(conv1)
-//                of a controlling node is written once (x1 row = snapshot row; the heads' GEMM reads the snapshot columns from
-//                x1); 0 = needed rows in node order per graph + a separate snapshot copy in z
 //   "fp32_tc":   1 = precision fp32 runs its dense layers on the tensor cores through 3-way bf16 operand splits
 //                (fp32-grade, dgn_forward.cu); 0 = SIMT sgemm
 //   "max_ctas":  test only: n > 0 caps the grid of the persistent kernels (the tcgen05 GEMM and fused dueling heads, conv2
 //                attention, the conv1 table kernels) at n CTAs, so that small inputs give every CTA many tiles; 0 = off
 #include <stdlib.h>
 #include <string.h>
-static int g_attn_mma = -1, g_conv2_mma = -1, g_fp32_tc = -1, g_attn_hp = -1, g_ctrl_first = -1, g_max_ctas = -1;
+static int g_attn_mma = -1, g_conv2_mma = -1, g_fp32_tc = -1, g_max_ctas = -1;
 extern "C" int mls_get_option(const char* key) {
   if (key && !strcmp(key, "attn_mma")) {
     if (g_attn_mma < 0) { const char* e = getenv("MLS_ATTN_MMA"); g_attn_mma = e ? atoi(e) : 1; }
     return g_attn_mma;
   }
-  if (key && !strcmp(key, "attn_hp")) {
-    if (g_attn_hp < 0) { const char* e = getenv("MLS_ATTN_HP"); g_attn_hp = e ? atoi(e) : 2; }
-    return g_attn_hp;
-  }
   if (key && !strcmp(key, "fp32_tc")) {
     if (g_fp32_tc < 0) { const char* e = getenv("MLS_FP32_TC"); g_fp32_tc = e ? atoi(e) : 1; }
     return g_fp32_tc;
-  }
-  if (key && !strcmp(key, "ctrl_first")) {
-    if (g_ctrl_first < 0) { const char* e = getenv("MLS_CTRL_FIRST"); g_ctrl_first = e ? atoi(e) : 1; }
-    return g_ctrl_first;
   }
   if (key && !strcmp(key, "conv2_mma")) {
     if (g_conv2_mma < 0) { const char* e = getenv("MLS_CONV2_MMA"); g_conv2_mma = e ? atoi(e) : 1; }
@@ -81,9 +68,7 @@ int mls_cap_grid(int grid) {
 extern "C" int mls_set_option(const char* key, int value) {
   if (key && !strcmp(key, "conv2_mma")) { g_conv2_mma = value ? 1 : 0; return MLS_OK; }
   if (key && !strcmp(key, "fp32_tc")) { g_fp32_tc = value ? 1 : 0; return MLS_OK; }
-  if (key && !strcmp(key, "attn_hp")) { g_attn_hp = value < 0 ? 0 : (value > 2 ? 2 : value); return MLS_OK; }
   if (key && !strcmp(key, "attn_mma")) { g_attn_mma = value ? 1 : 0; return MLS_OK; }
-  if (key && !strcmp(key, "ctrl_first")) { g_ctrl_first = value ? 1 : 0; return MLS_OK; }
   if (key && !strcmp(key, "max_ctas")) { g_max_ctas = value > 0 ? value : 0; return MLS_OK; }
   mls_set_error("unknown option %s", key ? key : "(null)");
   return MLS_ERR_INVALID;

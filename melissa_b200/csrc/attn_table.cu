@@ -8,15 +8,18 @@
 //   pair_logit_kernel     E[ci][cj][h] = base-2 logit of head h for target key ci, source key cj
 //                           GATv2:       0.6 (a_j + b_i) + 0.4 sum_c att_c |x_l[j,c] + x_r[i,c]|
 //                           Transformer: <q_i, k_j> / sqrt(C)
-//   attn_table_mma_kernel per tile of G graphs (G*N <= 64 node rows), per head:
-//       producers (SIMT)   softmax weights 2^(e_ij - max_i) / (sum_j + 1e-16) from E, written as a bf16 matrix
-//                          W_h[target][source] (fp16, K-major, 128B swizzle); value rows x_l[key_j] / v[key_j] (fp16)
-//                          gathered from the table into a [source][channel] operand (MN-major, 128B swizzle)
-//       tcgen05.mma        out_h^T[channel][target] = V_h^T x W_h^T, fp32 accumulators in TMEM (double buffered)
-//                          (bulk copies of pre-swizzled rows); the conv bias rides along as two extra value rows
-//       epilogue warps     tcgen05.ld, ReLU, bf16 -> x1 rows and controlling-node snapshots
-//     The weight matrix is block diagonal over the graphs of a tile; the aggregation over (at most 33)
-//     neighbours is done densely because the tensor core does the 64-wide row in 4 instructions.
+//   values_fp16_kernel    value rows x_l[key] / v[key] of the present keys as fp16
+//
+// The aggregation runs on tcgen05 per tile of G graphs (G*N <= 62 node rows), with the softmax weights
+// 2^(e_ij - max_i) / (sum_j + 1e-16) from E as an fp16 weight matrix W_h[target][source] (block diagonal
+// over the graphs of a tile) and the value rows of the tile's nodes as the other operand; the aggregation
+// over (at most 33) neighbours is done densely because the tensor core does the 64-wide row in 4 instructions.
+//
+//   attn_table_prep_kernel + attn_table_rows_kernel   L-DGN / DGN-R: relu(conv1) of the needed rows into x1.
+//       A pre-pass builds one record per tile (needed targets, softmax weights); the MMA kernel's producers only
+//       move data, D[target][channel] = W x V per (tile, head), and the epilogue writes whole x1 rows.
+//   attn_table_pool_kernel   HL-DGN: one graph per tile, out^T[channel][target] = V^T x W^T per (tile, head pair),
+//       the epilogue pools relu(conv) * dm over the graph's nodes into z.
 //
 // Reference math: PyG GATv2Conv / TransformerConv as used by l_dgn.py:125,133 and dgn_r.py; softmax
 // exp(e - max) / (sum + 1e-16).  Same results as edge_bf16_kernel up to bf16 rounding of the weights.
@@ -228,379 +231,38 @@ __global__ void __launch_bounds__(256) pair_logit_kernel(const AttnTableArgs a) 
   }
 }
 
-// ------------------------------------------------------------------------------ aggregation on the tensor cores
+// ------------------------------------------------------------------------------ graph pooling on the tensor cores
 // The MMA is issued transposed, out_h^T[channel][target] = V_h^T x W_h^T, so that M = 128 channels fills the
-// tensor core's rows whatever the tile's node count, N = 64 targets halves the cycles per instruction, and a
-// warp's 32 TMEM lanes are 32 consecutive channels of one target: coalesced 64-byte stores.
+// tensor core's rows whatever the graph's node count and a warp's 32 TMEM lanes are 32 consecutive channels:
+// the pooling over the graph's nodes is a reduction over each lane's registers.
 //   A operand = value panels [source][channel]   (MN-major, 128B swizzle)
 //   B operand = weight matrix [target][source]   (K-major,  128B swizzle)
-//   D         = 64 TMEM columns per head, 4 heads, double buffered over tiles (512 columns)
-// 24 warps.  w & 3 = TMEM lane quarter:
-//   warp 0   MMA issuer            warp 1   TMEM allocation
-//   warps 4..11   epilogue: quarter w & 3, heads 2p and 2p+1 with p = (w >> 2) - 1
-//   the other 14 warps   two producer teams of 7 warps; team g builds the tiles g, g+2, ... of this CTA in stage g
-constexpr int kTThreads = 768;
-constexpr int kTeam = 224;
+// Work item = (tile, head pair).  A stage is 48 KiB (2 weight matrices + 4 value panels), so four stages and four
+// producer teams of 3 warps are in flight.
+//   warp 0  MMA issuer      warp 1  TMEM allocation      warps 2..9  epilogue (quarter = w & 3, head of the pair = (w - 2) >> 2)
+//   warps 10..21  four producer teams of 3 warps; team t builds items t, t+4, ... (item k: tile k >> 1, head pair k & 1)
 constexpr int kAHead = 64 * 128;               // weight matrix of one head: 64 targets x 64 sources bf16
 constexpr int kBPanel = 64 * 128;              // value panel: 64 sources x 64 channels bf16
-constexpr int kStageA = 4 * kAHead;            // 32 KiB
-constexpr int kStageB = 8 * kBPanel;           // 64 KiB
-constexpr int kStage = kStageA + kStageB;      // 96 KiB
 constexpr int kMetaSrc = 64 * kMaxNbr;         // CSR source lists of a tile: G * csr_stride(N) <= 2048 for G * N <= 64, N <= 62
 static_assert(64 / 33 * csr_stride(33) <= kMetaSrc && csr_stride(62) <= kMetaSrc, "tile CSR lists");
-constexpr int kMetaTab = kMetaSrc + 64 * 4 /*need list, counts*/ + 64 * 2 /*ids*/ + 128 * 2 /*CSR row pointers*/ + 64 * 4 /*dm*/;
-constexpr int kMeta = kMetaTab + 2 * 64 * 4 /*x_out row and snapshot slot of every TMEM column*/;
-constexpr int kTSmem = 2 * kStage + 2 * kMeta + 256 /*barriers*/ + 1024;
+constexpr int kMeta = kMetaSrc + 64 * 2 /*ids*/ + 128 * 2 /*CSR row pointers*/ + 64 * 4 /*dm*/;
+constexpr int kPoolThreads = 704;
+constexpr int kPoolTeam = 96;
+constexpr int kStageA2 = 2 * kAHead;           // 16 KiB
+constexpr int kStageB2 = 4 * kBPanel;          // 32 KiB
+constexpr int kStage2 = kStageA2 + kStageB2;   // 48 KiB
+constexpr int kPoolSmem = 4 * kStage2 + 4 * kMeta + 256 /*barriers*/ + 1024;
 
 __device__ __forceinline__ float f_ex2(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float f_rcp(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ void bar_team(int team) { asm volatile("bar.sync %0, 224;" ::"r"(team + 1) : "memory"); }
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-// mbarrier wait for warps that are far ahead of the pipeline: sleep between polls so that the issue slots
-// go to the warps doing the work
-__device__ __forceinline__ void mbar_wait_backoff(uint32_t bar, uint32_t parity, unsigned ns = 200) {
-  for (;;) {
-    uint32_t ok;
-    asm volatile(
-        "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    if (ok) return;
-    __nanosleep(ns);
-  }
-}
-__device__ __forceinline__ uint16_t relu_bf16(float x) {
-  uint16_t d;
-  asm("cvt.rn.relu.bf16.f32 %0, %1;" : "=h"(d) : "f"(x));
-  return d;
-}
 __device__ __forceinline__ uint32_t a_off(int i, int j) {      // byte offset of W[i][j] inside a head's K-major SW128 tile
   return (uint32_t)(i * 128 + ((((j >> 3) ^ i) & 7) << 4) + (j & 7) * 2);
 }
-
-__global__ void __launch_bounds__(kTThreads, 1) attn_table_mma_kernel(const AttnTableArgs a, const int G) {
-  if (*a.n_used > kAttnUcap) return;            // uniform: the gather kernel handles this pass
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  // 1024-byte alignment by offset (not by integer round trip): the compiler keeps the shared address space -> LDS / STS
-  unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  unsigned char* meta = smem + 2 * kStage;                                        // [2][kMeta]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(meta + 2 * kMeta);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 8);
-  const uint32_t bar0 = smem_u32(bars);
-  auto full_bar = [&](int s) { return bar0 + 8u * s; };
-  auto empty_bar = [&](int s) { return bar0 + 8u * (2 + s); };
-  auto tfull_bar = [&](int b) { return bar0 + 8u * (4 + b); };
-  auto tempty_bar = [&](int b) { return bar0 + 8u * (6 + b); };
-
-  const int N = a.N, HC = 4 * kC;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int quarter = warp & 3, grp = warp >> 2;
-  const int n_tiles = (a.n_graphs + G - 1) / G;
-  const int kb = G * N;                          // K index of the two bias rows (hi, lo); <= 62
-  const int ksteps = (kb + 2 + 15) >> 4;
-
-  for (int u = threadIdx.x; u < 2 * kStage / 16; u += kTThreads) reinterpret_cast<uint4*>(smem)[u] = make_uint4(0, 0, 0, 0);
-  __syncthreads();
-  // conv bias as two extra value rows (fp16 hi + lo), multiplied by two columns of ones in the weight matrix
-  for (int u = threadIdx.x; u < 2 * 512; u += kTThreads) {
-    const int s = u >> 9, ch = u & 511;
-    const float b = a.bias ? a.bias[ch] : 0.f;
-    const __half hi = __float2half_rn(b), lo = __float2half_rn(b - __half2float(hi));
-    unsigned char* panel = smem + s * kStage + kStageA + (ch >> 6) * kBPanel;
-    const int e = ch & 63;
-    *reinterpret_cast<__half*>(panel + kb * 128 + ((((e >> 3) ^ kb) & 7) << 4) + (e & 7) * 2) = hi;
-    *reinterpret_cast<__half*>(panel + (kb + 1) * 128 + ((((e >> 3) ^ (kb + 1)) & 7) << 4) + (e & 7) * 2) = lo;
-  }
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(full_bar(s), kTeam); mbar_init(empty_bar(s), 1);
-      mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), 8 * 32);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc(smem_u32(tmem_slot), 512);
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const bool is_epi = grp == 1 || grp == 2;
-  if (warp == 0) {
-    // ===================================================================== MMA issuer
-    if (lane == 0) {
-      // both operands fp16 (format fields of the kind::f16 descriptor: bits 7-9 A, 10-12 B; 0 = F16; mixing F16 with
-      // BF16 is an illegal instruction): the softmax weights live in [0, 1], where fp16 carries 11 significant bits
-      // against bf16's 8, and the bf16 value rows convert to fp16 exactly (values_fp16_kernel).  A (values) MN-major.
-      int it = 0;
-      for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-        const int s = it & 1;                                                  // shared-memory stage == TMEM buffer
-        const uint32_t sA = smem_u32(smem + s * kStage), sB = sA + kStageA;
-        mbar_wait(full_bar(s), (it >> 1) & 1);                                 // one thread: no backoff, every hand-off latency counts
-        mbar_wait(tempty_bar(s), ((it >> 1) & 1) ^ 1);
-        tc_fence_after();
-        // the weight matrix holds one row per NEEDED target, compacted (producers): N = their count rounded to 16
-        const int* cnt_s = reinterpret_cast<const int*>(meta + s * kMeta + kMetaSrc + 64);
-        const int nn = cnt_s[0] + cnt_s[1];
-        const int nmma = a.pool_mode >= 0 ? 64 : (nn <= 16 ? 16 : ((nn + 15) & ~15));   // pooling reads all 64 columns
-        const uint32_t idesc = (make_idesc(128, nmma) & ~((7u << 7) | (7u << 10))) | (1u << 15);
-        for (int h = 0; h < 4; ++h) {
-          const uint64_t dv = make_smem_desc_ex(sB + h * 2 * kBPanel, kBPanel >> 4, 1024 >> 4);
-          const uint64_t dw = make_smem_desc(sA + h * kAHead);
-          for (int k = 0; k < ksteps; ++k)
-            umma_bf16(tmem_base + (uint32_t)(s * 256 + h * 64), dv + (uint64_t)(k * 128), dw + (uint64_t)(k * 2), idesc, k ? 1u : 0u);
-        }
-        umma_commit(tfull_bar(s));                                              // the epilogue frees the stage (empty_bar)
-      }
-    }
-  } else if (is_epi) {
-    // ===================================================================== epilogue: lane = channel, registers = targets
-    const int pair = grp - 1;
-    int it = 0;
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-      const int b = it & 1;
-      const int g0 = tile * G;
-      mbar_wait_backoff(tfull_bar(b), (it >> 1) & 1, 20);
-      tc_fence_after();
-      // TMEM column t = the t-th needed target of the tile; the producers left the column count and, per column, the
-      // x_out row and the snapshot slot (-1: not a controlling node) in the stage's metadata
-      const int* cnt_b = reinterpret_cast<const int*>(meta + b * kMeta + kMetaSrc + 64);
-      const int* tab_x = reinterpret_cast<const int*>(meta + b * kMeta + kMetaTab);
-      const int* tab_s = tab_x + 64;
-      const int nn = a.pool_mode >= 0 ? 64 : cnt_b[0] + cnt_b[1];
-      float pool = 0.f;                          // relu(conv) * dm >= 0: 0 is the identity of max and add here
-#pragma unroll 1
-      for (int q = 0; q < 4; ++q) {
-        const int h = pair * 2 + (q >> 1), t0 = (q & 1) * 32;
-        const bool skip = t0 >= nn;                                            // warp uniform: no needed target in this half
-        uint32_t v[32];
-        if (!skip) tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(b * 256 + h * 64 + t0), v);
-        if (q == 3) { tc_fence_before(); mbar_arrive(tempty_bar(b)); }
-        if (skip) continue;
-        const int col = h * kC + quarter * 32 + lane;
-        if (a.pool_mode >= 0) {
-          // lane = channel, registers = the graph's nodes (rows of scripted nodes and rows beyond the graph are
-          // all-zero weight rows -> exactly 0): the pooling is a reduction over this lane's registers
-          if (a.pool_mode == MLS_POOL_MAX) {
-#pragma unroll
-            for (int t = 0; t < 32; ++t) pool = fmaxf(pool, __uint_as_float(v[t]));
-          } else {
-#pragma unroll
-            for (int t = 0; t < 32; ++t) pool += fmaxf(__uint_as_float(v[t]), 0.f);
-          }
-          if (q & 1) {
-            if (a.pool_mode == MLS_POOL_MEAN) pool = pool / (float)N;
-            a.z[(size_t)g0 * a.ldz + a.z_col + col] = __float2bfloat16_rn(pool);
-            pool = 0.f;
-          }
-          continue;
-        }
-        // stage relu(conv) as bf16 rows [column t][512 channels] in the (now free) value region of the stage
-        unsigned char* stg = smem + b * kStage + kStageA + (size_t)t0 * 1024 + col * 2;
-        const int nv = nn - t0;                                                // columns of this half that hold a target
-#pragma unroll
-        for (int t = 0; t < 32; ++t)
-          if (t < nv) *reinterpret_cast<uint16_t*>(stg + t * 1024) = relu_bf16(__uint_as_float(v[t]));   // warp uniform
-      }
-      if (a.pool_mode < 0) {
-        // ... and write them out as whole 1 KiB rows, 16 bytes per lane: x1 row of every needed target, snapshot row of
-        // the controlling ones
-        asm volatile("bar.sync 3, 256;" ::: "memory");
-        const unsigned char* stg = smem + b * kStage + kStageA;
-        const int et = threadIdx.x - 128;                                      // 0..255 within the epilogue warps
-        for (int u = et; u < nn * 64; u += 256) {
-          const int t = u >> 6, c = u & 63;
-          const uint4 val = *reinterpret_cast<const uint4*>(stg + t * 1024 + c * 16);
-          *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(a.x_out) + (size_t)tab_x[t] * (HC * 2) + c * 16) = val;
-          const int sl = tab_s[t];
-          if (sl >= 0) *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(a.z) + ((size_t)sl * a.ldz + a.z_col) * 2 + c * 16) = val;
-        }
-        asm volatile("bar.sync 3, 256;" ::: "memory");
-      }
-      if (threadIdx.x == 128) mbar_arrive(empty_bar(b));                        // stage free for the producers
-    }
-  } else if (warp != 1) {
-    // ===================================================================== producer teams
-    const int p = warp < 4 ? warp - 2 : warp - 10;                            // warps 2, 3, 12..23 -> 0..13
-    const int team = p & 1, pt = (p >> 1) * 32 + lane;                        // 0..223
-    const int self = a.transformer ? 0 : 1;
-    const int cpg = csr_stride(N) / 16;                                         // 16-byte chunks of a graph's CSR lists
-    unsigned char* sA = smem + team * kStage;
-    const uint32_t sB32 = smem_u32(sA + kStageA);
-    uint8_t* src_s = meta + team * kMeta;                                       // [gt][N*32]
-    uint8_t* need_s = src_s + kMetaSrc;                                         // [64] node rows of the tile whose output is read
-    int* cnt_s = reinterpret_cast<int*>(need_s + 64);                           // [2]
-    uint16_t* cid = reinterpret_cast<uint16_t*>(need_s + 256);                  // [64]
-    uint16_t* ptr_s = cid + 64;                                                 // [gt][N+1]
-    float* dm_s = reinterpret_cast<float*>(ptr_s + 128);                        // [64] decision-maker flag (pooling variant)
-    int* tabx_s = reinterpret_cast<int*>(meta + team * kMeta + kMetaTab);       // [64] x_out row of TMEM column t
-    int* tabs_s = tabx_s + 64;                                                  // [64] snapshot slot of TMEM column t or -1
-    // value gather: 4 lanes per node, lane part p copies the 16-byte chunks 4i + p (i = 0..15) of the node's 1 KiB
-    // fp16 row: a warp instruction reads 64 contiguous bytes of each of 8 rows; chunk c lands in panel c >> 3 at
-    // 16-byte slot (c & 7) ^ (row & 7) -- all offsets but two per-thread registers are immediates
-    const int gp = pt & 3;
-    const unsigned char* gsrc = reinterpret_cast<const unsigned char*>(a.Vh) + gp * 16;   // fp16 value rows of the present keys
-    // The epilogue stages its output rows in this stage's value region, clobbering the two bias rows (kb, kb + 1) and the
-    // unused rows behind them: every tile restores the former and clears the latter (they meet zero weights, but must
-    // stay finite as fp16).  This thread's channels: pt, pt + 224, pt + 448.
-    uint32_t bias_hl[3];
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-      const int ch = pt + r * kTeam;
-      const float bv = (a.bias && ch < 512) ? a.bias[ch] : 0.f;
-      const __half hi = __float2half_rn(bv), lo = __float2half_rn(bv - __half2float(hi));
-      bias_hl[r] = (uint32_t)__half_as_ushort(hi) | ((uint32_t)__half_as_ushort(lo) << 16);
-    }
-    int use = 0;
-    for (int tile = blockIdx.x + team * gridDim.x; tile < n_tiles; tile += 2 * gridDim.x, ++use) {
-      const int g0 = tile * G, gt = min(G, a.n_graphs - g0), rt = gt * N;
-      const size_t m0 = (size_t)g0 * N;
-      // ---- phase A: tile metadata (global loads first) and the cleared weight matrices
-      uint32_t pv = 0;
-      uint16_t cv = 0;
-      uint4 sv = make_uint4(0, 0, 0, 0);
-      float dmv = 1.f;
-      int xrv = 0, slv = -1;                                                   // xrv >= 0: somebody reads this target's output (its x_out row)
-      if (pt < rt) {
-        cv = __ldg(a.row_cid + m0 + pt);
-        if (a.pool_mode >= 0) dmv = __ldg(a.obs + (long long)(g0 + pt / N) * a.obs_stride + (pt % N) * 8 + 7);
-        if (a.xrow) xrv = __ldg(a.xrow + m0 + pt);
-        else if (a.pool_mode < 0) xrv = (int)m0 + pt;
-        if (a.slot) slv = __ldg(a.slot + m0 + pt);
-      }
-      if (pt < gt * (N + 1)) {                                                 // gt * (N + 1) <= 128
-        const int gl = pt / (N + 1), il = pt - gl * (N + 1);
-        const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
-        pv = __ldg(a.csr_ptr + cg * (N + 1) + il);
-      }
-      if (pt < gt * cpg) {                                                     // csr_stride(N) bytes (cpg chunks of 16 B) per graph
-        const int gl = pt / cpg, cl = pt - gl * cpg;
-        const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
-        sv = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * csr_stride(N)) + cl);
-      }
-      // the tile's needed targets, compacted (team warps 0 and 1 hold node rows 0..63)
-      const uint32_t nbal = __ballot_sync(0xffffffffu, pt < rt && xrv >= 0);
-      mbar_wait_backoff(empty_bar(team), (use & 1) ^ 1, 40);                   // the epilogue is done with this stage
-      for (int u = pt; u < kStageA / 16; u += kTeam) reinterpret_cast<uint4*>(sA)[u] = make_uint4(0, 0, 0, 0);
-      if (a.pool_mode < 0) {
-        unsigned char* sBv = sA + kStageA;
-#pragma unroll
-        for (int r = 0; r < 3; ++r) {
-          const int ch = pt + r * kTeam;
-          if (ch < 512) {
-            unsigned char* panel = sBv + (ch >> 6) * kBPanel;
-            const int e = ch & 63;
-            *reinterpret_cast<uint16_t*>(panel + kb * 128 + ((((e >> 3) ^ kb) & 7) << 4) + (e & 7) * 2) = (uint16_t)(bias_hl[r] & 0xffffu);
-            *reinterpret_cast<uint16_t*>(panel + (kb + 1) * 128 + ((((e >> 3) ^ (kb + 1)) & 7) << 4) + (e & 7) * 2) = (uint16_t)(bias_hl[r] >> 16);
-          }
-        }
-        const int tail = 62 - rt;                                              // rows rt .. 63 of the 8 panels except kb, kb + 1
-        for (int u = pt; u < tail * 64; u += kTeam) {
-          int row = rt + (u >> 6);
-          if (row >= kb) row += 2;
-          const int pc = u & 63;                                               // panel = pc >> 3, 16-byte chunk = pc & 7
-          *reinterpret_cast<uint4*>(sBv + (pc >> 3) * kBPanel + row * 128 + ((pc & 7) << 4)) = make_uint4(0, 0, 0, 0);
-        }
-      }
-      if (pt < rt) { cid[pt] = cv; dm_s[pt] = dmv; }
-      if (pt < gt * (N + 1)) ptr_s[pt] = (uint16_t)pv;
-      if (pt < gt * cpg) reinterpret_cast<uint4*>(src_s)[pt] = sv;
-      if (pt < 64 && lane == 0) cnt_s[pt >> 5] = __popc(nbal);
-      bar_team(team);
-      if (pt < rt && xrv >= 0) {
-        const int rank = (pt >= 32 ? cnt_s[0] : 0) + __popc(nbal & ((1u << lane) - 1u));
-        need_s[rank] = (uint8_t)pt;
-        tabx_s[rank] = xrv;                                                    // for the epilogue (read after the accumulators are ready)
-        tabs_s[rank] = slv;
-      }
-      // ---- phase B: value rows of the tile's nodes, asynchronously (swizzled by the node's row residue) ...
-      for (int j = pt >> 2; j < rt; j += kTeam / 4) {
-        const unsigned char* src = gsrc + (size_t)cid[j] * (HC * 2);
-        const uint32_t row = sB32 + j * 128;
-        const uint32_t d0 = row + ((gp ^ (j & 7)) << 4), d1 = row + (((gp + 4) ^ (j & 7)) << 4);
-#pragma unroll
-        for (int i = 0; i < 16; ++i) cp_async16(((i & 1) ? d1 : d0) + (i >> 1) * kBPanel, src + i * 64);
-      }
-      bar_team(team);                                                          // need_s complete
-      // ---- ... and the normalised softmax weights of (needed target i, head h) as fp16 rows of the head's weight matrix
-      const int n_tasks = (cnt_s[0] + cnt_s[1]) * 4;
-      for (int tt = pt; tt < n_tasks; tt += kTeam) {
-        const int wr = tt >> 2, i = need_s[wr], h = tt & 3;                    // weight row = rank among the needed targets
-        if (a.pool_mode >= 0 && dm_s[i] == 0.f) continue;                       // relu(conv) * 0: the row stays all zero
-        const int gl = i / N, il = i - gl * N, rbase = gl * N;
-        const uint16_t* ptr = ptr_s + gl * (N + 1);
-        const int r0 = ptr[il], d = (int)ptr[il + 1] - r0;
-        const uint8_t* src = src_s + gl * csr_stride(N) + r0;
-        const float* Erow = a.E + (size_t)cid[i] * kAttnUcap * 4 + h;
-        // entry 0 = the self loop (GATv2), then the CSR neighbours; batches of 8 independent table reads
-        const int cnt = d + self;
-        unsigned char* arow = sA + h * kAHead;
-        float ev[8];
-        int jv[8];
-        float mx = -INFINITY;
-        for (int k0 = 0; k0 < cnt; k0 += 8) {
-#pragma unroll
-          for (int q = 0; q < 8; ++q) {
-            const int k = k0 + q;
-            jv[q] = (k < cnt && k >= self) ? rbase + src[k - self] : i;
-            ev[q] = __ldg(Erow + (int)cid[jv[q]] * 4);
-          }
-#pragma unroll
-          for (int q = 0; q < 8; ++q) if (k0 + q < cnt) mx = fmaxf(mx, ev[q]);
-        }
-        float sum = 0.f;
-        if (cnt <= 8) {
-#pragma unroll
-          for (int q = 0; q < 8; ++q) { ev[q] = q < cnt ? f_ex2(ev[q] - mx) : 0.f; sum += ev[q]; }
-        } else {
-          for (int k = 0; k < cnt; ++k) {
-            const int j = k >= self ? rbase + src[k - self] : i;
-            sum += f_ex2(__ldg(Erow + (int)cid[j] * 4) - mx);
-          }
-        }
-        const float inv = f_rcp(sum + 1e-16f);
-        if (cnt <= 8) {
-#pragma unroll
-          for (int q = 0; q < 8; ++q)
-            if (q < cnt) *reinterpret_cast<__half*>(arow + a_off(wr, jv[q])) = __float2half_rn(ev[q] * inv);
-        } else {
-          for (int k = 0; k < cnt; ++k) {
-            const int j = k >= self ? rbase + src[k - self] : i;
-            *reinterpret_cast<__half*>(arow + a_off(wr, j)) = __float2half_rn(f_ex2(__ldg(Erow + (int)cid[j] * 4) - mx) * inv);
-          }
-        }
-        *reinterpret_cast<uint16_t*>(arow + a_off(wr, kb)) = 0x3C00;         // 1.0 (fp16): + bias (hi)
-        *reinterpret_cast<uint16_t*>(arow + a_off(wr, kb + 1)) = 0x3C00;     // 1.0 (fp16): + bias (lo)
-      }
-      cp_async_wait_all();
-      fence_proxy_async();
-      mbar_arrive(full_bar(team));
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, 512);
-}
-
-// ------------------------------------------------------------------------------ head-pair stages (default)
-// Same algorithm with the work item cut in two: (tile, head pair).  A stage is 48 KiB (2 weight matrices + 4 value panels),
-// so FOUR stages fit and four producer teams of 3 warps are in flight; the per-stage chain produce -> MMA -> epilogue ->
-// produce is half as long and twice as many of them overlap (the two-stage kernel above is bound by exactly that chain:
-// ncu shows producers waiting 62 % and the epilogue 46 % of their time).
-//   warp 0  MMA issuer      warp 1  TMEM allocation      warps 2..9  epilogue (quarter = w & 3, head of the pair = (w - 2) >> 2)
-//   warps 10..21  four producer teams of 3 warps; team t builds items t, t+4, ... (item k: tile k >> 1, head pair k & 1)
-constexpr int kT4Threads = 704;
-constexpr int kTeam4 = 96;
-constexpr int kStageA2 = 2 * kAHead;           // 16 KiB
-constexpr int kStageB2 = 4 * kBPanel;          // 32 KiB
-constexpr int kStage2 = kStageA2 + kStageB2;   // 48 KiB
-constexpr int kT4Smem = 4 * kStage2 + 4 * kMeta + 256 /*barriers*/ + 1024;
-
-__device__ __forceinline__ void bar_team4(int team) { asm volatile("bar.sync %0, 96;" ::"r"(team + 1) : "memory"); }
+__device__ __forceinline__ void bar_pool_team(int team) { asm volatile("bar.sync %0, 96;" ::"r"(team + 1) : "memory"); }
 // bounded waits: a protocol bug traps instead of hanging the GPU
 __device__ __forceinline__ void mbar_wait_guard(uint32_t bar, uint32_t parity, unsigned ns) {
   for (unsigned spins = 0;; ++spins) {
@@ -616,7 +278,9 @@ __device__ __forceinline__ void mbar_wait_guard(uint32_t bar, uint32_t parity, u
   }
 }
 
-__global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const AttnTableArgs a, const int G) {
+// HL-DGN: z[graph][z_col + H*C] = pool over the graph's nodes of relu(conv1) * dm, dm = obs column 7.  G = 1: the
+// epilogue pools all 64 columns of a tile into one graph.
+__global__ void __launch_bounds__(kPoolThreads, 1) attn_table_pool_kernel(const AttnTableArgs a, const int G) {
   if (*a.n_used > kAttnUcap) return;            // uniform: the gather kernel handles this pass
   extern __shared__ __align__(16) unsigned char smem_raw[];
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -637,10 +301,10 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
   const int kb = G * N;                          // K index of the two bias rows (hi, lo); <= 62
   const int ksteps = (kb + 2 + 15) >> 4;
 
-  for (int u = threadIdx.x; u < 4 * kStage2 / 16; u += kT4Threads) reinterpret_cast<uint4*>(smem)[u] = make_uint4(0, 0, 0, 0);
+  for (int u = threadIdx.x; u < 4 * kStage2 / 16; u += kPoolThreads) reinterpret_cast<uint4*>(smem)[u] = make_uint4(0, 0, 0, 0);
   if (threadIdx.x == 0) {
     for (int s = 0; s < 4; ++s) {
-      mbar_init(full_bar(s), kTeam4); mbar_init(empty_bar(s), 1);
+      mbar_init(full_bar(s), kPoolTeam); mbar_init(empty_bar(s), 1);
       mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), 8 * 32);
     }
     fence_barrier_init();
@@ -655,16 +319,13 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
   if (warp == 0) {
     // ===================================================================== MMA issuer
     if (lane == 0) {
+      const uint32_t idesc = (make_idesc(128, 64) & ~((7u << 7) | (7u << 10))) | (1u << 15);   // fp16 x fp16, A MN-major
       for (int k = 0; k < n_items; ++k) {
         const int s = k & 3;                                                   // shared-memory stage == TMEM buffer
         const uint32_t sA = smem_u32(smem + s * kStage2), sB = sA + kStageA2;
         mbar_wait_guard(full_bar(s), (k >> 2) & 1, 0);
         mbar_wait_guard(tempty_bar(s), ((k >> 2) & 1) ^ 1, 0);
         tc_fence_after();
-        const int* cnt_s = reinterpret_cast<const int*>(meta + s * kMeta + kMetaSrc + 64);
-        const int nn = cnt_s[0] + cnt_s[1];
-        const int nmma = a.pool_mode >= 0 ? 64 : (nn <= 16 ? 16 : ((nn + 15) & ~15));   // pooling reads all 64 columns
-        const uint32_t idesc = (make_idesc(128, nmma) & ~((7u << 7) | (7u << 10))) | (1u << 15);   // fp16 x fp16, A MN-major
         for (int hl = 0; hl < 2; ++hl) {
           const uint64_t dv = make_smem_desc_ex(sB + hl * 2 * kBPanel, kBPanel >> 4, 1024 >> 4);
           const uint64_t dw = make_smem_desc(sA + hl * kAHead);
@@ -675,61 +336,33 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
       }
     }
   } else if (warp >= 2 && warp < 10) {
-    // ===================================================================== epilogue: lane = channel, registers = targets
+    // ===================================================================== epilogue: lane = channel, registers = the graph's nodes
+    // (rows of scripted nodes and rows beyond the graph are all-zero weight rows -> exactly 0)
     const int quarter = warp & 3, hl = (warp - 2) >> 2;
-    const int et = threadIdx.x - 64;                                           // 0..255 within the epilogue warps
     for (int k = 0; k < n_items; ++k) {
       const int b = k & 3, hp = k & 1;
       const int tile = blockIdx.x + (k >> 1) * gridDim.x;
       const int g0 = tile * G;
       mbar_wait_guard(tfull_bar(b), (k >> 2) & 1, 20);
       tc_fence_after();
-      const int* cnt_b = reinterpret_cast<const int*>(meta + b * kMeta + kMetaSrc + 64);
-      const int* tab_x = reinterpret_cast<const int*>(meta + b * kMeta + kMetaTab);
-      const int* tab_s = tab_x + 64;
-      const int nn = a.pool_mode >= 0 ? 64 : cnt_b[0] + cnt_b[1];
       const int h = hp * 2 + hl;
-      unsigned char* stg0 = smem + b * kStage2 + kStageA2;                      // staging rows [column t][256 channels of the pair]
       float pool = 0.f;                          // relu(conv) * dm >= 0: 0 is the identity of max and add here
 #pragma unroll 1
       for (int q = 0; q < 2; ++q) {
-        const int t0 = q * 32;
-        const bool skip = t0 >= nn;                                            // warp uniform: no needed target in this half
         uint32_t v[32];
-        if (!skip) tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(b * 128 + hl * 64 + t0), v);
+        tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(b * 128 + hl * 64 + q * 32), v);
         if (q == 1) { tc_fence_before(); mbar_arrive(tempty_bar(b)); }
-        if (skip) continue;
-        if (a.pool_mode >= 0) {
-          if (a.pool_mode == MLS_POOL_MAX) {
+        if (a.pool_mode == MLS_POOL_MAX) {
 #pragma unroll
-            for (int t = 0; t < 32; ++t) pool = fmaxf(pool, __uint_as_float(v[t]));
-          } else {
+          for (int t = 0; t < 32; ++t) pool = fmaxf(pool, __uint_as_float(v[t]));
+        } else {
 #pragma unroll
-            for (int t = 0; t < 32; ++t) pool += fmaxf(__uint_as_float(v[t]), 0.f);
-          }
-          if (q == 1) {
-            if (a.pool_mode == MLS_POOL_MEAN) pool = pool / (float)N;
-            a.z[(size_t)g0 * a.ldz + a.z_col + h * kC + quarter * 32 + lane] = __float2bfloat16_rn(pool);
-          }
-          continue;
+          for (int t = 0; t < 32; ++t) pool += fmaxf(__uint_as_float(v[t]), 0.f);
         }
-        unsigned char* stg = stg0 + (size_t)t0 * 512 + (hl * kC + quarter * 32 + lane) * 2;
-        const int nv = nn - t0;
-#pragma unroll
-        for (int t = 0; t < 32; ++t)
-          if (t < nv) *reinterpret_cast<uint16_t*>(stg + t * 512) = relu_bf16(__uint_as_float(v[t]));   // warp uniform
-      }
-      if (a.pool_mode < 0) {
-        asm volatile("bar.sync 5, 256;" ::: "memory");
-        for (int u = et; u < nn * 32; u += 256) {                              // 512-byte half rows, 16 bytes per lane
-          const int t = u >> 5, c = u & 31;
-          const uint4 val = *reinterpret_cast<const uint4*>(stg0 + t * 512 + c * 16);
-          *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(a.x_out) + (size_t)tab_x[t] * (HC * 2) + hp * 512 + c * 16) = val;
-          const int sl = tab_s[t];
-          if (sl >= 0)
-            *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(a.z) + ((size_t)sl * a.ldz + a.z_col) * 2 + hp * 512 + c * 16) = val;
+        if (q == 1) {
+          if (a.pool_mode == MLS_POOL_MEAN) pool = pool / (float)N;
+          a.z[(size_t)g0 * a.ldz + a.z_col + h * kC + quarter * 32 + lane] = __float2bfloat16_rn(pool);
         }
-        asm volatile("bar.sync 5, 256;" ::: "memory");
       }
       if (threadIdx.x == 64) mbar_arrive(empty_bar(b));                         // stage free for its producer team
     }
@@ -743,19 +376,15 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
     unsigned char* sBv = sA + kStageA2;
     const uint32_t sB32 = smem_u32(sBv);
     uint8_t* src_s = meta + team * kMeta;                                       // [gt][N*32]
-    uint8_t* need_s = src_s + kMetaSrc;                                         // [64] node rows of the tile whose output is read
-    int* cnt_s = reinterpret_cast<int*>(need_s + 64);                           // [2]
-    uint16_t* cid = reinterpret_cast<uint16_t*>(need_s + 256);                  // [64]
+    uint16_t* cid = reinterpret_cast<uint16_t*>(src_s + kMetaSrc);              // [64] compact key id of every tile row
     uint16_t* ptr_s = cid + 64;                                                 // [gt][N+1]
-    float* dm_s = reinterpret_cast<float*>(ptr_s + 128);                        // [64]
-    int* tabx_s = reinterpret_cast<int*>(meta + team * kMeta + kMetaTab);       // [64] x_out row of TMEM column t
-    int* tabs_s = tabx_s + 64;                                                  // [64] snapshot slot of TMEM column t or -1
+    float* dm_s = reinterpret_cast<float*>(ptr_s + 128);                        // [64] decision-maker flag
     const int gp = pt & 3;
     const unsigned char* gsrc = reinterpret_cast<const unsigned char*>(a.Vh) + hp * 512 + gp * 16;   // this pair's half of a value row
     uint32_t bias_hl[3];                                                        // channels pt, pt + 96, pt + 192 of the pair
 #pragma unroll
     for (int r = 0; r < 3; ++r) {
-      const int chl = pt + r * kTeam4;
+      const int chl = pt + r * kPoolTeam;
       const float bv = (a.bias && chl < 256) ? a.bias[hp * 256 + chl] : 0.f;
       const __half hi = __float2half_rn(bv), lo = __float2half_rn(bv - __half2float(hi));
       bias_hl[r] = (uint32_t)__half_as_ushort(hi) | ((uint32_t)__half_as_ushort(lo) << 16);
@@ -770,13 +399,9 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
       uint16_t cv = 0;
       uint4 sv0 = make_uint4(0, 0, 0, 0), sv1 = make_uint4(0, 0, 0, 0);
       float dmv = 1.f;
-      int xrv = 0, slv = -1;
       if (pt < rt) {
         cv = __ldg(a.row_cid + m0 + pt);
-        if (a.pool_mode >= 0) dmv = __ldg(a.obs + (long long)(g0 + pt / N) * a.obs_stride + (pt % N) * 8 + 7);
-        if (a.xrow) xrv = __ldg(a.xrow + m0 + pt);
-        else if (a.pool_mode < 0) xrv = (int)m0 + pt;
-        if (a.slot) slv = __ldg(a.slot + m0 + pt);
+        dmv = __ldg(a.obs + (long long)(g0 + pt / N) * a.obs_stride + (pt % N) * 8 + 7);
       }
       if (pt < gt * (N + 1)) {                                                 // gt * (N + 1) <= 64
         const int gl = pt / (N + 1), il = pt - gl * (N + 1);
@@ -784,7 +409,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
         pv = __ldg(a.csr_ptr + cg * (N + 1) + il);
       }
       {                                                                        // csr_stride(N) bytes (cpg chunks of 16 B) per graph: <= 128 chunks
-        const int c0 = pt, c1 = pt + kTeam4;
+        const int c0 = pt, c1 = pt + kPoolTeam;
         if (c0 < gt * cpg) {
           const int gl = c0 / cpg, cl = c0 - gl * cpg;
           const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl) * a.gid_stride) : (size_t)(g0 + gl);
@@ -796,14 +421,13 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
           sv1 = __ldg(reinterpret_cast<const uint4*>(a.csr_src + cg * csr_stride(N)) + cl);
         }
       }
-      const uint32_t nbal = __ballot_sync(0xffffffffu, pt < rt && xrv >= 0);
       mbar_wait_guard(empty_bar(team), (use & 1) ^ 1, 40);                     // the epilogue is done with this stage
-      for (int u = pt; u < kStageA2 / 16; u += kTeam4) reinterpret_cast<uint4*>(sA)[u] = make_uint4(0, 0, 0, 0);
-      if (a.pool_mode < 0 || use == 0) {
-        // bias rows (kb, kb + 1) of the pair's 4 panels; the epilogue's staging clobbers them and the rows behind them
+      for (int u = pt; u < kStageA2 / 16; u += kPoolTeam) reinterpret_cast<uint4*>(sA)[u] = make_uint4(0, 0, 0, 0);
+      if (use == 0) {
+        // bias rows (kb, kb + 1) of the pair's 4 panels and the rows behind them, once: every tile has the same rows
 #pragma unroll
         for (int r = 0; r < 3; ++r) {
-          const int chl = pt + r * kTeam4;
+          const int chl = pt + r * kPoolTeam;
           if (chl < 256) {
             unsigned char* panel = sBv + (chl >> 6) * kBPanel;
             const int e = chl & 63;
@@ -812,7 +436,7 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
           }
         }
         const int tail = 62 - rt;                                              // rows rt .. 63 of the 4 panels except kb, kb + 1
-        for (int u = pt; u < tail * 32; u += kTeam4) {
+        for (int u = pt; u < tail * 32; u += kPoolTeam) {
           int row = rt + (u >> 5);
           if (row >= kb) row += 2;
           const int pc = u & 31;                                               // panel = pc >> 3, 16-byte chunk = pc & 7
@@ -822,29 +446,20 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
       if (pt < rt) { cid[pt] = cv; dm_s[pt] = dmv; }
       if (pt < gt * (N + 1)) ptr_s[pt] = (uint16_t)pv;
       if (pt < gt * cpg) reinterpret_cast<uint4*>(src_s)[pt] = sv0;
-      if (pt + kTeam4 < gt * cpg) reinterpret_cast<uint4*>(src_s)[pt + kTeam4] = sv1;
-      if (pt < 64 && lane == 0) cnt_s[pt >> 5] = __popc(nbal);
-      bar_team4(team);
-      if (pt < rt && xrv >= 0) {
-        const int rank = (pt >= 32 ? cnt_s[0] : 0) + __popc(nbal & ((1u << lane) - 1u));
-        need_s[rank] = (uint8_t)pt;
-        tabx_s[rank] = xrv;
-        tabs_s[rank] = slv;
-      }
+      if (pt + kPoolTeam < gt * cpg) reinterpret_cast<uint4*>(src_s)[pt + kPoolTeam] = sv1;
+      bar_pool_team(team);
       // ---- phase B: this pair's half (512 B) of the value rows of the tile's nodes, asynchronously ...
-      for (int j = pt >> 2; j < rt; j += kTeam4 / 4) {
+      for (int j = pt >> 2; j < rt; j += kPoolTeam / 4) {
         const unsigned char* src = gsrc + (size_t)cid[j] * (HC * 2);
         const uint32_t row = sB32 + j * 128;
         const uint32_t d0 = row + ((gp ^ (j & 7)) << 4), d1 = row + (((gp + 4) ^ (j & 7)) << 4);
 #pragma unroll
         for (int i = 0; i < 8; ++i) cp_async16(((i & 1) ? d1 : d0) + (i >> 1) * kBPanel, src + i * 64);
       }
-      bar_team4(team);                                                         // need_s complete
-      // ---- ... and the normalised softmax weights of (needed target i, head hl of the pair)
-      const int n_tasks = (cnt_s[0] + cnt_s[1]) * 2;
-      for (int tt = pt; tt < n_tasks; tt += kTeam4) {
-        const int wr = tt >> 1, i = need_s[wr], hl = tt & 1, h = hp * 2 + hl;
-        if (a.pool_mode >= 0 && dm_s[i] == 0.f) continue;                       // relu(conv) * 0: the row stays all zero
+      // ---- ... and the normalised softmax weights of (target i, head hl of the pair): weight row i
+      for (int tt = pt; tt < rt * 2; tt += kPoolTeam) {
+        const int i = tt >> 1, hl = tt & 1, h = hp * 2 + hl;
+        if (dm_s[i] == 0.f) continue;                                           // relu(conv) * 0: the row stays all zero
         const int gl = i / N, il = i - gl * N, rbase = gl * N;
         const uint16_t* ptr = ptr_s + gl * (N + 1);
         const int r0 = ptr[il], d = (int)ptr[il + 1] - r0;
@@ -879,15 +494,15 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
         if (cnt <= 8) {
 #pragma unroll
           for (int q = 0; q < 8; ++q)
-            if (q < cnt) *reinterpret_cast<__half*>(arow + a_off(wr, jv[q])) = __float2half_rn(ev[q] * inv);
+            if (q < cnt) *reinterpret_cast<__half*>(arow + a_off(i, jv[q])) = __float2half_rn(ev[q] * inv);
         } else {
           for (int kk = 0; kk < cnt; ++kk) {
             const int j = kk >= self ? rbase + src[kk - self] : i;
-            *reinterpret_cast<__half*>(arow + a_off(wr, j)) = __float2half_rn(f_ex2(__ldg(Erow + (int)cid[j] * 4) - mx) * inv);
+            *reinterpret_cast<__half*>(arow + a_off(i, j)) = __float2half_rn(f_ex2(__ldg(Erow + (int)cid[j] * 4) - mx) * inv);
           }
         }
-        *reinterpret_cast<uint16_t*>(arow + a_off(wr, kb)) = 0x3C00;         // 1.0 (fp16): + bias (hi)
-        *reinterpret_cast<uint16_t*>(arow + a_off(wr, kb + 1)) = 0x3C00;     // 1.0 (fp16): + bias (lo)
+        *reinterpret_cast<uint16_t*>(arow + a_off(i, kb)) = 0x3C00;          // 1.0 (fp16): + bias (hi)
+        *reinterpret_cast<uint16_t*>(arow + a_off(i, kb + 1)) = 0x3C00;      // 1.0 (fp16): + bias (lo)
       }
       cp_async_wait_all();
       fence_proxy_async();
@@ -899,22 +514,22 @@ __global__ void __launch_bounds__(kT4Threads, 1) attn_table_mma4_kernel(const At
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-// ------------------------------------------------------------------------------ per-tile records + row-major MMA kernel (option attn_hp = 2)
-// The staged kernels above spend their time in the per-item PROGRAM of a producer team (metadata loads, ballots, need
+// ------------------------------------------------------------------------------ per-tile records + row-major MMA kernel
+// A producer team that builds a whole item itself spends its time in a per-item PROGRAM (metadata loads, ballots, need
 // list, CSR walk, pair-logit reads, softmax: chains of dependent latencies run by 2-3 warps; profiles/
 // r02_conv1_experiments.txt).  Here that program runs ONCE per tile in a full-occupancy pre-pass (one warp per tile, all
 // four heads from one float4 table read) that leaves a record per tile:
-//     hdr {nn, ne, 0, 0} | x_out row of every needed target [64] | its snapshot slot [64] | compact key id of every tile row [64]
+//     hdr {nn, ne, 0, 0} | x_out row of every needed target [64] | compact key id of every tile row [64]
 //     | entries: (target rank << 8 | source row) [ne] | normalised softmax weights fp16 [4 heads][ne]
 // and the MMA kernel's producers only move data: three bulk copies (cp.async.bulk -> mbarrier) bring the record's fixed
 // part and the head's entry list into the stage, the value rows are gathered with cp.async by the record's key ids, and the
 // weights are scattered into the (cleared) K-major weight tile.
 //   D[target][channel] = W[target][source] (A, K-major) x V[source][channel] (B, MN-major), M = 128, N = 128 per (tile, head)
 // item; a TMEM lane is a target: an epilogue thread adds the conv bias, converts and writes 16-byte pieces of its target's
-// x1 row (and snapshot row) through a transposition tile (whole 128-byte row segments per store).  Six 24 KiB stages /
-// producer teams of 2 warps; four independent pairs of DRAIN warps (pair g owns head g and TMEM buffer g; TMEM -> tile) each
-// followed by its STORE warp (tile -> global); a stage returns to its team on tcgen05.commit.
-constexpr int kRecFixed = 16 + 64 * 4 + 64 * 4 + 64 * 2;   // 656 bytes: header, x_out rows, snapshot slots, key ids
+// x1 row through a transposition tile (whole 128-byte row segments per store).  Six 24 KiB stages / producer teams of 2
+// warps; four independent pairs of DRAIN warps (pair g owns head g and TMEM buffer g; TMEM -> tile) each followed by its
+// STORE warp (tile -> global); a stage returns to its team on tcgen05.commit.
+constexpr int kRecFixed = 16 + 64 * 4 + 64 * 2;            // 400 bytes: header, x_out rows, key ids (a multiple of 16: bulk copies)
 constexpr int kRecChunk = 512;                             // entries per in-kernel chunk
 __host__ __device__ inline int rec_entry_cap(int rows) { return (rows * (kMaxList + 1) + 7) & ~7; }   // sources + self loop
 __host__ __device__ inline int rec_stride(int rows) { return kRecFixed + 10 * rec_entry_cap(rows); }
@@ -941,17 +556,16 @@ __global__ void __launch_bounds__(256, 4) attn_table_prep_kernel(const AttnTable
   uint8_t* need_s = need_sm[warp];
   uint8_t* cnt_s = cnt_sm[warp];
   int* cg_s = cg_sm[warp];
-  int xr[2], sl[2], cnt[2], p0[2], gl[2];
+  int xr[2], cnt[2], p0[2], gl[2];
   uint16_t cv[2];
   const uint8_t* srcp[2];
 #pragma unroll
   for (int q = 0; q < 2; ++q) {
     const int r = lane + 32 * q;
-    xr[q] = -1; sl[q] = -1; cnt[q] = 0; cv[q] = 0; p0[q] = 0; gl[q] = 0; srcp[q] = nullptr;
+    xr[q] = -1; cnt[q] = 0; cv[q] = 0; p0[q] = 0; gl[q] = 0; srcp[q] = nullptr;
     if (r < rt) {
       cv[q] = __ldg(a.row_cid + m0 + r);
       xr[q] = a.xrow ? __ldg(a.xrow + m0 + r) : (int)m0 + r;
-      if (a.slot) sl[q] = __ldg(a.slot + m0 + r);
       gl[q] = r / N;
       const int il = r - gl[q] * N;
       const size_t cg = a.graph_id ? (size_t)__ldg(a.graph_id + (size_t)(g0 + gl[q]) * a.gid_stride) : (size_t)(g0 + gl[q]);
@@ -985,15 +599,14 @@ __global__ void __launch_bounds__(256, 4) attn_table_prep_kernel(const AttnTable
     a.tile_idx[tile] = make_int2(ne_pad, nn);
   }
   int* tab_x = reinterpret_cast<int*>(rec + 16);
-  int* tab_s = tab_x + 64;
-  uint16_t* cid_g = reinterpret_cast<uint16_t*>(rec + 16 + 512);
+  uint16_t* cid_g = reinterpret_cast<uint16_t*>(rec + 16 + 256);
   uint16_t* jr = reinterpret_cast<uint16_t*>(rec + kRecFixed);
   __half* wts = reinterpret_cast<__half*>(rec + kRecFixed + 2 * cap);          // [4][cap]
 #pragma unroll
   for (int q = 0; q < 2; ++q) {
     const int r = lane + 32 * q;
     cid_g[r] = cv[q];
-    if (xr[q] >= 0) { tab_x[rank[q]] = xr[q]; tab_s[rank[q]] = sl[q]; need_s[rank[q]] = (uint8_t)r; off_s[rank[q]] = (uint16_t)off[q]; }
+    if (xr[q] >= 0) { tab_x[rank[q]] = xr[q]; need_s[rank[q]] = (uint8_t)r; off_s[rank[q]] = (uint16_t)off[q]; }
   }
   __syncwarp();
   // padding entries (read by the 16-byte granular copies, never scattered): keep them defined
@@ -1069,7 +682,7 @@ constexpr int kT6Threads = 960;
 constexpr int kTeam6 = 64;
 constexpr int kNumSt6 = 6;
 constexpr int kStage1 = kAHead + 2 * kBPanel;  // 24 KiB
-constexpr int kMetaFix = 768;                  // record fixed part (656) rounded up
+constexpr int kMetaFix = (kRecFixed + 127) & ~127;   // record fixed part rounded up
 constexpr int kMeta8 = kMetaFix + 4 * kRecChunk;   // + one chunk of entries (2 B each) and of weights (2 B each)
 constexpr int kEpiRow = 144;                   // epilogue staging row: 64 bf16 + 16 B pad (conflict-free 16-byte accesses)
 constexpr int kEpiTile = 32 * kEpiRow;         // one warp's transposition tile
@@ -1194,7 +807,7 @@ __global__ void __launch_bounds__(kT6Threads, 1) attn_table_rows_kernel(const At
     // Drain warps (this branch) move the accumulator into the pair's transposition tile; a STORE warp per drain warp
     // (below) writes the rows out, so that the address arithmetic / global stores of item k overlap the tcgen05.ld /
     // conversion of item k + 4 (the epilogue was the kernel's limiter: its warps were 75 % busy).  A tile row = 128 bytes of
-    // channels + 16 bytes {x1 row, snapshot slot, rows in the tile (-1: stop), byte offset inside a row}.
+    // channels + 16 bytes {x1 row, rows in the tile (-1: stop), byte offset inside a row, 0}.
     const int dw = b * 2 + qq;
     unsigned char* tile_s = epi_tiles + dw * kEpiTile;
     uint32_t msg = 0;
@@ -1204,13 +817,12 @@ __global__ void __launch_bounds__(kT6Threads, 1) attn_table_rows_kernel(const At
       tc_fence_after();
       const int4 hdr = *reinterpret_cast<const int4*>(meta + s * kMeta8);      // {nn, ne, 0, 0}
       const int* tab_x = reinterpret_cast<const int*>(meta + s * kMeta8 + 16);
-      const int* tab_s = tab_x + 64;
       const int nn = hdr.x;
       const bool rep = nn <= 32;
       const int t0 = rep ? 0 : qq * 32;                                        // first target of this warp's TMEM lanes
       const int nv = max(0, min(32, nn - t0));                                 // targets among them
-      int xr = 0, sl = -1;
-      if (lane < nv) { xr = tab_x[t0 + lane]; sl = tab_s[t0 + lane]; }
+      int xr = 0;
+      if (lane < nv) xr = tab_x[t0 + lane];
       __syncwarp();
       if (lane == 0) mbar_arrive(empty_bar(s));                                // this warp is done with the stage's record
       s += 4; if (s >= kNumSt6) s -= kNumSt6;
@@ -1234,33 +846,30 @@ __global__ void __launch_bounds__(kT6Threads, 1) attn_table_rows_kernel(const At
             }
           }
         }
-        *reinterpret_cast<int4*>(tile_s + lane * kEpiRow + 128) = make_int4(xr, sl, nv, (b * kC + c0 + hf * 64) * 2);
+        *reinterpret_cast<int4*>(tile_s + lane * kEpiRow + 128) = make_int4(xr, nv, (b * kC + c0 + hf * 64) * 2, 0);
         if (hf == nhalf - 1) { tc_fence_before(); mbar_arrive(tempty_bar(b)); }   // accumulator drained
         mbar_arrive(tile_full_bar(dw));
         ++msg;
       }
     }
     mbar_wait_guard(tile_free_bar(dw), (msg & 1u) ^ 1u, 20);
-    *reinterpret_cast<int4*>(tile_s + lane * kEpiRow + 128) = make_int4(0, -1, -1, 0);   // stop
+    *reinterpret_cast<int4*>(tile_s + lane * kEpiRow + 128) = make_int4(0, -1, 0, 0);    // stop
     mbar_arrive(tile_full_bar(dw));
   } else if (is_store) {
-    // ===================================================================== store warps: tile -> x1 rows / snapshot rows
+    // ===================================================================== store warps: tile -> x1 rows
     const int sw = warp - 22;
     const unsigned char* tile_s = epi_tiles + sw * kEpiTile;
     const int srow = lane >> 3, schunk = lane & 7;                             // 4 rows x 8 chunks per instruction
     for (uint32_t msg = 0;; ++msg) {
       mbar_wait_guard(tile_full_bar(sw), msg & 1u, 20);
-      const int nv = reinterpret_cast<const int*>(tile_s + 128)[2];
+      const int nv = reinterpret_cast<const int*>(tile_s + 128)[1];
       if (nv < 0) break;
       for (int r0 = 0; r0 < nv; r0 += 4) {
         const int r = r0 + srow;
         if (r < nv) {
           const int4 pd = *reinterpret_cast<const int4*>(tile_s + r * kEpiRow + 128);
           const uint4 val = *reinterpret_cast<const uint4*>(tile_s + r * kEpiRow + schunk * 16);
-          const size_t colb = (size_t)pd.w + schunk * 16;
-          *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(a.x_out) + (size_t)pd.x * (HC * 2) + colb) = val;
-          if (pd.y >= 0)
-            *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(a.z) + ((size_t)pd.y * a.ldz + a.z_col) * 2 + colb) = val;
+          *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(a.x_out) + (size_t)pd.x * (HC * 2) + pd.z + schunk * 16) = val;
         }
       }
       __syncwarp();
@@ -1273,7 +882,7 @@ __global__ void __launch_bounds__(kT6Threads, 1) attn_table_rows_kernel(const At
     unsigned char* sA = smem + team * kStage1;
     const uint32_t sB32 = smem_u32(sA + kAHead);
     unsigned char* mt = meta + team * kMeta8;
-    const uint16_t* cid = reinterpret_cast<const uint16_t*>(mt + 16 + 512);     // [64] compact key id of every tile row
+    const uint16_t* cid = reinterpret_cast<const uint16_t*>(mt + 16 + 256);     // [64] compact key id of every tile row
     const uint16_t* jr_s = reinterpret_cast<const uint16_t*>(mt + kMetaFix);    // [kRecChunk]
     const __half* w_s = reinterpret_cast<const __half*>(mt + kMetaFix + 2 * kRecChunk);
     const uint32_t mt32 = smem_u32(mt), mbar = meta_bar(team);
@@ -1373,14 +982,12 @@ int attn_table_conv_launch(const AttnTableArgs& a, int sm_count, cudaStream_t st
     mls_set_error("table-mode attention: unsupported shape (N=%d, H=%d)", a.N, a.H);
     return MLS_ERR_UNSUPPORTED;
   }
-  if (!a.z || (a.pool_mode < 0 && (!a.x_out || (long long)a.n_graphs * a.N * a.ldz >= (1ll << 31))) || (a.pool_mode >= 0 && !a.obs)) {
-    mls_set_error("table-mode attention: snapshot matrix too large for 32-bit offsets or missing outputs");
-    return MLS_ERR_UNSUPPORTED;
-  }
+  const bool pool = a.pool_mode >= 0;
+  MLS_CHECK_ARG(pool ? a.z && a.obs : a.x_out && a.rec && a.tile_idx,
+                "table-mode attention: pooling needs z and obs, the row output needs x_out, rec and tile_idx");
   static bool configured = false;
   if (!configured) {
-    MLS_CUDA(cudaFuncSetAttribute(attn_table_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTSmem));
-    MLS_CUDA(cudaFuncSetAttribute(attn_table_mma4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kT4Smem));
+    MLS_CUDA(cudaFuncSetAttribute(attn_table_pool_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPoolSmem));
     MLS_CUDA(cudaFuncSetAttribute(attn_table_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kT6Smem));
     configured = true;
   }
@@ -1389,19 +996,16 @@ int attn_table_conv_launch(const AttnTableArgs& a, int sm_count, cudaStream_t st
   row_cid_kernel<<<(rows + 255) / 256, 256, 0, st>>>(a.key, a.cid_of_key, rows, a.row_cid);
   values_fp16_kernel<<<kAttnUcap * 64 / 256, 256, 0, st>>>(a);
   pair_logit_kernel<<<sm_count * 2, 256, 0, st>>>(a);
-  const int G = a.pool_mode >= 0 ? 1 : kAttnMaxRows / a.N;     // pooling: one graph per tile
+  const int G = pool ? 1 : kAttnMaxRows / a.N;                  // pooling: one graph per tile
   const int n_tiles = (a.n_graphs + G - 1) / G;
-  const int grid = mls_cap_grid(n_tiles < sm_count ? n_tiles : sm_count);   // all three kernels below take any grid
+  const int grid = mls_cap_grid(n_tiles < sm_count ? n_tiles : sm_count);   // the persistent kernels take any grid
   if (grid > 0) {
-    const int mode = mls_get_option("attn_hp");
-    if (mode >= 2 && a.pool_mode < 0 && a.rec && a.tile_idx) {                 // per-tile records + row-major MMA (default)
+    if (pool) {
+      attn_table_pool_kernel<<<grid, kPoolThreads, kPoolSmem, st>>>(a, G);
+    } else {
       attn_table_prep_kernel<<<(n_tiles + 7) / 8, 256, 0, st>>>(a, G);
       attn_table_rows_kernel<<<grid, kT6Threads, kT6Smem, st>>>(a, G);
       mls_count_launch();
-    } else if (mode) {
-      attn_table_mma4_kernel<<<grid, kT4Threads, kT4Smem, st>>>(a, G);        // head-pair stages, channel-major (pooling)
-    } else {
-      attn_table_mma_kernel<<<grid, kTThreads, kTSmem, st>>>(a, G);
     }
   }
   mls_count_launch(5);

@@ -24,19 +24,18 @@ struct AttnTableArgs {
   int N, H, n_graphs;
   const uint16_t* csr_ptr;   // [graphs][N+1]
   const uint8_t* csr_src;    // [graphs][csr_stride(N)]
-  const int* slot;           // [rows] controlling-list slot or -1
   // optional "needed" row map (ctrl_need_list_kernel): x_out row of every node row, -1 = nobody reads this node's
-  // conv output (its softmax weights are not even built); needed rows of a graph are consecutive, in node order
+  // conv output (its softmax weights are not even built)
   const int* xrow;
   // CSR lists of graph g live at index graph_id[g * gid_stride] (topology cache of a static graph pool), else at g
   const int* graph_id;
   int gid_stride;
   __nv_bfloat16* x_out;      // [rows][H*C] relu(conv)  (or [needed rows][H*C] with xrow)
-  __nv_bfloat16* z;          // snapshot rows
-  int ldz, z_col;
-  // HL-DGN: pool_mode >= 0 (enum MlsPool): instead of x_out / snapshots, z[graph][z_col + H*C] = pool over the graph's
-  // nodes of relu(conv) * dm, dm = obs column 7 (one graph per tile)
+  // HL-DGN: pool_mode >= 0 (enum MlsPool): instead of x_out, z[graph][z_col + H*C] = pool over the graph's nodes of
+  // relu(conv) * dm, dm = obs column 7 (one graph per tile)
   int pool_mode;
+  __nv_bfloat16* z;
+  int ldz, z_col;
   const float* obs;
   long long obs_stride;
   // scratch (workspace)
@@ -48,8 +47,8 @@ struct AttnTableArgs {
   int* n_used;               // [1] number of distinct keys; > kAttnUcap: the caller's gather kernel runs instead
   void* Vh;                  // [kAttnUcap][H*C] fp16 value rows of the present keys (by compact id)
   float* E;                  // [kAttnUcap][kAttnUcap][4] base-2 logits of (target key, source key) for the 4 heads
-  // optional (x_out / snapshot variant): per-tile records written by the pre-pass, attn_table_record_bytes() bytes, and
-  // {padded entry count, needed targets} of every tile; NULL: the staged kernel builds everything per item
+  // x_out (pool_mode < 0): per-tile records written by the pre-pass, attn_table_record_bytes() bytes, and
+  // {padded entry count, needed targets} of every tile
   unsigned char* rec;
   int2* tile_idx;            // [tiles]
 };

@@ -155,7 +155,7 @@ __global__ void __launch_bounds__(kThreads, TR ? 4 : kCtasPerSm) conv2_attn_kern
     }
   };
   // row of source k (compact index) in Ps / as
-  auto src_row = [&](int first, int cnt, int nf, int k) { return a.ctrl_first ? (k < cnt ? first + k : nf + k - cnt) : nf + k; };
+  auto src_row = [&](int first, int cnt, int nf, int k) { return k < cnt ? first + k : nf + k - cnt; };
   auto issue_A = [&](int first, int cnt, int nf, int nc) {
     load_targets(first, 0, cnt < kTB ? cnt : kTB);
     if (!TR) {
@@ -164,6 +164,7 @@ __global__ void __launch_bounds__(kThreads, TR ? 4 : kCtasPerSm) conv2_attn_kern
     }
   };
   auto issue_B = [&](int first, int cnt, int nf, int nc, int ef, int ne) {
+#pragma unroll 2   // unrolled further, the GATv2 kernel spills more under its 72-register cap and runs slower
     for (int t = tid; t < nc * 16; t += kThreads) {
       const int k = t >> 4, c = t & 15;
       const __half* row = a.Ps + (size_t)src_row(first, cnt, nf, k) * a.lds + h * kC + c * 8;

@@ -26,7 +26,9 @@ struct Conv2Args {
   int transformer;
   int N, H, n_graphs;
   // row sets and edge lists (ctrl_need_list_kernel): the slots / needed rows / edge entries of graph g are consecutive
-  //   gmeta[g] = {first slot, controlling nodes, first needed row, needed rows, first edge entry, edge entries, 0, 0}
+  //   gmeta[g] = {first slot, controlling nodes, first other needed row, needed rows, first edge entry, edge entries, 0, 0}
+  //   needed rows are ordered [controlling nodes by slot][the others]: source k of graph g (compact index, controlling
+  //   nodes first) lives in row first slot + k for k < controlling nodes, else gmeta[2] + k - controlling nodes
   //   eabs[slot] = position of the slot's first edge entry (its entries run to the next slot's, the last to the block end)
   //   eent[e]    = compact source index (rank in the graph's needed list) | target index within the graph << 8;
   //                the GATv2 self loop is an ordinary entry; blocks start 16-byte aligned
@@ -36,9 +38,6 @@ struct Conv2Args {
   // output: relu(conv2)[slot] as bf16 at z[slot][z_col + h*C ...]
   __nv_bfloat16* z;
   int ldz, z_col;
-  // needed rows ordered [controlling nodes by slot][the others]: source k of graph g (compact index, controlling nodes
-  // first) lives in row first_slot + k for k < controlling nodes, else gmeta[2] + k - controlling nodes
-  int ctrl_first;
 };
 
 inline bool conv2_attn_supported(int N, int H) { return N >= 1 && N <= kConv2MaxNodes && H >= 1; }

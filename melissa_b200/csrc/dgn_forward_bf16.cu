@@ -517,8 +517,11 @@ __global__ void __launch_bounds__(EdgeCfg<TRANSFORMER>::kThreads, EdgeCfg<TRANSF
 //     consecutive, in node order (gfirst / gcnt; one atomic reservation per graph)
 //   needed rows (two-conv models, adj != NULL): the network reads conv2 only at the controlling nodes
 //     (l_dgn.py:133-139), so conv2's sources -- and therefore the only rows of relu(conv1) anybody reads -- are the
-//     controlling nodes themselves (self loop, snapshot) and their radius-graph sources.  nidx[r] = node row of
-//     needed row r, xrow[node row] = r or -1, consecutive per graph in node order (nfirst / ncnt).
+//     controlling nodes themselves (self loop, snapshot) and their radius-graph sources.  The needed rows are ordered
+//     [all controlling nodes, in slot order][the other needed nodes]: a controlling node's needed row IS its slot, so
+//     relu(conv1) of a controlling node is written once and x1[0 : count) doubles as the snapshot matrix.  Here the other
+//     needed nodes get xrow = -2 - j (j from a counter of their own, ncount); need_rows_fixup_kernel turns that into
+//     count + j once the total number of controlling nodes is known, and builds nidx[r] = node row of needed row r.
 // mode 1 (agent-observation rows, one controlling node per graph): slot of graph g is g.
 template <int W>
 __global__ void ctrl_need_list_kernel(const uint8_t* __restrict__ ctrl_mask, const float* __restrict__ obs, int64_t obs_stride,
@@ -529,7 +532,7 @@ __global__ void ctrl_need_list_kernel(const uint8_t* __restrict__ ctrl_mask, con
                                       int* __restrict__ ncount, int* __restrict__ nfirst, int* __restrict__ ncnt,
                                       const uint16_t* __restrict__ csr_ptr, const uint8_t* __restrict__ csr_src, int self_loops,
                                       int* __restrict__ ecount, int* __restrict__ eabs, uint16_t* __restrict__ eent,
-                                      int* __restrict__ gmeta, int ctrl_first) {
+                                      int* __restrict__ gmeta) {
   const int lane = threadIdx.x & 31;
   const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (g >= n_graphs) return;
@@ -590,43 +593,24 @@ __global__ void ctrl_need_list_kernel(const uint8_t* __restrict__ ctrl_mask, con
     nw[w] = __reduce_or_sync(0xffffffffu, nw[w]) | cw[w];
     nn += __popc(nw[w]);
   }
-  // ctrl_first: the needed rows are ordered [all controlling nodes, in slot order][the other needed nodes]: a controlling
-  // node's compact row IS its slot, so relu(conv1) of the controlling rows is written once and x1[0 : count) doubles as the
-  // snapshot matrix.  The other needed nodes get -2 - j here (j from a counter of their own); need_rows_fixup_kernel turns
-  // that into count + j once the total number of controlling nodes is known, and builds nidx.
-  const int nalloc = ctrl_first ? nn - total : nn;
+  const int nalloc = nn - total;
   int ns = 0;
   if (lane == 0 && nalloc) ns = atomicAdd(ncount, nalloc);
   ns = __shfl_sync(0xffffffffu, ns, 0);
   if (lane == 0) { nfirst[g] = ns; ncnt[g] = nn; }
-  if (ctrl_first) {
-    int run_c = slot0, run_o = ns;
+  int run_c = slot0, run_o = ns;
 #pragma unroll
-    for (int w = 0; w < W; ++w) {
-      const int i = w * 32 + lane;
-      const uint32_t ow = nw[w] & ~cw[w], below = (1u << lane) - 1;
-      if (i < N) {
-        int r = -1;
-        if ((cw[w] >> lane) & 1u) r = run_c + __popc(cw[w] & below);
-        else if ((ow >> lane) & 1u) r = -2 - (run_o + __popc(ow & below));
-        xrow[(size_t)g * N + i] = r;
-      }
-      run_c += __popc(cw[w]);
-      run_o += __popc(ow);
+  for (int w = 0; w < W; ++w) {
+    const int i = w * 32 + lane;
+    const uint32_t ow = nw[w] & ~cw[w], below = (1u << lane) - 1;
+    if (i < N) {
+      int r = -1;
+      if ((cw[w] >> lane) & 1u) r = run_c + __popc(cw[w] & below);
+      else if ((ow >> lane) & 1u) r = -2 - (run_o + __popc(ow & below));
+      xrow[(size_t)g * N + i] = r;
     }
-  } else {
-    int run = ns;
-#pragma unroll
-    for (int w = 0; w < W; ++w) {
-      const int i = w * 32 + lane;
-      if (i < N) {
-        const bool c = (nw[w] >> lane) & 1u;
-        const int r = run + __popc(nw[w] & ((1u << lane) - 1));
-        if (c) nidx[r] = g * N + i;
-        xrow[(size_t)g * N + i] = c ? r : -1;
-      }
-      run += __popc(nw[w]);
-    }
+    run_c += __popc(cw[w]);
+    run_o += __popc(ow);
   }
   if (!eent) return;
   // conv2 edge list of the graph, shared by the heads: per controlling node (slot order) one entry per incoming edge
@@ -668,16 +652,10 @@ __global__ void ctrl_need_list_kernel(const uint8_t* __restrict__ ctrl_mask, con
       const int tk = tk_base + __popc(cw[w] & ((1u << lane) - 1));
       int pos = e0 + offv[w];
       eabs[slot0 + tk] = pos;
-      auto rank_of = [&](int j) {
+      auto rank_of = [&](int j) {                        // controlling nodes first (rank among them), then the other needed nodes
         const int jw = j >> 5;
         const uint32_t below = (1u << (j & 31)) - 1u;
         int r = 0;
-        if (!ctrl_first) {
-#pragma unroll
-          for (int v = 0; v < W; ++v) r += __popc(nw[v] & (v < jw ? 0xffffffffu : (v == jw ? below : 0u)));
-          return r;
-        }
-        // controlling nodes first (rank among them), then the other needed nodes
         const bool jc = (cw[jw] >> (j & 31)) & 1u;
 #pragma unroll
         for (int v = 0; v < W; ++v) {
@@ -693,7 +671,7 @@ __global__ void ctrl_need_list_kernel(const uint8_t* __restrict__ ctrl_mask, con
   }
 }
 
-// ctrl_first: final compact rows (see ctrl_need_list_kernel).  One thread per node row: -2 - j -> count + j, nidx[row] = node
+// Final needed rows (see ctrl_need_list_kernel).  One thread per node row: -2 - j -> count + j, nidx[row] = node
 // row; one thread per graph: first non-controlling needed row of the graph (gmeta[2]) made absolute; thread 0: ncount (the
 // other needed nodes so far) -> total number of needed rows.
 __global__ void need_rows_fixup_kernel(int* __restrict__ xrow, int* __restrict__ nidx, int* __restrict__ gmeta, const int* __restrict__ count,
@@ -755,7 +733,9 @@ __global__ void head_out_bf16_kernel(const bf16* __restrict__ hid, int hh, const
 }
 
 // Network without dueling heads: q = out_linear(latent) (l_dgn.py:88-90,149) on the bf16 latent rows.  One warp per row.
-__global__ void head_linear_b_kernel(const bf16* __restrict__ z, int latent, const int* __restrict__ idx, const int* __restrict__ count,
+// With x1 (L-DGN / DGN-R) the snapshot columns [hid, hid + HC) of latent row t are x1 row t, the rest come from z.
+__global__ void head_linear_b_kernel(const bf16* __restrict__ z, int latent, const bf16* __restrict__ x1, int hid, int HC,
+                                     const int* __restrict__ idx, const int* __restrict__ count,
                                      int max_rows, const float* __restrict__ w, const float* __restrict__ b, int64_t row0, int per_graph_N,
                                      float* __restrict__ q_out, int8_t* __restrict__ act_out, int out_mode, ActArgsB aa) {
   const int lane = threadIdx.x & 31;
@@ -763,9 +743,11 @@ __global__ void head_linear_b_kernel(const bf16* __restrict__ z, int latent, con
   const int n = count ? min(*count, max_rows) : max_rows;
   if (t >= n) return;
   const bf16* zr = z + (size_t)t * latent;
+  const bf16* xr = x1 ? x1 + (size_t)t * HC : nullptr;
   float s0 = 0.f, s1 = 0.f;
   for (int c = lane; c < latent; c += 32) {
-    const float v = __bfloat162float(zr[c]);
+    const bool snap = x1 && c >= hid && c < hid + HC;
+    const float v = __bfloat162float(snap ? xr[c - hid] : zr[c]);
     s0 = fmaf(v, w[c], s0);
     s1 = fmaf(v, w[latent + c], s1);
   }
@@ -827,7 +809,7 @@ struct WsB {
   float* qg;
   int *idx, *slot, *count, *gfirst, *gcnt;
   int *nidx, *xrow, *ncount, *nfirst, *ncnt;   // needed rows (conv2 sources)
-  int* ntotal;                                 // ctrl_first: controlling + other needed rows (ncount then counts the others only)
+  int* ntotal;                                 // controlling + other needed rows (ncount counts the others only)
   int *ecount, *eabs, *gmeta;                  // conv2 edge lists (conv2_attn.cu)
   uint16_t* eent;
   uint16_t* csr_ptr;
@@ -1149,23 +1131,17 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
     const uint32_t* adjm = cached ? cache.adjm : ws.adjm;
     // radius graph (unless cached), then the controlling-node list and the needed rows
     if (!cached && (rc = launch_csr(st, obs, a->obs_stride, N, gc, ws.csr_ptr, ws.csr_src, hl ? nullptr : ws.adjm))) return rc;
-    // needed rows ordered with the controlling nodes first (row = slot): relu(conv1) of a controlling node is written once
-    // (not with the single-linear head, which reads whole latent rows of z)
-    const bool ctrl_first = !hl && !w->out_w && mls_get_option("ctrl_first");
     if (!hl) {
       MLS_CUDA(cudaMemsetAsync(ws.count, 0, 4 * sizeof(int), st));
       const unsigned grid = (unsigned)((gc * 32 + 255) / 256);
 #define MLS_LIST(WW) ctrl_need_list_kernel<WW><<<grid, 256, 0, st>>>(cm, obs, a->obs_stride, N, gc, a->ctrl_mode, adjm, gid, gid_stride, ws.idx, \
                                                                       ws.slot, ws.count, ws.gfirst, ws.gcnt, ws.nidx, ws.xrow, ws.ncount, ws.nfirst, ws.ncnt, \
-                                                                      csr_ptr, csr_src, tr ? 0 : 1, ws.ecount, ws.eabs, use_c2 ? ws.eent : nullptr, ws.gmeta, ctrl_first ? 1 : 0)
+                                                                      csr_ptr, csr_src, tr ? 0 : 1, ws.ecount, ws.eabs, use_c2 ? ws.eent : nullptr, ws.gmeta)
       switch (Wn) { case 1: MLS_LIST(1); break; case 2: MLS_LIST(2); break; case 4: MLS_LIST(4); break; default: MLS_LIST(8); break; }
 #undef MLS_LIST
-      mls_count_launch();
-      if (ctrl_first) {
-        const int nthr = rows > gc ? rows : gc;
-        need_rows_fixup_kernel<<<(nthr + 255) / 256, 256, 0, st>>>(ws.xrow, ws.nidx, use_c2 ? ws.gmeta : nullptr, ws.count, ws.ncount, ws.ntotal, rows, gc);
-        mls_count_launch();
-      }
+      const int nthr = rows > gc ? rows : gc;
+      need_rows_fixup_kernel<<<(nthr + 255) / 256, 256, 0, st>>>(ws.xrow, ws.nidx, use_c2 ? ws.gmeta : nullptr, ws.count, ws.ncount, ws.ntotal, rows, gc);
+      mls_count_launch(2);
     }
     // encoder (or, in discrete-feature mode, just the table keys of this pass)
     if (use_table) {
@@ -1185,25 +1161,24 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
       if ((rc = gemm_bf16_launch(ws.x0, hid, ws.w_c1, hid, GemmShape{rows, nproj * HC, hid, nullptr}, e1, sms, st))) return rc;
       prof_end(MLS_PROF_PROJ1);
     }
-    // conv1 attention (+ReLU): relu(conv1) of the needed rows (compacted, x1), snapshot x1[ctrl] (pre-mask) into z;
-    // HL-DGN: graph pooling into z
+    // conv1 attention (+ReLU): relu(conv1) of the needed rows (compacted, x1; x1[0 : count) are the controlling nodes'
+    // snapshot rows, pre-mask); HL-DGN: graph pooling into z
     {
       EdgeArgs ea{};
       ea.P = use_table ? ws.t_P : ws.P; ea.ldp = nproj * HC; ea.obs = obs; ea.obs_stride = a->obs_stride; ea.N = N; ea.H = H;
       ea.n_graphs = gc; ea.row_key = use_table ? ws.key : nullptr;
       ea.att = w->c1_att; ea.bias = w->c1_bias; ea.csr_ptr = csr_ptr; ea.csr_src = csr_src; ea.ab = use_table ? ws.t_ab : ws.ab;
       ea.graph_id = gid; ea.gid_stride = gid_stride;
-      if (hl) { ea.x_out = nullptr; ea.slot = nullptr; ea.z = ws.z; ea.ldz = latent; ea.z_col = 0; ea.ctrl_only = 0; ea.pool_mode = d->pool; }
-      else { ea.x_out = ws.x1; ea.slot = ctrl_first ? nullptr : ws.slot; ea.z = ws.z; ea.ldz = latent; ea.z_col = hid; ea.ctrl_only = 0; ea.pool_mode = -1; ea.xrow_out = ws.xrow; }
+      if (hl) { ea.x_out = nullptr; ea.z = ws.z; ea.ldz = latent; ea.z_col = 0; ea.ctrl_only = 0; ea.pool_mode = d->pool; }
+      else { ea.x_out = ws.x1; ea.ctrl_only = 0; ea.pool_mode = -1; ea.xrow_out = ws.xrow; }
       prof_begin(MLS_PROF_EDGE1);
       if (use_mma) {
         AttnTableArgs ta{};
         ta.t_P = ws.t_P; ta.ldp = nproj * HC; ta.t_ab = ws.t_ab; ta.att = w->c1_att; ta.bias = tr ? nullptr : w->c1_bias;
         ta.transformer = tr ? 1 : 0; ta.key = ws.key; ta.N = N; ta.H = H; ta.n_graphs = gc; ta.csr_ptr = csr_ptr;
         ta.csr_src = csr_src; ta.graph_id = gid; ta.gid_stride = gid_stride;
-        ta.slot = ctrl_first ? nullptr : ws.slot; ta.xrow = ws.xrow; ta.x_out = ws.x1; ta.z = ws.z; ta.ldz = latent; ta.z_col = hid;
-        ta.pool_mode = -1;
-        if (hl) { ta.slot = nullptr; ta.xrow = nullptr; ta.x_out = nullptr; ta.z_col = 0; ta.pool_mode = d->pool; ta.obs = obs; ta.obs_stride = a->obs_stride; }
+        if (hl) { ta.z = ws.z; ta.ldz = latent; ta.z_col = 0; ta.pool_mode = d->pool; ta.obs = obs; ta.obs_stride = a->obs_stride; }
+        else { ta.xrow = ws.xrow; ta.x_out = ws.x1; ta.pool_mode = -1; }
         ta.used_bits = ws.used; ta.n_keys = n_keys; ta.cid_of_key = ws.cid_of_key; ta.key_of_cid = ws.key_of_cid;
         ta.n_used = ws.n_used; ta.E = ws.pairE; ta.row_cid = ws.row_cid; ta.Vh = ws.Vh;
         ta.rec = ws.rec; ta.tile_idx = ws.tile_idx;
@@ -1216,9 +1191,8 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
     if (!hl) {
       // conv2 projections on x1 * dm (the row mask commutes with the GEMM, applied in its epilogue), both in one launch
       // over the packed weight rows (Transformer [q; k; v], GATv2 [l; r]).  Source side (GATv2 x_l, Transformer k | v) on
-      // the needed rows; target side (GATv2 x_r, Transformer q) on the controlling nodes: x1[0 : count) itself
-      // (ctrl_first, the x1 tile is read once for both), else their snapshot columns of z.  fp16 outputs for the
-      // tensor-core attention.
+      // the needed rows; target side (GATv2 x_r, Transformer q) on the controlling nodes: x1[0 : count) itself (the x1
+      // tile is read once for both).  fp16 outputs for the tensor-core attention.
       const int nsrc = nproj - 1;
       bf16* Psrc = ws.P;                                    // [needed rows][nsrc*HC]
       bf16* Ptgt = ws.P + (size_t)rows * nsrc * HC;         // [count][HC]
@@ -1226,9 +1200,8 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
       GemmEpilogue e{Psrc, nsrc * HC, ws.b_c2, obs, a->obs_stride, N, 0, tr ? nullptr : ws.att2, tr ? nullptr : ws.ab, ws.nidx};
       e.c_fp16 = use_c2 ? 1 : 0;
       e.Ct = Ptgt; e.ldct = HC; e.dots_t = tr ? nullptr : dots_t; e.row_index_t = ws.idx;
-      GemmShape sh{rows, nproj * HC, HC, ctrl_first ? ws.ntotal : ws.ncount};
+      GemmShape sh{rows, nproj * HC, HC, ws.ntotal};
       sh.m_dev_t = ws.count; sh.t_lo = tr ? 0 : HC; sh.t_hi = sh.t_lo + HC;
-      if (!ctrl_first) { sh.A2 = ws.z + hid; sh.lda2 = latent; sh.k2_lo = 0; sh.k2_hi = HC; }
       prof_begin(MLS_PROF_PROJ2);
       if ((rc = gemm_bf16_launch(ws.x1, HC, ws.w_c2, HC, sh, e, sms, st))) return rc;
       prof_end(MLS_PROF_PROJ2);
@@ -1239,7 +1212,7 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
         ca.Ps = reinterpret_cast<const __half*>(Psrc); ca.lds = nsrc * HC; ca.Pt = reinterpret_cast<const __half*>(Ptgt); ca.ldt = HC;
         ca.as = ws.ab; ca.bt = dots_t; ca.att = w->c2_att; ca.bias = tr ? nullptr : w->c2_bias; ca.transformer = tr ? 1 : 0;
         ca.N = N; ca.H = H; ca.n_graphs = gc; ca.gmeta = ws.gmeta; ca.eabs = ws.eabs; ca.eent = ws.eent;
-        ca.z = ws.z; ca.ldz = latent; ca.z_col = hid + HC; ca.ctrl_first = ctrl_first ? 1 : 0;
+        ca.z = ws.z; ca.ldz = latent; ca.z_col = hid + HC;
         if ((rc = conv2_attn_launch(ca, sms, st))) return rc;
       } else {
         EdgeArgs ea{};
@@ -1260,19 +1233,19 @@ int dgn_forward_bf16(const MlsNetDesc* d, const MlsNetWeights* w, const MlsForwa
     const int* m_dev = hl ? nullptr : ws.count;
     if (w->out_w) {                                           // no dueling heads: one linear layer on the latent row
       if (!hl) {
-        head_linear_b_kernel<<<(rows * 32 + 255) / 256, 256, 0, st>>>(ws.z, latent, ws.idx, ws.count, rows, w->out_w, w->out_b,
-                                                                      (int64_t)g0 * N, N, a->q, a->act, a->ctrl_mode, aa);
+        head_linear_b_kernel<<<(rows * 32 + 255) / 256, 256, 0, st>>>(ws.z, latent, ws.x1, hid, HC, ws.idx, ws.count, rows, w->out_w,
+                                                                      w->out_b, (int64_t)g0 * N, N, a->q, a->act, a->ctrl_mode, aa);
         mls_count_launch();
       } else {
-        head_linear_b_kernel<<<(gc * 32 + 255) / 256, 256, 0, st>>>(ws.z, latent, nullptr, nullptr, gc, w->out_w, w->out_b, 0, N, ws.qg,
-                                                                    nullptr, 2, aa);
+        head_linear_b_kernel<<<(gc * 32 + 255) / 256, 256, 0, st>>>(ws.z, latent, nullptr, 0, HC, nullptr, nullptr, gc, w->out_w, w->out_b,
+                                                                    0, N, ws.qg, nullptr, 2, aa);
         const long long nthr = a->ctrl_mode == 1 ? gc : (long long)gc * N;
         hl_scatter_b_kernel<<<(unsigned)((nthr + 255) / 256), 256, 0, st>>>(ws.qg, cm, N, gc, g0, a->ctrl_mode, a->q, a->act, aa);
         mls_count_launch(2);
       }
     } else {
       GemmShape sh0{head_rows, hh2, latent, m_dev};
-      if (ctrl_first) { sh0.A2 = ws.x1; sh0.lda2 = HC; sh0.k2_lo = hid; sh0.k2_hi = hid + HC; }   // snapshot columns come from x1
+      if (!hl) { sh0.A2 = ws.x1; sh0.lda2 = HC; sh0.k2_lo = hid; sh0.k2_hi = hid + HC; }   // snapshot columns come from x1
       prof_begin(MLS_PROF_HEAD0);
       if (hh == 128) {
         // both hidden layers, the output layer and the action in one kernel: the hidden activations stay on chip
