@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define MLS_VERSION 213
+#define MLS_VERSION 214
 #define MLS_MAX_NODES 256
 
 /* ---- errors ------------------------------------------------------------------------- */
@@ -180,6 +180,41 @@ int mls_env_step(const MlsEnvDesc* desc, const MlsEnvState* state, const MlsRoun
 
 /* get_info (graph.py:149-179) for all episodes without stepping. */
 int mls_env_info(const MlsEnvDesc* desc, const MlsEnvState* state, MlsInfo* info, void* stream);
+
+/* ---- device episode sampler (since version 214).  The second source of episode resets, next to MlsResetTuples:
+ * instead of reading a row of a host-drawn pool, every restart draws a fresh training-mode tuple (core.py:371-395) from
+ * a counter-based Philox stream keyed by (seed, global slot, episode number of that slot).  It matches the reference in
+ * distribution, not draw for draw (the host pool is the draw-for-draw path):
+ *   graph   uniform over [0, pool_size)            source  uniform over [0, N)
+ *   k       int((0.1 + 0.9 u) * N), u a 53-bit uniform, in fp64 as numpy's uniform(0.1, 1.0) computes it
+ *   interested  a uniform k-subset of the nodes, independent of source
+ *   scripted    an independent uniform n_scripted-subset, minus source when drop_source_from_scripted
+ * Episode number r of a slot is its episode[b][MLS_EP_N_RESETS] before the restart bumps it (r = 0: first reset).
+ * The global slot is the batch-wide episode index (episode_offset + b for a sub-batch view) + slot_offset, so
+ * sub-batch views draw what a full-batch call draws, and rank k of a job passing slot_offset = k * B draws
+ * episodes no other rank draws.  The counters never meet those of the movement or epsilon-greedy streams. */
+typedef struct MlsEpisodeSampler {
+  uint64_t seed;
+  int32_t pool_size;                 /* graphs drawn from [0, pool_size); 1 <= pool_size <= state.pool_size     */
+  int32_t n_scripted;                /* round(ratio * N) with round half to even (Python's round); 0 <= . <= N */
+  int32_t drop_source_from_scripted; /* ratio < 1 (core.py:213-215)                                           */
+  int32_t slot_offset;               /* added to the batch-wide episode index                                 */
+} MlsEpisodeSampler;
+
+/* mls_env_reset with the tuple of episode k drawn by the sampler: slot env_ids[k] (NULL: k), episode number
+ * episode[slot][MLS_EP_N_RESETS].  n episodes; `in` rows are indexed by k as in mls_env_reset. */
+int mls_env_reset_sampled(const MlsEnvDesc* desc, const MlsEnvState* state, const int32_t* env_ids, int32_t n,
+                          const MlsEpisodeSampler* sampler, const MlsRoundInputs* in, const MlsRoundOutputs* out,
+                          void* stream);
+/* mls_env_step whose finished episodes restart, in the same launch, from the sampler instead of a tuple pool. */
+int mls_env_step_sampled(const MlsEnvDesc* desc, const MlsEnvState* state, const MlsRoundInputs* in,
+                         const MlsRoundOutputs* out, const MlsEpisodeSampler* sampler, void* stream);
+/* Materialise n sampled tuples: tuple m is episode number episode_no[m] of batch-wide slot slot[m] (slot_offset is
+ * added as in the environment calls).  Output in the MlsResetTuples layout: graph_index [n], source [n],
+ * interested / scripted [n][W] bitmasks with W = mls_words_per_row(n_nodes) (words past ceil(N/32) are zero). */
+int mls_episode_sample(const MlsEpisodeSampler* sampler, int32_t n_nodes, const int32_t* slot, const int32_t* episode_no,
+                       int32_t n, int32_t* graph_index, int32_t* source, uint32_t* interested, uint32_t* scripted,
+                       void* stream);
 
 /* ===== Q-network forward + action selection ============================================
  * Replaces graph_env/env/utils/networks/{common.py:6-64, dgn_r.py:82-129, l_dgn.py:92-151,

@@ -39,6 +39,11 @@ class MlsResetTuples(C.Structure):
                 ("pad_", C.c_int32)]
 
 
+class MlsEpisodeSampler(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("pool_size", C.c_int32), ("n_scripted", C.c_int32),
+                ("drop_source_from_scripted", C.c_int32), ("slot_offset", C.c_int32)]
+
+
 class MlsInfo(C.Structure):
     _fields_ = [(k, C.c_int32) for k in (
         "total_messages_transmitted", "covered", "messages_sent", "messages_received", "n_neighbours",
@@ -95,7 +100,7 @@ EXPORTS = ["mls_version", "mls_last_error", "mls_device_info", "mls_words_per_ro
            "mls_adam_step", "mls_train_list_capacity", "mls_train_lists", "mls_gatv2_edge_fwd", "mls_gatv2_edge_bwd_blocks",
            "mls_gatv2_edge_bwd", "mls_transformer_edge_fwd", "mls_transformer_edge_bwd", "mls_per_tree_size",
            "mls_per_build", "mls_per_sample", "mls_per_update", "mls_linear_bf16_workspace_bytes", "mls_linear_bf16_fwd",
-           "mls_linear_bf16_bwd"]
+           "mls_linear_bf16_bwd", "mls_env_reset_sampled", "mls_env_step_sampled", "mls_episode_sample"]
 PACKED_NODE_BYTES = 12
 
 _lib = None
@@ -128,6 +133,11 @@ def lib():
     L.mls_env_step.argtypes = [P(MlsEnvDesc), P(MlsEnvState), P(MlsRoundInputs), P(MlsRoundOutputs),
                                P(MlsResetTuples), vp]
     L.mls_env_info.argtypes = [P(MlsEnvDesc), P(MlsEnvState), vp, vp]
+    L.mls_env_reset_sampled.argtypes = [P(MlsEnvDesc), P(MlsEnvState), vp, C.c_int32, P(MlsEpisodeSampler),
+                                        P(MlsRoundInputs), P(MlsRoundOutputs), vp]
+    L.mls_env_step_sampled.argtypes = [P(MlsEnvDesc), P(MlsEnvState), P(MlsRoundInputs), P(MlsRoundOutputs),
+                                       P(MlsEpisodeSampler), vp]
+    L.mls_episode_sample.argtypes = [P(MlsEpisodeSampler), C.c_int32, vp, vp, C.c_int32, vp, vp, vp, vp, vp]
     L.mls_dgn_workspace_bytes.argtypes = [P(MlsNetDesc), C.c_int32]
     L.mls_dgn_workspace_bytes.restype = C.c_size_t
     L.mls_dgn_chunk_graphs.argtypes = [P(MlsNetDesc), C.c_int32]

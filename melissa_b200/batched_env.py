@@ -59,6 +59,62 @@ class ResetTuplesDevice:
                                    _lib.ptr(self.scripted), self.count, 0)
 
 
+def scripted_count(scripted_agents_ratio: float, n_nodes: int) -> int:
+    """Scripted agents per episode, ``round(ratio * N)`` with Python's round (half to even), as the reference draws
+    them (core.py:213)."""
+    return int(round(scripted_agents_ratio * n_nodes))
+
+
+class EpisodeStream:
+    """Training-mode episode resets drawn on the device: a fresh tuple (graph, source, interested set, scripted set)
+    for every reset, without a host-built pool.  Episode number ``r`` of global slot ``s`` is a counter-based Philox
+    draw keyed by ``(seed, s, r)`` (include/melissa_b200.h, ``MlsEpisodeSampler``); the global slot of environment
+    episode ``b`` is ``b + slot_offset``, so ranks that pass ``slot_offset = rank * B`` never play each other's episodes
+    (:func:`melissa_b200.sharding.rank_slot_offset`).  Graphs are drawn uniformly from the first ``pool_size`` graphs
+    of the environment's topology pool.
+
+    The tuples follow the reference's training reset chain in distribution, not draw for draw; a
+    :class:`ResetTuplesDevice` pool built by :func:`melissa_b200.reset_chain.episode_pool` is the draw-for-draw path."""
+
+    def __init__(self, n_nodes: int, pool_size: int, seed: int, scripted_agents_ratio: float = 0.0, slot_offset: int = 0):
+        if not (0.0 <= scripted_agents_ratio <= 1.0):
+            raise ValueError("`scripted_agents_ratio` must be in [0.0, 1.0].")          # core.py:143-144
+        if not 1 <= int(n_nodes) <= 256:
+            raise ValueError(f"n_nodes must be in [1, 256], got {n_nodes}")
+        if int(pool_size) < 1:
+            raise ValueError(f"pool_size must be >= 1, got {pool_size}")
+        if not 0 <= int(slot_offset) < 2 ** 31:
+            raise ValueError(f"slot_offset must be in [0, 2**31), got {slot_offset}")
+        self.n_nodes, self.pool_size, self.seed = int(n_nodes), int(pool_size), int(seed)
+        self.scripted_agents_ratio, self.slot_offset = float(scripted_agents_ratio), int(slot_offset)
+        self.n_scripted = scripted_count(self.scripted_agents_ratio, self.n_nodes)
+        self.sampler = _lib.MlsEpisodeSampler(self.seed % 2 ** 64, self.pool_size, self.n_scripted,
+                                              int(self.scripted_agents_ratio < 1.0), self.slot_offset)
+
+    def sample(self, slots, episode_no, device="cuda") -> ResetTuplesDevice:
+        """The tuples episode ``episode_no`` of slot ``slots`` plays (both broadcast to one shape, flattened), as a
+        :class:`ResetTuplesDevice` in row order -- exactly what a stream environment draws for those restarts."""
+        s, r = np.broadcast_arrays(np.asarray(slots, dtype=np.int64), np.asarray(episode_no, dtype=np.int64))
+        s, r = s.ravel(), r.ravel()
+        if len(s) and (s.min() < 0 or r.min() < 0 or s.max() >= 2 ** 31 or r.max() >= 2 ** 31):
+            raise ValueError("slots and episode numbers must be in [0, 2**31)")
+        n, W, dev = len(s), _lib.words_per_row(self.n_nodes), torch.device(device)
+        out = ResetTuplesDevice.__new__(ResetTuplesDevice)
+        out.count, out.max_graph = n, self.pool_size - 1
+        out.graph_index = torch.empty(n, dtype=torch.int32, device=dev)
+        out.source = torch.empty(n, dtype=torch.int32, device=dev)
+        out.interested = torch.empty(n, W, dtype=torch.int32, device=dev)
+        out.scripted = torch.empty(n, W, dtype=torch.int32, device=dev)
+        if n:
+            sd = torch.as_tensor(s.astype(np.int32), device=dev)
+            rd = torch.as_tensor(r.astype(np.int32), device=dev)
+            _lib.check(_lib.lib().mls_episode_sample(C.byref(self.sampler), self.n_nodes, sd.data_ptr(), rd.data_ptr(), n,
+                                                     out.graph_index.data_ptr(), out.source.data_ptr(),
+                                                     out.interested.data_ptr(), out.scripted.data_ptr(),
+                                                     _lib.current_stream_ptr()))
+        return out
+
+
 class BatchedGraphEnv:
     """Device-resident vector of ``n_episodes`` graph environments.
 
@@ -104,7 +160,7 @@ class BatchedGraphEnv:
         self.done = torch.zeros(B, dtype=torch.uint8, device=dev)
         self.info_buf = torch.zeros(B, C.sizeof(_lib.MlsInfo) // 4, dtype=torch.int32, device=dev) if want_info else None
         self.transitions = torch.zeros(1, dtype=torch.int64, device=dev)
-        self.recycle: ResetTuplesDevice | None = None
+        self.recycle: ResetTuplesDevice | EpisodeStream | None = None
         self.philox_seed = 9
         self._state = _lib.MlsEnvState(
             _lib.ptr(self.node), _lib.ptr(self.recv_count), _lib.ptr(self.recv_from), _lib.ptr(self.episode),
@@ -138,10 +194,14 @@ class BatchedGraphEnv:
         return st, keep
 
     # ------------------------------------------------------------------ API
-    def reset(self, tuples: ResetTuplesDevice, env_ids=None, *, move_offsets=None, gossip_bits=None, relay_bits=None):
+    def reset(self, tuples: ResetTuplesDevice | EpisodeStream, env_ids=None, *, move_offsets=None, gossip_bits=None,
+              relay_bits=None):
         """Reset episodes ``env_ids`` (default: 0..count) from ``tuples`` -- World.reset +
         GraphEnv.reset (reference core.py:388-437, graph.py:222-248) incl. the forced
-        first broadcast.  Returns (obs, active)."""
+        first broadcast.  With an :class:`EpisodeStream` the episodes ``env_ids`` (default: all) draw their next
+        episode on the device.  Returns (obs, active)."""
+        if isinstance(tuples, EpisodeStream):
+            return self._reset_sampled(tuples, env_ids, move_offsets, gossip_bits, relay_bits)
         ids = None
         if env_ids is not None:
             ids = torch.as_tensor(np.asarray(env_ids, dtype=np.int32), device=self.device)
@@ -156,15 +216,48 @@ class BatchedGraphEnv:
                                           C.byref(inp), C.byref(self._out), _lib.current_stream_ptr()))
         return self.obs, self.active
 
-    def set_recycling(self, tuples: ResetTuplesDevice | None):
-        """Episodes that finish are restarted inside the step kernel from this pool."""
-        if tuples is not None:
+    def _reset_sampled(self, stream: EpisodeStream, env_ids, move_offsets, gossip_bits, relay_bits):
+        self._check_stream(stream)
+        ids = None
+        n = self.B
+        if env_ids is not None:
+            ids = torch.as_tensor(np.asarray(env_ids, dtype=np.int32).ravel(), device=self.device)
+            n = len(ids)
+        inp, keep = self._inputs(None, move_offsets, gossip_bits, relay_bits)
+        _lib.check(self.lib.mls_env_reset_sampled(C.byref(self.desc), C.byref(self._state), _lib.ptr(ids), n,
+                                                  C.byref(stream.sampler), C.byref(inp), C.byref(self._out),
+                                                  _lib.current_stream_ptr()))
+        return self.obs, self.active
+
+    def set_recycling(self, tuples: ResetTuplesDevice | EpisodeStream | None):
+        """Episodes that finish are restarted inside the step kernel from this pool, or with a fresh episode drawn on
+        the device when ``tuples`` is an :class:`EpisodeStream`."""
+        if isinstance(tuples, EpisodeStream):
+            self._check_stream(tuples)
+        elif tuples is not None:
             self._check_tuples(tuples)
         self.recycle = tuples
 
     def _check_tuples(self, tuples: ResetTuplesDevice):
         if getattr(tuples, "max_graph", -1) >= len(self.pool):
             raise ValueError(f"reset tuples name graph {tuples.max_graph} but the topology pool holds {len(self.pool)} graphs")
+
+    def _check_stream(self, stream: EpisodeStream):
+        if stream.n_nodes != self.N:
+            raise ValueError(f"episode stream draws {stream.n_nodes}-node episodes, the environment has {self.N} nodes")
+        if stream.pool_size > len(self.pool):
+            raise ValueError(f"episode stream draws from {stream.pool_size} graphs but the topology pool holds {len(self.pool)}")
+
+    def _step(self, desc, state, inp, out):
+        rec = self.recycle
+        if isinstance(rec, EpisodeStream):
+            rc = self.lib.mls_env_step_sampled(C.byref(desc), C.byref(state), C.byref(inp), C.byref(out), C.byref(rec.sampler),
+                                               _lib.current_stream_ptr())
+        else:
+            t = rec.c_struct() if rec is not None else None
+            rc = self.lib.mls_env_step(C.byref(desc), C.byref(state), C.byref(inp), C.byref(out),
+                                       C.byref(t) if t is not None else None, _lib.current_stream_ptr())
+        _lib.check(rc)
 
     def step(self, actions, *, move_offsets=None, gossip_bits=None, relay_bits=None):
         """One round for all episodes.  ``actions`` int8 [B, N] (device tensor or numpy):
@@ -173,17 +266,13 @@ class BatchedGraphEnv:
         if tuple(actions.shape) != (self.B, self.N):
             raise ValueError(f"actions must have shape {(self.B, self.N)}, got {tuple(actions.shape)}")
         inp, keep = self._inputs(actions, move_offsets, gossip_bits, relay_bits)
-        rec = self.recycle.c_struct() if self.recycle is not None else None
-        _lib.check(self.lib.mls_env_step(C.byref(self.desc), C.byref(self._state), C.byref(inp), C.byref(self._out),
-                                         C.byref(rec) if rec is not None else None, _lib.current_stream_ptr()))
+        self._step(self.desc, self._state, inp, self._out)
         return self.obs, self.reward, self.active, self.terminated, self.done
 
     def step_device(self, actions_i8: torch.Tensor):
         """Hot-loop variant of :meth:`step`: ``actions_i8`` is already a contiguous int8 device tensor."""
         inp = _lib.MlsRoundInputs(actions_i8.data_ptr(), None, None, None, self.philox_seed)
-        rec = self.recycle.c_struct() if self.recycle is not None else None
-        _lib.check(self.lib.mls_env_step(C.byref(self.desc), C.byref(self._state), C.byref(inp), C.byref(self._out),
-                                         C.byref(rec) if rec is not None else None, _lib.current_stream_ptr()))
+        self._step(self.desc, self._state, inp, self._out)
 
     def step_device_slice(self, actions_i8: torch.Tensor, b0: int, b1: int):
         """One round for episodes ``[b0, b1)`` only (``actions_i8`` = the matching int8 rows).  The slices of
@@ -202,9 +291,7 @@ class BatchedGraphEnv:
             views[key] = (desc, state, out)
         desc, state, out = views[key]
         inp = _lib.MlsRoundInputs(actions_i8.data_ptr(), None, None, None, self.philox_seed)
-        rec = self.recycle.c_struct() if self.recycle is not None else None
-        _lib.check(self.lib.mls_env_step(C.byref(desc), C.byref(state), C.byref(inp), C.byref(out),
-                                         C.byref(rec) if rec is not None else None, _lib.current_stream_ptr()))
+        self._step(desc, state, inp, out)
 
     def info(self):
         """``get_info`` counters for every episode (reference graph.py:149-179) as a dict of numpy arrays."""

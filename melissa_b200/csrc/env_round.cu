@@ -16,6 +16,7 @@
 //                         graph_env/env/graph.py:303-389,402-463,254-271 -> finalize_round()
 //   World.reset + GraphEnv.reset  core.py:388-437, graph.py:222-248 -> reset path
 #include "common.cuh"
+#include "episode_sampler.cuh"
 
 namespace {
 
@@ -30,6 +31,8 @@ struct EnvParams {
   MlsRoundInputs in;
   MlsRoundOutputs out;
   MlsResetTuples tup;      // reset tuples (mode 1) / recycle pool (mode 0, count==0 -> none)
+  MlsEpisodeSampler smp;   // smp_on: resets / restarts draw from the device episode sampler instead of `tup`
+  int smp_on;              // selects the SAMPLED kernels
   const int32_t* env_ids;  // mode 1
   int mode;                // 0 step, 1 reset, 2 info only
   int n_work;
@@ -379,8 +382,10 @@ __device__ __forceinline__ void load_topology(const EnvParams& p, const Smem<W>&
   for (int w = 0; w < W; ++w) mine[w] = th.adj[w];
 }
 
-template <int W>
-__global__ void __launch_bounds__(kThreads) env_round_kernel(const EnvParams p) {
+// SAMPLED: the reset / recycle branch draws its tuples from the device episode sampler (p.smp) instead of p.tup.
+// The sampled kernels of W <= 2 are held to the 64 registers of the pool kernels (16 CTAs of 64 threads per SM).
+template <int W, bool SAMPLED>
+__global__ void __launch_bounds__(kThreads, SAMPLED && W <= 2 ? 4 : 0) env_round_kernel(const EnvParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int N = p.d.n_nodes;
   const int NP = ((N + 31) >> 5) << 5;
@@ -563,7 +568,7 @@ __global__ void __launch_bounds__(kThreads) env_round_kernel(const EnvParams p) 
       if (p.out.reward) p.out.reward[row] = r;
       if (p.out.terminated) p.out.terminated[row] = trunc ? 1 : 0;
     }
-    do_reset = ep_valid && done && p.tup.count > 0;
+    do_reset = ep_valid && done && (SAMPLED || p.tup.count > 0);
   } else if (p.mode == 2) {
     // ------------------------------------------------------------ get_info only (graph.py:149-179)
     publish<W>(sm, M_B, le, wq, valid && (th.node & MLS_F_HAS_MESSAGE));
@@ -605,17 +610,39 @@ __global__ void __launch_bounds__(kThreads) env_round_kernel(const EnvParams p) 
     atomicAdd(p.out.transitions, (unsigned long long)sm.cnt[G * 4]);      // one atomic per CTA
   if (any_reset) {
     size_t trow = 0;
+    bool s_int = false, s_scr = false;
+    if constexpr (SAMPLED) {
+      // episode number n_resets of global slot b + b_off + slot_offset.  The node keys go through sm.pos, which nobody
+      // reads again before the forced step rewrites it (after the barrier in front of world_step)
+      ulonglong2* keys = reinterpret_cast<ulonglong2*>(sm.pos) + (size_t)le * NP;
+      episode_sampler::Scalars es{};
+      uint32_t slot = 0;
+      if (do_reset) {
+        if (p.mode == 1) ep.n_resets = p.s.episode[(size_t)b * MLS_EP_STRIDE + MLS_EP_N_RESETS];
+        slot = (uint32_t)(b + b_off) + (uint32_t)p.smp.slot_offset;
+        es = episode_sampler::scalars(p.smp, N, slot, (uint32_t)ep.n_resets);
+        if (valid) keys[i] = episode_sampler::node_keys(p.smp, slot, (uint32_t)ep.n_resets, i);
+      }
+      __syncthreads();
+      if (do_reset) {
+        ep.graph = es.graph;
+        ep.source = es.source;
+        if (valid) episode_sampler::membership(keys, N, i, es, p.smp, s_int, s_scr);
+      }
+    }
     if (do_reset) {
       // World.reset (core.py:388-437) + GraphEnv.reset (graph.py:227-248)
-      trow = (p.mode == 1) ? (size_t)k : (size_t)(((long long)b + b_off + (long long)ep.n_resets * B) % p.tup.count);
-      ep.graph = p.tup.graph_index[trow];
-      ep.source = p.tup.source[trow];
+      if constexpr (!SAMPLED) {
+        trow = (p.mode == 1) ? (size_t)k : (size_t)(((long long)b + b_off + (long long)ep.n_resets * B) % p.tup.count);
+        ep.graph = p.tup.graph_index[trow];
+        ep.source = p.tup.source[trow];
+      }
       ep.world_msgs = 0; ep.num_moves = 0; ep.rsum = 0.0;
-      if (p.mode == 1) ep.n_resets = p.s.episode[(size_t)b * MLS_EP_STRIDE + MLS_EP_N_RESETS];
+      if (!SAMPLED && p.mode == 1) ep.n_resets = p.s.episode[(size_t)b * MLS_EP_STRIDE + MLS_EP_N_RESETS];
       if (valid) {
         uint32_t f = 0;
-        if (p.tup.interested[trow * W + wq] & mybit) f |= MLS_F_INTERESTED;
-        if (p.tup.scripted[trow * W + wq] & mybit) f |= MLS_F_SCRIPTED;
+        if (SAMPLED ? s_int : (p.tup.interested[trow * W + wq] & mybit) != 0) f |= MLS_F_INTERESTED;
+        if (SAMPLED ? s_scr : (p.tup.scripted[trow * W + wq] & mybit) != 0) f |= MLS_F_SCRIPTED;
         if (i == ep.source) f |= MLS_F_ORIGIN | MLS_F_HAS_MESSAGE | (1u << MLS_NODE_STEPS_SHIFT);   // core.py:432-435
         th.node = f;
         th.rc = 0;
@@ -665,7 +692,7 @@ __global__ void __launch_bounds__(kThreads) env_round_kernel(const EnvParams p) 
   }
 }
 
-template <int W>
+template <int W, bool SAMPLED>
 int launch_env(const EnvParams& p, cudaStream_t stream) {
   const int N = p.d.n_nodes;
   const int NP = ((N + 31) / 32) * 32;
@@ -678,19 +705,24 @@ int launch_env(const EnvParams& p, cudaStream_t stream) {
   size_t smem = sizeof(double) * G * NP * 3 + sizeof(uint32_t) * G * NP * W * 2 +
                 sizeof(uint32_t) * M_COUNT * G * W + sizeof(int) * (G * 4 + 1);
   if (blocks == 0) return MLS_OK;
-  env_round_kernel<W><<<blocks, threads, smem, stream>>>(p);
+  env_round_kernel<W, SAMPLED><<<blocks, threads, smem, stream>>>(p);
   mls_count_launch();
   MLS_LAUNCH_CHECK();
   return MLS_OK;
 }
 
+template <bool SAMPLED>
+int dispatch_w(const EnvParams& p, cudaStream_t st) {
+  const int W = (p.d.n_nodes + 31) / 32;
+  if (W <= 1) return launch_env<1, SAMPLED>(p, st);
+  if (W <= 2) return launch_env<2, SAMPLED>(p, st);
+  if (W <= 4) return launch_env<4, SAMPLED>(p, st);
+  return launch_env<8, SAMPLED>(p, st);
+}
+
 int dispatch_env(const EnvParams& p, void* stream) {
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int W = (p.d.n_nodes + 31) / 32;
-  if (W <= 1) return launch_env<1>(p, st);
-  if (W <= 2) return launch_env<2>(p, st);
-  if (W <= 4) return launch_env<4>(p, st);
-  return launch_env<8>(p, st);
+  return p.smp_on ? dispatch_w<true>(p, st) : dispatch_w<false>(p, st);
 }
 
 int check_common(const MlsEnvDesc* d, const MlsEnvState* s) {
@@ -704,6 +736,39 @@ int check_common(const MlsEnvDesc* d, const MlsEnvState* s) {
   const bool relay = d->heuristic == MLS_HEUR_MPR || d->heuristic == MLS_HEUR_PROBABILISTIC_RELAY;
   MLS_CHECK_ARG(!relay || s->recv_from, "heuristic %d needs state.recv_from", d->heuristic);
   return MLS_OK;
+}
+
+// mls_episode_sample: one thread per (tuple, node), NP = 32*ceil(N/32) threads per tuple as in the round kernel.
+__global__ void __launch_bounds__(kThreads) episode_sample_kernel(const MlsEpisodeSampler smp, int N, int W,
+                                                                  const int32_t* slot, const int32_t* episode_no, int n,
+                                                                  int32_t* graph_index, int32_t* source, uint32_t* interested,
+                                                                  uint32_t* scripted) {
+  __shared__ ulonglong2 keys[kThreads];
+  const int NP = ((N + 31) >> 5) << 5;
+  const int G = blockDim.x / NP;
+  const int le = threadIdx.x / NP;
+  const int i = threadIdx.x - le * NP;
+  const int m = blockIdx.x * G + le;
+  const bool ok = m < n;          // uniform over the tuple's warps
+  const bool valid = ok && i < N;
+  episode_sampler::Scalars es{};
+  if (ok) {
+    const uint32_t s = (uint32_t)slot[m] + (uint32_t)smp.slot_offset, r = (uint32_t)episode_no[m];
+    es = episode_sampler::scalars(smp, N, s, r);
+    if (valid) keys[le * NP + i] = episode_sampler::node_keys(smp, s, r, i);
+  }
+  __syncthreads();
+  bool in_i = false, in_s = false;
+  if (valid) episode_sampler::membership(keys + le * NP, N, i, es, smp, in_i, in_s);
+  const uint32_t bi = __ballot_sync(0xffffffffu, in_i), bs = __ballot_sync(0xffffffffu, in_s);
+  if (!ok) return;
+  const size_t row = (size_t)m * W;
+  if ((i & 31) == 0) { interested[row + (i >> 5)] = bi; scripted[row + (i >> 5)] = bs; }
+  if (i == 0) {
+    graph_index[m] = es.graph;
+    source[m] = es.source;
+    for (int w = NP >> 5; w < W; ++w) { interested[row + w] = 0u; scripted[row + w] = 0u; }
+  }
 }
 
 }  // namespace
@@ -758,6 +823,58 @@ extern "C" int mls_env_step(const MlsEnvDesc* desc, const MlsEnvState* state, co
   return dispatch_env(p, stream);
 }
 
+static int check_sampler(const MlsEnvDesc* d, const MlsEnvState* s, const MlsEpisodeSampler* smp) {
+  MLS_CHECK_ARG(smp, "sampler is NULL");
+  MLS_CHECK_ARG(smp->pool_size >= 1 && smp->pool_size <= s->pool_size,
+                "sampler pool_size must be in [1, %d] (the topology pool), got %d", s->pool_size, smp->pool_size);
+  MLS_CHECK_ARG(smp->n_scripted >= 0 && smp->n_scripted <= d->n_nodes, "sampler n_scripted must be in [0, %d], got %d",
+                d->n_nodes, smp->n_scripted);
+  return MLS_OK;
+}
+
+extern "C" int mls_env_reset_sampled(const MlsEnvDesc* desc, const MlsEnvState* state, const int32_t* env_ids, int32_t n,
+                                     const MlsEpisodeSampler* sampler, const MlsRoundInputs* in, const MlsRoundOutputs* out,
+                                     void* stream) {
+  int rc = check_common(desc, state);
+  if (rc) return rc;
+  rc = check_sampler(desc, state, sampler);
+  if (rc) return rc;
+  MLS_CHECK_ARG(n >= 0, "n < 0");
+  MLS_CHECK_ARG(n <= desc->n_episodes || env_ids, "more resets than episodes");
+  if (n == 0) return MLS_OK;
+  EnvParams p{};
+  p.d = *desc; p.s = *state;
+  if (in) p.in = *in;
+  if (out) p.out = *out;
+  p.smp = *sampler;
+  p.smp_on = 1;
+  p.env_ids = env_ids;
+  p.mode = 1;
+  p.n_work = n;
+  MLS_CHECK_ARG(desc->heuristic != MLS_HEUR_PROBABILISTIC_GOSSIP || p.in.gossip_bits, "probabilistic_gossip needs gossip_bits");
+  MLS_CHECK_ARG(desc->heuristic != MLS_HEUR_PROBABILISTIC_RELAY || p.in.relay_bits, "probabilistic_relay needs relay_bits");
+  return dispatch_env(p, stream);
+}
+
+extern "C" int mls_env_step_sampled(const MlsEnvDesc* desc, const MlsEnvState* state, const MlsRoundInputs* in,
+                                    const MlsRoundOutputs* out, const MlsEpisodeSampler* sampler, void* stream) {
+  int rc = check_common(desc, state);
+  if (rc) return rc;
+  rc = check_sampler(desc, state, sampler);
+  if (rc) return rc;
+  MLS_CHECK_ARG(in && in->actions, "actions missing");
+  EnvParams p{};
+  p.d = *desc; p.s = *state; p.in = *in;
+  if (out) p.out = *out;
+  p.smp = *sampler;
+  p.smp_on = 1;
+  p.mode = 0;
+  p.n_work = desc->n_episodes;
+  MLS_CHECK_ARG(desc->heuristic != MLS_HEUR_PROBABILISTIC_GOSSIP || p.in.gossip_bits, "probabilistic_gossip needs gossip_bits");
+  MLS_CHECK_ARG(desc->heuristic != MLS_HEUR_PROBABILISTIC_RELAY || p.in.relay_bits, "probabilistic_relay needs relay_bits");
+  return dispatch_env(p, stream);
+}
+
 extern "C" int mls_env_info(const MlsEnvDesc* desc, const MlsEnvState* state, MlsInfo* info, void* stream) {
   int rc = check_common(desc, state);
   if (rc) return rc;
@@ -768,4 +885,24 @@ extern "C" int mls_env_info(const MlsEnvDesc* desc, const MlsEnvState* state, Ml
   p.mode = 2;
   p.n_work = desc->n_episodes;
   return dispatch_env(p, stream);
+}
+
+extern "C" int mls_episode_sample(const MlsEpisodeSampler* sampler, int32_t n_nodes, const int32_t* slot,
+                                  const int32_t* episode_no, int32_t n, int32_t* graph_index, int32_t* source,
+                                  uint32_t* interested, uint32_t* scripted, void* stream) {
+  MLS_CHECK_ARG(sampler, "sampler is NULL");
+  MLS_CHECK_ARG(n_nodes >= 1 && n_nodes <= MLS_MAX_NODES, "n_nodes must be in [1, %d], got %d", MLS_MAX_NODES, n_nodes);
+  MLS_CHECK_ARG(sampler->pool_size >= 1, "sampler pool_size must be >= 1, got %d", sampler->pool_size);
+  MLS_CHECK_ARG(sampler->n_scripted >= 0 && sampler->n_scripted <= n_nodes, "sampler n_scripted must be in [0, %d], got %d",
+                n_nodes, sampler->n_scripted);
+  MLS_CHECK_ARG(n >= 0, "n < 0");
+  MLS_CHECK_ARG(slot && episode_no && graph_index && source && interested && scripted, "episode_sample arrays missing");
+  if (n == 0) return MLS_OK;
+  const int NP = ((n_nodes + 31) / 32) * 32;
+  const int G = kThreads / NP;
+  episode_sample_kernel<<<(n + G - 1) / G, G * NP, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      *sampler, n_nodes, mls_words_per_row(n_nodes), slot, episode_no, n, graph_index, source, interested, scripted);
+  mls_count_launch();
+  MLS_LAUNCH_CHECK();
+  return MLS_OK;
 }

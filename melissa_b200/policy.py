@@ -25,7 +25,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .batched_env import BatchedGraphEnv, ResetTuplesDevice
+from .batched_env import BatchedGraphEnv, EpisodeStream, ResetTuplesDevice
 from .networks.autograd import q_values
 from .networks.common import DGNBase
 
@@ -493,11 +493,13 @@ class BatchedCollector:
     """``MultiAgentCollector`` over a :class:`BatchedGraphEnv` (built with ``want_info=True``): same constructor
     keywords (``agents_num=, policy=, env=, buffer=, exploration_noise=``) and ``collect`` signature.  One iteration =
     forward + action selection + one environment round for every episode, on the device; finished episodes restart
-    inside the step kernel from ``tuples`` (the reference's vector env resets them one by one).  With ``buffer`` (a
+    inside the step kernel from ``tuples`` (the reference's vector env resets them one by one): a
+    :class:`ResetTuplesDevice` pool, or an :class:`EpisodeStream` that draws a fresh episode on the device for every
+    reset.  With ``buffer`` (a
     :class:`melissa_b200.replay.DeviceReplay`) every agent transition of the round is stored, completed by the
     world step's reward exactly as multi_agent_collector.py:240-308 completes it on the agent's next observation."""
 
-    def __init__(self, policy=None, env: BatchedGraphEnv = None, tuples: ResetTuplesDevice = None,
+    def __init__(self, policy=None, env: BatchedGraphEnv = None, tuples: ResetTuplesDevice | EpisodeStream = None,
                  exploration_noise: bool = False, *, agents_num: int | None = None, buffer=None, **kwargs):
         if policy is None or env is None:
             raise TypeError("BatchedCollector needs policy= and env=")
@@ -525,12 +527,15 @@ class BatchedCollector:
         self.reset()
 
     def reset(self, reset_buffer: bool = True, gym_reset_kwargs=None):
-        if self.tuples.count < self.env.B:
-            raise ValueError(f"need at least {self.env.B} reset tuples (one per episode), got {self.tuples.count}")
-        first = ResetTuplesDevice.__new__(ResetTuplesDevice)
-        first.count = self.env.B
-        for k in ("graph_index", "source", "interested", "scripted"):
-            setattr(first, k, getattr(self.tuples, k)[: self.env.B])
+        if isinstance(self.tuples, EpisodeStream):
+            first = self.tuples                  # every episode, the first ones included, is a fresh device draw
+        else:
+            if self.tuples.count < self.env.B:
+                raise ValueError(f"need at least {self.env.B} reset tuples (one per episode), got {self.tuples.count}")
+            first = ResetTuplesDevice.__new__(ResetTuplesDevice)
+            first.count = self.env.B
+            for k in ("graph_index", "source", "interested", "scripted"):
+                setattr(first, k, getattr(self.tuples, k)[: self.env.B])
         self.env.episode.zero_()
         self.env.reset(first)
         self.env.set_recycling(self.tuples)

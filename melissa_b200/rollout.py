@@ -12,7 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .batched_env import BatchedGraphEnv, ResetTuplesDevice
+from .batched_env import BatchedGraphEnv, EpisodeStream, ResetTuplesDevice
 from .networks.common import DGNBase
 from . import reset_chain
 
@@ -51,15 +51,20 @@ class Rollout:
         gi, src, inter, scr, _ = reset_chain.episode_pool(base_seed, count, env.N, len(env.pool), scripted_agents_ratio)
         return ResetTuplesDevice(gi, src, inter, scr, env.N, env.device)
 
-    def start(self, tuples: ResetTuplesDevice, recycle: bool = True):
-        """Reset every episode from the first B tuples; finished episodes restart from the pool."""
-        if tuples.count < self.env.B:
-            raise ValueError(f"need at least {self.env.B} reset tuples (one per episode), got {tuples.count}")
-        first = ResetTuplesDevice.__new__(ResetTuplesDevice)
-        first.count = self.env.B
-        first.graph_index, first.source = tuples.graph_index[: self.env.B], tuples.source[: self.env.B]
-        first.interested, first.scripted = tuples.interested[: self.env.B], tuples.scripted[: self.env.B]
-        self.env.episode.zero_()            # restart counters too: the recycle pool is walked from its beginning again
+    def start(self, tuples: ResetTuplesDevice | EpisodeStream, recycle: bool = True):
+        """Reset every episode from the first B tuples; finished episodes restart from the pool.  With an
+        :class:`EpisodeStream` every episode, the first ones and every restart (also under CUDA-graph replay: the
+        episode numbers live in device state), is a fresh device draw."""
+        if isinstance(tuples, EpisodeStream):
+            first = tuples
+        else:
+            if tuples.count < self.env.B:
+                raise ValueError(f"need at least {self.env.B} reset tuples (one per episode), got {tuples.count}")
+            first = ResetTuplesDevice.__new__(ResetTuplesDevice)
+            first.count = self.env.B
+            first.graph_index, first.source = tuples.graph_index[: self.env.B], tuples.source[: self.env.B]
+            first.interested, first.scripted = tuples.interested[: self.env.B], tuples.scripted[: self.env.B]
+        self.env.episode.zero_()            # restart counters too: the recycle pool / stream is walked from its beginning again
         self.env.reset(first)
         self.env.set_recycling(tuples if recycle else None)
         self.round_index = 0

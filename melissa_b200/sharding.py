@@ -18,6 +18,13 @@ def rank_seed_range(base_seed: int, rank: int, pool_count: int):
     return int(base_seed) + first, first
 
 
+def rank_slot_offset(rank: int, episodes_per_rank: int) -> int:
+    """``slot_offset`` of rank ``rank``'s :class:`melissa_b200.batched_env.EpisodeStream`: ``rank * episodes_per_rank``.
+    The device episode stream is keyed by the global slot (episode index + slot_offset), so ranks of equal batch size
+    that share a seed draw disjoint episode sequences, as :func:`rank_seed_range` gives disjoint pools."""
+    return int(rank) * int(episodes_per_rank)
+
+
 def shard_tuples(arrays, rank: int, episodes_per_rank: int, world: int = 1):
     """Slice of a SHARED reset-tuple pool owned by ``rank``: rows [rank*P, (rank+1)*P) with
     P = len(pool) // world >= episodes_per_rank.  Raises when the pool is too small for disjoint slices."""
